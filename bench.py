@@ -19,6 +19,8 @@ batch of synthetic 8x224^2 clips (ViT-B/16 student with the shipped drop_path 0.
   ddp_parity (N > 1)  one fused NVLink optimizer step against NCCL all-reduce + ub_adamw_seg on the same gradients
 --impl reference times the reference's own CPU implementation (see cpu_baseline) with the optimizer step included.
 --workload stage2|stage3|vitl: the other BASELINE.json configs as their own lines (not the driver's headline).
+--dump-outputs DIR: after the timed steps, the last step's results as DIR/<name>.npy (see dump_outputs); the inputs depend only on
+the arguments, so two builds run with the same arguments can be compared array by array.
 """
 import argparse
 import json
@@ -323,6 +325,38 @@ def ddp_parity_check(eng, batch0, world):
     return res
 
 
+def dump_outputs(out_dir, eng, student, loss, world, rows=8192, per_param=8192):
+    """What the last timed step handed its caller, as float32 DIR/<name>.npy (about 35 MB at B = 32), so that two builds can be
+    compared output for output: loss, gradient norm, the teacher's attention and the token mask (1 = masked) in full; the student's
+    outputs and the teacher's targets at the same seeded sample of `rows` (layer, clip, token position) triples, zero where the
+    token is masked; a seeded sample of up to `per_param` elements of every updated student parameter, taken by name in sorted
+    order (independent of the parameter arena's layout).
+    Rows are addressed by token position, not by place among the visible rows: a token whose visibility flips between two runs
+    (attention values within fp noise of each other, a few of 50 176 tokens) then changes its own row only and shifts no other."""
+    import numpy as np
+    import torch
+    eng.optimizer.consolidate()            # collective: with the optimizer sharded by rank, every rank then holds all weights
+    if int(os.environ.get("RANK", "0")) != 0:
+        return
+    rng = np.random.default_rng(0)
+    last = eng.last
+    out, vis = last["outputs"], last["vis_idx"].long()                     # [K, B, Nv, C]; [B, Nv] ascending token positions
+    K, B, Nv, C = out.shape
+    N = last["mask"].shape[1]
+    pick = lambda n, k: torch.from_numpy(np.sort(rng.choice(n, min(n, k), replace=False))).to(out.device)
+    r = pick(K * B * N, rows)
+    k, b, n = r // (B * N), r // N % B, r % N
+    row = torch.full((B, N), -1, dtype=torch.long, device=out.device).scatter_(1, vis, torch.arange(Nv, device=out.device).expand(B, Nv))
+    j = row[b, n]                                                           # -1: token masked
+    at = lambda t: torch.where((j >= 0)[:, None], t.reshape(K, B, Nv, C)[k, b, j.clamp(min=0)], 0)
+    params = [p.detach().reshape(-1)[pick(p.numel(), per_param)] for _, p in sorted(student.named_parameters())]
+    arrays = dict(loss=loss, grad_norm=eng.optimizer.grad_norm(1.0 / world), teacher_attn=last["attn"], mask=last["mask"],
+                  student_outputs=at(out), teacher_targets=at(last["targets"]), student_params=torch.cat(params))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 # ---------------------------------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -335,7 +369,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-eager-baseline", action="store_true")
     ap.add_argument("--profile-out", default=None, help="write the per-op breakdown of one instrumented step here (json)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (float32, stage1 workload)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "stage1"):
+        ap.error("--dump-outputs needs --impl ours --workload stage1")
     if args.batch is None:
         args.batch = 8 if args.workload == "stage3" else 32
     if args.impl == "reference":
@@ -423,6 +463,8 @@ def main():
     value = world * B / (ms_per_step * 1e-3)
     loss_value = loss.item()
     graphs_captured = len(eng._graphs)
+    if args.dump_outputs:                  # before the end-to-end runs below train further and overwrite eng.last
+        dump_outputs(args.dump_outputs, eng, student, loss, world)
 
     # ---- end to end through the public API: pinned host batches, H2D inside the timed region, loss read back ------
     u8_default = world > 1        # N > 1: one host feeds every GPU — decoded uint8 frames (a quarter of the bytes) are the default feed

@@ -17,8 +17,15 @@ def _free_port():
     return p
 
 
+def _cpu_rank_env(rank, world, port):
+    # the ranks stay on the CPU even on a GPU box: with CUDA visible, init_distributed_from_env binds cuda:LOCAL_RANK, and a box
+    # with one GPU has no cuda:1
+    os.environ.update(CUDA_VISIBLE_DEVICES="", MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world),
+                      LOCAL_RANK=str(rank))
+
+
 def _worker(rank, world, port, q):
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank))
+    _cpu_rank_env(rank, world, port)
     from unite_b200.ddp import GradSync, init_distributed_from_env
     r, _, w = init_distributed_from_env(backend="gloo")
     assert (r, w) == (rank, world)
@@ -80,7 +87,7 @@ def test_nvls_shards_tile_the_decay_segment():
 
 def _consolidate_worker(rank, world, port, q):
     import types
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank))
+    _cpu_rank_env(rank, world, port)
     from unite_b200.ddp import NvlsShardedStep, init_distributed_from_env
     init_distributed_from_env(backend="gloo")
     n, n_decay = 4096, 4096 - 72
