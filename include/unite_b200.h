@@ -208,6 +208,13 @@ UB_API int ub_patchify(const float* x, void* out, int B, int T, int H, int W, in
  * (src/datasets/kinetics_sparse.py:236-243, 434-451); mean3 / std3 are HOST pointers to 3 floats.                     */
 UB_API int ub_patchify_u8(const uint8_t* x, void* out, const float* mean3, const float* std3, int B, int T, int H, int W,
                           int tubelet, void* stream);
+/* resize + patchify for the teacher: fp32 clip [B,3,T,H,W] (x_is_u8 = 0) or decoded uint8 frames [B,T,H,W,3] (x_is_u8 = 1,
+ * normalised with the HOST mean3 / std3 as ub_patchify_u8 does, before the resize) -> bicubic resize of every (c, t) plane to
+ * R x R (torch interpolate mode="bicubic", align_corners=False, antialias=False; no resize when R == H == W) -> bf16 im2col rows
+ * [B*(T/tubelet)*(R/patch)^2, ld_out] in ub_patchify's token / feature order, for any even patch size.  ld_out >= 3*tubelet*patch^2,
+ * a multiple of 8; the padding columns are written as zeros (a GEMM may contract over the padded K against zero weights). */
+UB_API int ub_resize_patchify(const void* x, int x_is_u8, const float* mean3, const float* std3, void* out, int64_t ld_out, int B,
+                              int T, int H, int W, int R, int patch, int tubelet, void* stream);
 UB_API int ub_mask_select(const float* attn, const float* q, uint8_t* mask, int* vis_idx, int* tea_rows, int frames,
                           int P, int T, int k, int n_vis, void* stream);
 UB_API int ub_gather_rows(const void* in, const int* idx, void* out, int64_t n_rows, int64_t row_bytes,

@@ -70,13 +70,15 @@ class VisionTransformer(nn.Module):
         super().__init__()
         if clip_norm_type != "l2":
             raise NotImplementedError("clip_norm_type must be 'l2'")
-        if patch_size != 16:
-            raise NotImplementedError("the patchify kernel is specialised for 16x16 patches (clip_b16)")
+        if patch_size not in (14, 16):
+            raise NotImplementedError(f"patch_size {patch_size}: the teacher runs 14x14 (clip_l14) or 16x16 (clip_b16) patches")
         if width // heads != 64:
             raise NotImplementedError("the attention kernels are specialised for head_dim 64")
         self.clip_norm_type, self.return_attn, self.return_cls = clip_norm_type, return_attn, return_cls
         self.output_dim, self.width, self.heads, self.kernel_size = output_dim, width, heads, kernel_size
         self.input_resolution, self.patch_size = input_resolution, patch_size
+        # conv1 runs as a GEMM over im2col rows of 3*ks*p*p features, padded to a multiple of 64 (588 for a 14-pixel patch)
+        self.k_pad = ops.padded_k(3 * kernel_size * patch_size * patch_size)
         self.conv1 = nn.Conv3d(3, width, (kernel_size, patch_size, patch_size), (kernel_size, patch_size, patch_size), (0, 0, 0),
                                bias=False)
         scale = width ** -0.5
@@ -100,7 +102,8 @@ class VisionTransformer(nn.Module):
             raise RuntimeError("unite_b200 models compute on CUDA only: call teacher.cuda() first (there is no CPU path)")
         if self._w16 is None or v != self._w_version or self._w16["proj_t"].device != dev:
             W = self.width
-            w = {"conv1": self.conv1.weight.detach().reshape(W, -1).to(BF16).contiguous(),
+            conv1 = self.conv1.weight.detach().reshape(W, -1)
+            w = {"conv1": torch.nn.functional.pad(conv1, (0, self.k_pad - conv1.shape[1])).to(BF16).contiguous(),
                  "proj_t": self.proj.detach().t().to(BF16).contiguous()}
             for i, blk in enumerate(self.transformer.resblocks):
                 w[f"{i}.in_proj"] = blk.attn.in_proj_weight.detach().to(BF16).contiguous()
@@ -134,9 +137,12 @@ class VisionTransformer(nn.Module):
 
     # ---- compute ---------------------------------------------------------------------------
     @torch.no_grad()
-    def forward_features(self, x, patches=None, select=None):
-        """Runs the tower.  Returns (layers: list of K fp32 [B*T'*(HW+1), W] residual-stream snapshots after the
-        blocks in clip_return_layers, attn fp32 [B*T', HW] or None, patches bf16 im2col rows).
+    def forward_features(self, x, patches=None, select=None, resolution=None):
+        """Runs the tower on the clip x fp32 [B,3,T,H,W] seen at `resolution` x `resolution` (None: H).  When that differs
+        from H or W the clip is resized on the device (bicubic, as the reference's engine does before its teacher call);
+        `patches` (bf16 im2col rows [frames*P, k_pad] of the clip at that resolution) are used as they are.
+        Returns (layers: list of K fp32 [B*T'*(HW+1), W] residual-stream snapshots after the blocks in clip_return_layers,
+        attn fp32 [B*T', HW] or None, patches bf16 im2col rows).
 
         select: optional callable(attn) -> int32 row indices (into the [frames*(HW+1)] token stream) of the tokens whose
         features will be used.  The LAST block's attention map only needs its QKV projection, and nothing after it reads
@@ -144,12 +150,22 @@ class VisionTransformer(nn.Module):
         (80 % fewer rows in stage 1); that snapshot is then [n_selected, W] and `self.last_gathered` is True."""
         w = self._weights()
         B, _, T, H, Wd = x.shape
-        ks, W = self.kernel_size, self.width
-        Tp, P = T // ks, (H // 16) * (Wd // 16)
+        ks, W, p = self.kernel_size, self.width, self.patch_size
+        R = H if resolution is None else int(resolution)
+        resize = R != H or R != Wd
+        if R % p or (not resize and Wd % p):
+            raise ValueError(f"teacher resolution {R}x{R if resize else Wd} is not a multiple of its patch size {p}")
+        Tp, P = T // ks, (R // p) * ((R if resize else Wd) // p)
+        if P + 1 != self.positional_embedding.shape[0]:
+            raise ValueError(f"the teacher sees {P} patches per frame at {R} px, but its positional embedding holds "
+                             f"{self.positional_embedding.shape[0] - 1} (input_resolution {self.input_resolution}, patch size {p})")
         frames = B * Tp
         if patches is None:
-            patches = torch.empty(frames * P, 3 * ks * 256, device=x.device, dtype=BF16)
-            ops.patchify(x.contiguous(), patches, ks)
+            patches = torch.empty(frames * P, self.k_pad, device=x.device, dtype=BF16)
+            if p == 16 and not resize:
+                ops.patchify(x.contiguous(), patches, ks)
+            else:
+                ops.resize_patchify(x.contiguous(), patches, R, p, ks)
         bufs = self._work_buffers(frames, P)
         S = P + 1
         ops.gemm(patches, w["conv1"], bufs["E"])
@@ -269,7 +285,13 @@ class VisionTransformer(nn.Module):
         if self.return_cls:
             raise NotImplementedError("return_cls is off in every shipped config")
         B, _, T, H, Wd = x.shape
-        Tp, P = T // self.kernel_size, (H // 16) * (Wd // 16)
+        p = self.patch_size
+        P = (H // p) * (Wd // p)
+        if H % p or Wd % p or P + 1 != self.positional_embedding.shape[0]:
+            raise ValueError(f"a {H}x{Wd} clip does not match the teacher's patch grid: {p}-pixel patches and a positional embedding "
+                             f"for {self.positional_embedding.shape[0] - 1} patches per frame (input_resolution {self.input_resolution}); "
+                             "forward() does not resize, resize the clip to input_resolution first")
+        Tp = T // self.kernel_size
         layers, attn, _ = self.forward_features(x)
         feat = self.project_rows(layers, self._all_patch_rows(B, Tp, P, x.device)).view(len(layers), B, Tp * P, self.output_dim)
         return (feat, attn) if self.return_attn else feat

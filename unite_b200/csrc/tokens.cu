@@ -86,6 +86,144 @@ __global__ void __launch_bounds__(256) patchify_u8_kernel(const uint8_t* __restr
 }
 
 // ------------------------------------------------------------------------------------------------
+// resize_patchify: fp32 clip [B,3,T,H,W] or uint8 frames [B,T,H,W,3] -> (bicubic resize to R x R) -> bf16 im2col rows
+// [B*(T/tub)*(R/p)^2, ld] for any even patch size p; feature order (c,kt,kh,kw) as ub_patchify, columns [3*tub*p*p, ld) zero.
+// The resize is torch.nn.functional.interpolate(mode="bicubic", align_corners=False, antialias=False) per (c, t) plane:
+//   src = scale * (dst + 0.5) - 0.5, scale = in / out;  i0 = min(floor(src), in - 1), f = clamp(src - i0, 0, 1);
+//   taps i0-1 .. i0+2 clamped to the border, cubic-convolution weights with A = -0.75 computed in fp32;
+//   out = sum_j wy_j * (sum_i wx_i * x[y_j, x_i]), summed in that order (ATen's separable upsample kernel).
+// uint8 input is normalised first (same IEEE divides as patchify_u8), as the reference's loader normalises and its engine
+// then resizes.  One CTA = one (clip, output frame, kt, patch row): the source rows that band of p output rows reads are
+// staged [3][rows][W] fp32 in shared memory (each source pixel leaves HBM once, up to the 3-4 rows two bands share), then
+// consecutive threads write consecutive bf16 pairs of one token's row.
+// ------------------------------------------------------------------------------------------------
+UB_DEVINL float cubic_near(float x, float A) { return ((A + 2.f) * x - (A + 3.f)) * x * x + 1.f; }          // |x| <= 1
+UB_DEVINL float cubic_far(float x, float A) { return ((A * x - 5.f * A) * x + 8.f * A) * x - 4.f * A; }     // 1 < |x| < 2
+
+// source tap indices (clamped to [0, n)) and weights of output coordinate `dst`
+UB_DEVINL void bicubic_taps(int dst, float scale, int n, int* idx, float* w) {
+  const float src = __fsub_rn(__fmul_rn(scale, __fadd_rn((float)dst, 0.5f)), 0.5f);
+  const int i0 = min((int)floorf(src), n - 1);
+  const float f = fminf(fmaxf(src - (float)i0, 0.f), 1.f);
+  const float A = -0.75f;
+  w[0] = cubic_far(f + 1.f, A);
+  w[1] = cubic_near(f, A);
+  w[2] = cubic_near(1.f - f, A);
+  w[3] = cubic_far((1.f - f) + 1.f, A);
+#pragma unroll
+  for (int j = 0; j < 4; ++j) idx[j] = min(max(i0 - 1 + j, 0), n - 1);
+}
+
+template <bool U8>
+__global__ void __launch_bounds__(256) resize_patchify_kernel(const void* __restrict__ xin, bf16* __restrict__ out, long ld, float m0,
+                                                              float m1, float m2, float s0, float s1, float s2, int T, int H, int W,
+                                                              int R, int p, int tub, int rows_max, float sy, float sx, int identity) {
+  pdl_grid_sync();
+  extern __shared__ float rp_smem[];
+  const int gr = R / p, Tp = T / tub;
+  int blk = blockIdx.x;
+  const int ph = blk % gr; blk /= gr;
+  const int kt = blk % tub; blk /= tub;
+  const int tp = blk % Tp;
+  const int b = blk / Tp;
+  const int t = tp * tub + kt;
+  float* pix = rp_smem;                                      // [3][rows_max][W]
+  float* wx = pix + 3 * rows_max * W;                        // [R][4]
+  int* ix = reinterpret_cast<int*>(wx + 4 * R);              // [R][4]
+  float* wy = reinterpret_cast<float*>(ix + 4 * R);          // [p][4]
+  int* iy = reinterpret_cast<int*>(wy + 4 * p);              // [p][4], relative to y_lo
+  const int oy0 = ph * p;
+  int y_lo = oy0, nrows = p;
+  if (!identity) {
+    int i[4];
+    float w[4];
+    bicubic_taps(oy0, sy, H, i, w);
+    y_lo = i[0];
+    bicubic_taps(oy0 + p - 1, sy, H, i, w);
+    nrows = i[3] - y_lo + 1;
+    for (int o = threadIdx.x; o < R + p; o += blockDim.x) {
+      if (o < R) {
+        bicubic_taps(o, sx, W, ix + 4 * o, wx + 4 * o);
+      } else {
+        const int r = o - R;
+        bicubic_taps(oy0 + r, sy, H, iy + 4 * r, wy + 4 * r);
+#pragma unroll
+        for (int j = 0; j < 4; ++j) iy[4 * r + j] -= y_lo;
+      }
+    }
+  }
+  // ---- stage the band's source rows ----
+  const long plane = (long)H * W;
+  if constexpr (U8) {
+    const uint8_t* src = static_cast<const uint8_t*>(xin) + (((long)b * T + t) * H + y_lo) * (long)W * 3;
+    const int n = nrows * W * 3;
+    for (int e = threadIdx.x; e < n; e += blockDim.x) {
+      const int c = e % 3, px = e / 3;
+      const float mean = c == 0 ? m0 : (c == 1 ? m1 : m2), sd = c == 0 ? s0 : (c == 1 ? s1 : s2);
+      const float v = __fdiv_rn(__fsub_rn(__fdiv_rn((float)src[e], 255.0f), mean), sd);
+      pix[(c * rows_max + px / W) * W + px % W] = v;
+    }
+  } else {
+    const float* x = static_cast<const float*>(xin);
+    const int n = nrows * W;
+    for (int c = 0; c < 3; ++c) {
+      const float* src = x + (((long)b * 3 + c) * T + t) * plane + (long)y_lo * W;
+      float* dst = pix + c * rows_max * W;
+      if ((W & 3) == 0) {
+        for (int e = threadIdx.x; e < n / 4; e += blockDim.x)
+          reinterpret_cast<float4*>(dst)[e] = __ldg(reinterpret_cast<const float4*>(src) + e);
+      } else {
+        for (int e = threadIdx.x; e < n; e += blockDim.x) dst[e] = __ldg(src + e);
+      }
+    }
+  }
+  __syncthreads();
+  // ---- resample + write: item = (pw, c, kh, kw pair), kw pair fastest ----
+  const int hp = p / 2, pp = p * p, feat = 3 * tub * pp;
+  const long tok0 = (((long)b * Tp + tp) * gr + ph) * gr;
+  const int n_items = gr * 3 * p * hp;
+  for (int e = threadIdx.x; e < n_items; e += blockDim.x) {
+    const int kwp = e % hp;
+    int r = e / hp;
+    const int kh = r % p; r /= p;
+    const int c = r % 3;
+    const int pw = r / 3;
+    const int ox = pw * p + 2 * kwp;
+    const float* pc = pix + c * rows_max * W;
+    float v[2];
+    if (identity) {
+      v[0] = pc[kh * W + ox];
+      v[1] = pc[kh * W + ox + 1];
+    } else {
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const int* xi = ix + 4 * (ox + h);
+        const float* xw = wx + 4 * (ox + h);
+        float acc = 0.f;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          const float* row = pc + iy[4 * kh + j] * W;
+          float s = row[xi[0]] * xw[0];
+          s += row[xi[1]] * xw[1];
+          s += row[xi[2]] * xw[2];
+          s += row[xi[3]] * xw[3];
+          acc = j == 0 ? s * wy[4 * kh] : acc + s * wy[4 * kh + j];
+        }
+        v[h] = acc;
+      }
+    }
+    bf16* dst = out + (tok0 + pw) * ld + c * (tub * pp) + kt * pp + kh * p + 2 * kwp;
+    *reinterpret_cast<uint32_t*>(dst) = pack_bf16x2(v[0], v[1]);
+  }
+  // ---- zero the row padding of this band's tokens (once per token: the kt == 0 CTA) ----
+  if (kt == 0 && ld > feat) {
+    const int hpad = (int)(ld - feat) / 2;
+    for (int e = threadIdx.x; e < gr * hpad; e += blockDim.x)
+      *reinterpret_cast<uint32_t*>(out + (tok0 + e / hpad) * ld + feat + 2 * (e % hpad)) = 0u;
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
 // mask selection.  One warp per frame (row of attn): score = attn / q (IEEE fp32 divide, same as torch),
 // rank_i = #{j : s_j > s_i or (s_j == s_i and j < i)};  member = rank % k, visible for that member iff rank / k < n_vis.
 // Outputs (all per member m):
@@ -255,6 +393,42 @@ extern "C" int ub_patchify_u8(const uint8_t* x, void* out, const float* mean3, c
   UB_LAUNCH(patchify_u8_kernel, flat_grid(runs, 256), 256, 0, (cudaStream_t)stream, x, (bf16*)out, mean3[0], mean3[1], mean3[2], std3[0],
             std3[1], std3[2], B, T, H, W, tubelet, runs);
   return check_launch("patchify_u8_kernel");
+}
+
+extern "C" int ub_resize_patchify(const void* x, int x_is_u8, const float* mean3, const float* std3, void* out, int64_t ld_out, int B,
+                                  int T, int H, int W, int R, int patch, int tubelet, void* stream) {
+  UB_REQUIRE(x && out, "resize_patchify: null pointer");
+  UB_REQUIRE(B > 0 && T > 0 && tubelet > 0 && T % tubelet == 0, "resize_patchify: bad temporal shape T=%d tubelet=%d", T, tubelet);
+  UB_REQUIRE(patch >= 2 && patch <= 32 && patch % 2 == 0, "resize_patchify: patch size %d must be even (2..32)", patch);
+  UB_REQUIRE(H > 0 && W > 0 && R > 0 && R % patch == 0, "resize_patchify: output resolution R=%d must be a multiple of the patch size %d",
+             R, patch);
+  const int feat = 3 * tubelet * patch * patch;
+  UB_REQUIRE(ld_out >= feat && ld_out % 8 == 0, "resize_patchify: row pitch %lld must be >= %d and a multiple of 8", (long long)ld_out, feat);
+  UB_REQUIRE((reinterpret_cast<uintptr_t>(out) & 15) == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0,
+             "resize_patchify: input and output must be 16-byte aligned");
+  UB_REQUIRE(!x_is_u8 || (mean3 && std3 && std3[0] != 0.f && std3[1] != 0.f && std3[2] != 0.f), "resize_patchify: uint8 input needs mean / std");
+  const int identity = (R == H && R == W) ? 1 : 0;
+  const float sy = (float)H / (float)R, sx = (float)W / (float)R;           // ATen area_pixel_compute_scale (align_corners=False)
+  int rows_max = identity ? patch : (int)ceilf((patch - 1) * sy) + 6;      // source rows one band of `patch` output rows reads
+  if (rows_max > H) rows_max = H;
+  const size_t smem = ((size_t)3 * rows_max * W + (identity ? 0 : (size_t)8 * (R + patch))) * sizeof(float);
+  UB_REQUIRE(smem <= 220 * 1024, "resize_patchify: a band of %d source rows x W=%d does not fit in shared memory", rows_max, W);
+  const long ctas = (long)B * (T / tubelet) * tubelet * (R / patch);
+  UB_REQUIRE(ctas < (1L << 31), "resize_patchify: too many tokens");
+  float m[3] = {0.f, 0.f, 0.f}, s[3] = {1.f, 1.f, 1.f};
+  if (x_is_u8) {
+    for (int i = 0; i < 3; ++i) { m[i] = mean3[i]; s[i] = std3[i]; }
+  }
+  auto kern = x_is_u8 ? resize_patchify_kernel<true> : resize_patchify_kernel<false>;
+  static size_t smem_set[2] = {48 * 1024, 48 * 1024};
+  if (smem > smem_set[x_is_u8 ? 1 : 0]) {
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    UB_REQUIRE(e == cudaSuccess, "cudaFuncSetAttribute(resize_patchify smem=%zu): %s", smem, cudaGetErrorString(e));
+    smem_set[x_is_u8 ? 1 : 0] = smem;
+  }
+  UB_LAUNCH(kern, (int)ctas, 256, smem, (cudaStream_t)stream, x, (bf16*)out, (long)ld_out, m[0], m[1], m[2], s[0], s[1], s[2], T, H, W, R,
+            patch, tubelet, rows_max, sy, sx, identity);
+  return check_launch("resize_patchify_kernel");
 }
 
 extern "C" int ub_mask_select(const float* attn, const float* q, uint8_t* mask, int* vis_idx, int* tea_rows, int frames,

@@ -313,7 +313,12 @@ class Stage1Engine:
                     raise
                 import warnings
                 warnings.warn(f"unite_b200: NVLS fused optimizer step unavailable ({type(e).__name__}: {e}); using NCCL all-reduce")
-        self.share_patches = student.encoder.patch_embed.tubelet_size == teacher.kernel_size
+        # the resolution the teacher sees (train_one_epoch's clip_input_resolution): a clip of another size is resized for the
+        # teacher only (bicubic, on the device); the student always patchifies the clip as it comes
+        self.teacher_resolution = teacher.input_resolution
+        if student.clip_output_dim != teacher.output_dim:
+            raise ValueError(f"the student's clip_output_dim {student.clip_output_dim} differs from the teacher's output_dim "
+                             f"{teacher.output_dim}: the alignment loss compares the two")
         self.loss = torch.zeros(1, device=self.core.arena.device, dtype=F32)
         self.last = {}
         self.drop_path = self.core.drop_path       # vit_core.DropPathSource: device-side draws, one launch per step
@@ -335,6 +340,26 @@ class Stage1Engine:
         self._graphs.clear()                    # captured graphs hold the old optimizer's buffers
         self._graph_count.clear()
 
+    @property
+    def share_patches(self) -> bool:
+        """Student and teacher read one im2col of the clip: same temporal kernel, 16-pixel teacher patches, no resize."""
+        side = self.student.encoder.patch_embed.img_size
+        return (self.student.encoder.patch_embed.tubelet_size == self.teacher.kernel_size and self.teacher.patch_size == 16
+                and tuple(side) == (self.teacher_resolution, self.teacher_resolution))
+
+    def teacher_view(self, H: int, W: int):
+        """(resolution, resize?) of the teacher for an H x W clip; ValueError when the configuration cannot align the teacher's
+        attention map with the student's tokens."""
+        R, p = int(self.teacher_resolution), self.teacher.patch_size
+        if R % p:
+            raise ValueError(f"teacher resolution {R} is not a multiple of the teacher's patch size {p}")
+        ps = self.student.encoder.patch_embed.patch_size[0]
+        n_t, n_s = (R // p) ** 2, (H // ps) * (W // ps)
+        if n_t != n_s:
+            raise ValueError(f"the teacher sees {n_t} patches per frame ({R} px / {p}), the student {n_s} ({H}x{W} px / {ps}): "
+                             "the attention-guided mask needs the same number")
+        return R, (R != H or R != W)
+
     def n_visible(self, P):
         return P - int(P * self.mask_ratio)                      # run_stage1.py:380
 
@@ -345,19 +370,26 @@ class Stage1Engine:
         grads_ready: event after which the gradient arena may be written (its fill runs on a side stream, _step_body_dev)."""
         core, teacher = self.core, self.teacher
         B = videos.shape[0]
+        H_, W_ = videos.shape[2:4] if videos.dtype == U8 else videos.shape[3:5]
+        R, resize = self.teacher_view(H_, W_)
+        share = self.share_patches and not resize
         patches = None
         patches_s = None
         if videos.dtype == U8:
             # decoded frames uint8 [B,T,H,W,3]: normalise + patchify in one pass (SURVEY.md §8 row f2); the fp32 clip the
             # reference materialises never exists — `videos` below is a zero-stride shape carrier
-            _, T_, H_, W_, _c = videos.shape
-            ks, tub = teacher.kernel_size, self.student.encoder.patch_embed.tubelet_size
-            n_tok = lambda k: B * (T_ // k) * (H_ // 16) * (W_ // 16)
-            patches = ops.patchify_u8(videos, torch.empty(n_tok(ks), 3 * ks * 256, device=videos.device, dtype=BF16), ks)
-            patches_s = patches if self.share_patches else ops.patchify_u8(
-                videos, torch.empty(n_tok(tub), 3 * tub * 256, device=videos.device, dtype=BF16), tub)
+            T_ = videos.shape[1]
+            ks, tub, p = teacher.kernel_size, self.student.encoder.patch_embed.tubelet_size, teacher.patch_size
+            if p == 16 and not resize:
+                n_tok = lambda k: B * (T_ // k) * (H_ // 16) * (W_ // 16)
+                patches = ops.patchify_u8(videos, torch.empty(n_tok(ks), 3 * ks * 256, device=videos.device, dtype=BF16), ks)
+            else:
+                patches = ops.resize_patchify(videos, torch.empty(B * (T_ // ks) * (R // p) ** 2, teacher.k_pad, device=videos.device,
+                                                                  dtype=BF16), R, p, ks)
+            patches_s = patches if share else ops.patchify_u8(
+                videos, torch.empty(B * (T_ // tub) * (H_ // 16) * (W_ // 16), 3 * tub * 256, device=videos.device, dtype=BF16), tub)
             videos = torch.empty(1, device=videos.device, dtype=F32).expand(B, 3, T_, H_, W_)
-        elif self.share_patches:
+        elif share:
             ks = teacher.kernel_size
             n_tok = B * (videos.shape[2] // ks) * (videos.shape[3] // 16) * (videos.shape[4] // 16)
             patches = torch.empty(n_tok, 3 * ks * 256, device=videos.device, dtype=BF16)
@@ -376,7 +408,7 @@ class Stage1Engine:
                             n_vis)
             return sel["tea_rows"].view(-1)
 
-        layers, attn, _ = teacher.forward_features(videos, patches, select=select)
+        layers, attn, _ = teacher.forward_features(videos, patches, select=select, resolution=R)
         if not sel:                                                               # teacher without return_attn / last-layer tap
             select(attn)
         frames, P = attn.shape
@@ -388,7 +420,7 @@ class Stage1Engine:
         loss_clips = self._loss_clips(B)
         self.loss.zero_()
         if patches_s is None:
-            patches_s = patches if self.share_patches else None
+            patches_s = patches if share else None
         kind = clip_loss_type or self.clip_loss_type
         if kind == "l2":
             # shipped config: the loss and its gradient are fused into the decoder-tail kernels

@@ -5,6 +5,9 @@ What changes versus the reference loop body: no per-step `.item()` / `torch.cuda
 458) — the loss and grad-norm are accumulated on the device and read once per `log_freq` steps and at the end;
 non-finite loss is still fatal (run_stage1.py:447-449) but is checked at those read points.
 Batches are `(videos, mask_placeholder, labels[, noise])`; without `noise` the Exp(1) draw is made on the device.
+`clip_input_resolution` is the side the teacher sees (run_stage1.py:360-377: the teacher's copy of the clip is resized to it,
+bicubic, when it differs from the clip's); None (the default here) means the teacher's own input_resolution, the only side its
+positional embedding fits.  A CLIP ViT-L/14 teacher behind a 16-pixel student at 224 px needs 196.
 """
 import math
 import sys
@@ -45,7 +48,7 @@ def _engine_for(model, teacher_model, mask_ratio, optimizer, use_graph=False):
 def train_one_epoch(model: torch.nn.Module, data_loader: Iterable, data_loader_train_target: Optional[Iterable] = None,
                     optimizer=None, device=None, epoch: int = 0, loss_scaler=None, max_norm: float = 0, log_writer=None,
                     lr_scheduler=None, start_steps=0, lr_schedule_values=None, wd_schedule_values=None, src_classifier=None,
-                    teacher_model=None, clip_input_resolution=224, clip_loss_type="l2", clip_loss_ratio=0.5,
+                    teacher_model=None, clip_input_resolution=None, clip_loss_type="l2", clip_loss_ratio=0.5,
                     mask_type="attention", mask_ratio=0.0, use_wandb=False, args=None):
     if mask_type != "attention":
         # the reference itself only runs with mask_type='attention': run_stage1.py:378 reads `attn`, which the other mask
@@ -61,6 +64,7 @@ def train_one_epoch(model: torch.nn.Module, data_loader: Iterable, data_loader_t
     model.train()
     eng = _engine_for(model, teacher_model, mask_ratio, optimizer, use_graph=bool(getattr(args, "use_cuda_graph", False)))
     eng.clip_loss_type = clip_loss_type
+    eng.teacher_resolution = eng.teacher.input_resolution if clip_input_resolution is None else int(clip_input_resolution)
     eng.clip_loss_data = clip_loss_data
     eng.max_norm = float(max_norm) if max_norm else None       # loss_scaler(..., clip_grad=max_norm, ...), run_stage1.py:451-455
     opt = eng.optimizer
@@ -148,7 +152,8 @@ def train_one_epoch(model: torch.nn.Module, data_loader: Iterable, data_loader_t
             # fp32 clips are [B,3,T,H,W]; decoded uint8 frames are [B,T,H,W,3]
             T_, H_, W_ = (videos.shape[1:4] if videos.dtype == torch.uint8 else videos.shape[2:5])
             frames = videos.shape[0] * (T_ // eng.teacher.kernel_size)
-            noise = torch.empty(frames, (H_ // 16) * (W_ // 16), device=dev).exponential_(1)
+            R, _ = eng.teacher_view(H_, W_)                                    # the mask is drawn over the teacher's patch grid
+            noise = torch.empty(frames, (R // eng.teacher.patch_size) ** 2, device=dev).exponential_(1)
         staged = fetch(nxt) if nxt is not None else None                       # overlaps with this step's compute
         loss = eng.step(videos, noise)
         done = torch.cuda.Event()

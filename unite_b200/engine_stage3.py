@@ -37,6 +37,10 @@ class Stage3Engine:
         exchange and AdamW: ~900 launches) is captured in a CUDA graph and replayed (engine.GraphReplay); nothing in it reads a
         device value on the host, DropPath factors and optimizer scalars come from device memory."""
         from .engine import GraphReplay
+        if teacher.patch_size != 16:
+            # the zero-shot head stands the teacher's CLS embedding in for OpenAI CLIP's image tower against a 512-wide text
+            # matrix; which stand-in a ViT-L/14 teacher should provide is not settled
+            raise NotImplementedError(f"stage 3 runs a 16-pixel (clip_b16) teacher; got patch size {teacher.patch_size}")
         self.use_graph = use_graph
         self.graphs = GraphReplay()
         self.student, self.teacher = student, teacher

@@ -298,6 +298,35 @@ def patchify_u8(x, out, tubelet, mean=IMAGENET_MEAN, std=IMAGENET_STD):
     return out
 
 
+def padded_k(features: int) -> int:
+    """Row pitch of resize_patchify's output: the im2col width rounded up to 64 elements (one GEMM K block; also keeps the
+    rows 16-byte aligned for TMA, which 3*14*14 = 588 bf16 would not be)."""
+    return (features + 63) // 64 * 64
+
+
+@_instrument("resize_patchify", 1)
+def resize_patchify(x, out, resolution, patch, tubelet, mean=IMAGENET_MEAN, std=IMAGENET_STD):
+    """Teacher im2col rows of a clip seen at `resolution` x `resolution` with `patch`-pixel patches.
+    x: fp32 clip [B,3,T,H,W], or decoded uint8 frames [B,T,H,W,3] (normalised with mean / std before the resize).
+    out: bf16 [B*(T/tubelet)*(resolution/patch)^2, ld], ld >= 3*tubelet*patch^2 (columns past that are written as zeros).
+    When resolution != H or W the clip is resized as F.interpolate(mode="bicubic", align_corners=False) does."""
+    if x.dtype == U8:
+        if x.dim() != 5 or x.shape[-1] != 3:
+            raise _cabi.UBError(f"resize_patchify: uint8 frames [B,T,H,W,3] expected, got {tuple(x.shape)}")
+        B, T, H, W, _ = x.shape
+    else:
+        if x.dim() != 5 or x.shape[1] != 3:
+            raise _cabi.UBError(f"resize_patchify: fp32 clip [B,3,T,H,W] expected, got {tuple(x.shape)}")
+        B, _, T, H, W = x.shape
+    n_tok = B * (T // tubelet) * (resolution // patch) ** 2
+    if out.dim() != 2 or out.shape[0] != n_tok:
+        raise _cabi.UBError(f"resize_patchify: out must be [{n_tok}, ld], got {tuple(out.shape)}")
+    m3, s3 = (C.c_float * 3)(*mean), (C.c_float * 3)(*std)
+    check(lib.ub_resize_patchify(_p(x, U8 if x.dtype == U8 else F32, "videos"), int(x.dtype == U8), m3, s3, _p(out, BF16, "patches"),
+                                 out.shape[1], B, T, H, W, resolution, patch, tubelet, _stream()), "ub_resize_patchify")
+    return out
+
+
 @_instrument("mask_select", 1)
 def mask_select(attn, q, mask, vis_idx, tea_rows, T, k, n_vis):
     frames, P = attn.shape
