@@ -51,6 +51,8 @@ def test_sass_uses_blackwell_tensor_and_tma_paths():
         import pytest
         pytest.skip("cuobjdump not available")
     assert "UTCHMMA" in r.stdout and "UTMALDG" in r.stdout and "LDTM" in r.stdout
+    # every tensor-core product is a tcgen05 MMA (UTCHMMA): no kernel uses the older warp-level mma.sync (plain HMMA)
+    assert not re.search(r"(?<!UTC)HMMA\.", r.stdout)
 
 
 def test_product_package_never_imports_the_oracle():

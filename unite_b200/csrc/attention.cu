@@ -1,236 +1,22 @@
-// Fused (flash-style) multi-head self-attention, head_dim 64, non-causal, no dropout — forward, backward
-// and the teacher's last-layer CLS-row attention map.
+// Multi-head self-attention (head_dim 64, non-causal, no dropout): the C-ABI entry points, the backward's D pre-pass and
+// the teacher's last-layer CLS-row attention map.
 //
 // Replaces   student  modeling_finetune.py:110-116 (q*scale, q@k^T, softmax, @v) and its autograd backward,
 //            teacher  clip.py:40-52 (nn.MultiheadAttention core), clip.py:95-96,183 (head-averaged CLS row).
 // Layout     qkv bf16 [n_seq*S, 3*H*64]: per token row q|k|v, each H heads x 64 (what both the packed in_proj
 //            of nn.MultiheadAttention and `qkv.reshape(B,N,3,H,-1)` produce); o bf16 [n_seq*S, H*64].
-// The S x S score matrix never reaches HBM (the reference materialises [B,H,S,S] and keeps it for backward):
-// forward keeps only the per-row log-sum-exp, backward recomputes P tile by tile.
-// Tensor-core path here is warp-level mma.sync (bf16, fp32 accumulate) with ldmatrix from XOR-swizzled smem and
-// cp.async double buffering; attention is ~5% of the step FLOPs (SURVEY.md §2.3), the tcgen05 budget went
-// to the GEMMs first.
+// ub_attn_fwd / ub_attn_bwd pick one of four tcgen05 / TMEM kernels by S and by whether an LSE is kept: attention_tc.cu,
+// attention_fwd_lse_tc.cu and attention_bwd_tc.cu for short sequences, attention_long_tc.cu for every longer one.  None of
+// them writes the S x S score matrix to HBM: the forward keeps only the per-row log-sum-exp, the backward recomputes P.
 #include "common.cuh"
-#include <cstdlib>
 #include "../../include/unite_b200.h"
 
 namespace ub {
 
 constexpr int HD = 64;          // head dim
-constexpr int TQ = 64;          // rows per tile
-constexpr float LOG2E = 1.4426950408889634f;
-
-UB_DEVINL uint32_t sw_off(int r, int c) { return (uint32_t)(r * 128 + ((c ^ (r & 7)) << 4)); }
-
-UB_DEVINL void ldsm_x4(uint32_t addr, uint32_t (&r)[4]) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0, %1, %2, %3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
-               : "r"(addr));
-}
-UB_DEVINL void ldsm_x4_t(uint32_t addr, uint32_t (&r)[4]) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0, %1, %2, %3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
-               : "r"(addr));
-}
-UB_DEVINL void mma16816(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, "
-      "{%0, %1, %2, %3};"
-      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-UB_DEVINL void cp_async16(uint32_t saddr, const void* g, bool pred) {
-  const int sz = pred ? 16 : 0;
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(saddr), "l"(g), "r"(sz) : "memory");
-}
-UB_DEVINL void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-UB_DEVINL void cp_async_wait() {
-  asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
-}
-
-// Load a [64 rows][64 bf16] tile (rows row0.. of a sequence, zero-filled past `S`) into swizzled smem.
-// `g` points at (sequence row 0, first column of the head slice); ld in elements.  128 threads.
-UB_DEVINL void load_tile(uint32_t s_base, const bf16* g, int64_t ld, int row0, int S) {
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int idx = threadIdx.x + i * 128;
-    const int r = idx >> 3, c = idx & 7;
-    const bool ok = (row0 + r) < S;
-    const bf16* src = g + (int64_t)(ok ? row0 + r : 0) * ld + c * 8;
-    cp_async16(s_base + sw_off(r, c), src, ok);
-  }
-}
-// A-operand fragment: 16 rows starting at row0, k-step ks of a swizzled tile
-UB_DEVINL void frag_a(uint32_t s_base, int row0, int ks, int lane, uint32_t (&a)[4]) {
-  ldsm_x4(s_base + sw_off(row0 + (lane & 15), 2 * ks + (lane >> 4)), a);
-}
-// B-operand fragments for two n-tiles (16 tile rows n0..n0+15 are the n index), k-step ks:  b[0],b[1] | b[2],b[3]
-UB_DEVINL void frag_b_rows(uint32_t s_base, int n0, int ks, int lane, uint32_t (&b)[4]) {
-  ldsm_x4(s_base + sw_off(n0 + (lane & 7) + ((lane >> 4) << 3), 2 * ks + ((lane >> 3) & 1)), b);
-}
-// B-operand fragments when tile rows are the k index (16 rows k0..) and columns the n index (n-pair np)
-UB_DEVINL void frag_b_cols(uint32_t s_base, int k0, int np, int lane, uint32_t (&b)[4]) {
-  ldsm_x4_t(s_base + sw_off(k0 + (lane & 7) + (((lane >> 3) & 1) << 3), 2 * np + (lane >> 4)), b);
-}
-
-// Write a warp's 16x64 fp32 accumulator tile (mma C layout) as bf16 rows to global through its own smem rows.
-// `tile_row0` = sequence row of the tile's row 0; rows >= S are not written.
-UB_DEVINL void store_acc_bf16(uint8_t* s_tile, int warp_row0, int lane, const float (&acc)[8][4], float mul, bf16* g,
-                              int64_t ld, int tile_row0, int S) {
-  const int g4 = lane >> 2, t4 = lane & 3;
-#pragma unroll
-  for (int nt = 0; nt < 8; ++nt) {
-    const uint32_t lo = pack_bf16x2(acc[nt][0] * mul, acc[nt][1] * mul);
-    const uint32_t hi = pack_bf16x2(acc[nt][2] * mul, acc[nt][3] * mul);
-    *reinterpret_cast<uint32_t*>(s_tile + sw_off(warp_row0 + g4, nt) + t4 * 4) = lo;
-    *reinterpret_cast<uint32_t*>(s_tile + sw_off(warp_row0 + g4 + 8, nt) + t4 * 4) = hi;
-  }
-  __syncwarp();
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int idx = lane + i * 32;
-    const int r = idx >> 3, c = idx & 7;
-    const int grow = tile_row0 + warp_row0 + r;
-    if (grow < S) {
-      const uint4 v = *reinterpret_cast<const uint4*>(s_tile + sw_off(warp_row0 + r, c));
-      *reinterpret_cast<uint4*>(g + (int64_t)grow * ld + c * 8) = v;
-    }
-  }
-}
 
 // ------------------------------------------------------------------------------------------------
-// forward
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) attn_fwd_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ o,
-                                                       float* __restrict__ lse, int S, int H, float scale) {
-  pdl_grid_sync();
-  __shared__ __align__(1024) uint8_t sQ[TQ * 128];
-  __shared__ __align__(1024) uint8_t sK[2][TQ * 128];
-  __shared__ __align__(1024) uint8_t sV[2][TQ * 128];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int q0 = blockIdx.x * TQ, h = blockIdx.y, seq = blockIdx.z;
-  const int64_t ld = 3 * (int64_t)H * HD;
-  const bf16* base = qkv + (int64_t)seq * S * ld;
-  const bf16* gq = base + h * HD;
-  const bf16* gk = base + (H + h) * HD;
-  const bf16* gv = base + (2 * H + h) * HD;
-  const uint32_t sQa = smem_u32(sQ), sKa = smem_u32(sK[0]), sVa = smem_u32(sV[0]);
-  const int nkv = (S + TQ - 1) / TQ;
-
-  load_tile(sQa, gq, ld, q0, S);
-  load_tile(sKa, gk, ld, 0, S);
-  load_tile(sVa, gv, ld, 0, S);
-  cp_async_commit();
-
-  const int wrow0 = warp * 16;
-  const bool warp_active = (q0 + wrow0) < S;
-  const float sl2 = scale * LOG2E;
-  uint32_t qf[4][4];
-  float oacc[8][4];
-#pragma unroll
-  for (int i = 0; i < 8; ++i)
-#pragma unroll
-    for (int j = 0; j < 4; ++j) oacc[i][j] = 0.f;
-  float m0 = -INFINITY, m1 = -INFINITY, l0 = 0.f, l1 = 0.f;
-
-  for (int j = 0; j < nkv; ++j) {
-    cp_async_wait<0>();
-    __syncthreads();
-    if (j + 1 < nkv) {
-      load_tile(sKa + ((j + 1) & 1) * TQ * 128, gk, ld, (j + 1) * TQ, S);
-      load_tile(sVa + ((j + 1) & 1) * TQ * 128, gv, ld, (j + 1) * TQ, S);
-      cp_async_commit();
-    }
-    if (!warp_active) continue;
-    if (j == 0) {
-#pragma unroll
-      for (int ks = 0; ks < 4; ++ks) frag_a(sQa, wrow0, ks, lane, qf[ks]);
-    }
-    const uint32_t kb = sKa + (j & 1) * TQ * 128, vb = sVa + (j & 1) * TQ * 128;
-    float s[8][4];
-#pragma unroll
-    for (int i = 0; i < 8; ++i)
-#pragma unroll
-      for (int jj = 0; jj < 4; ++jj) s[i][jj] = 0.f;
-#pragma unroll
-    for (int ks = 0; ks < 4; ++ks) {
-#pragma unroll
-      for (int np = 0; np < 4; ++np) {
-        uint32_t b[4];
-        frag_b_rows(kb, np * 16, ks, lane, b);
-        mma16816(s[2 * np], qf[ks], b[0], b[1]);
-        mma16816(s[2 * np + 1], qf[ks], b[2], b[3]);
-      }
-    }
-    // mask keys past the end of the sequence (only the last tile can have any)
-    const int kbase = j * TQ + (lane & 3) * 2;
-    if (j * TQ + TQ > S) {
-#pragma unroll
-      for (int nt = 0; nt < 8; ++nt) {
-        const int key = kbase + nt * 8;
-        if (key >= S) { s[nt][0] = -INFINITY; s[nt][2] = -INFINITY; }
-        if (key + 1 >= S) { s[nt][1] = -INFINITY; s[nt][3] = -INFINITY; }
-      }
-    }
-    float mx0 = m0, mx1 = m1;
-#pragma unroll
-    for (int nt = 0; nt < 8; ++nt) {
-      mx0 = fmaxf(mx0, fmaxf(s[nt][0], s[nt][1]));
-      mx1 = fmaxf(mx1, fmaxf(s[nt][2], s[nt][3]));
-    }
-    mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 1));
-    mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 2));
-    mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 1));
-    mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 2));
-    const float c0 = exp2f((m0 - mx0) * sl2), c1 = exp2f((m1 - mx1) * sl2);
-    m0 = mx0; m1 = mx1;
-    const float ms0 = mx0 * sl2, ms1 = mx1 * sl2;
-    float rs0 = 0.f, rs1 = 0.f;
-    uint32_t pf[4][4];
-#pragma unroll
-    for (int nt = 0; nt < 8; ++nt) {
-      const float p0 = exp2f(s[nt][0] * sl2 - ms0), p1 = exp2f(s[nt][1] * sl2 - ms0);
-      const float p2 = exp2f(s[nt][2] * sl2 - ms1), p3 = exp2f(s[nt][3] * sl2 - ms1);
-      rs0 += p0 + p1; rs1 += p2 + p3;
-      pf[nt >> 1][(nt & 1) * 2 + 0] = pack_bf16x2(p0, p1);
-      pf[nt >> 1][(nt & 1) * 2 + 1] = pack_bf16x2(p2, p3);
-    }
-    l0 = l0 * c0 + rs0; l1 = l1 * c1 + rs1;
-#pragma unroll
-    for (int nt = 0; nt < 8; ++nt) {
-      oacc[nt][0] *= c0; oacc[nt][1] *= c0; oacc[nt][2] *= c1; oacc[nt][3] *= c1;
-    }
-#pragma unroll
-    for (int ks = 0; ks < 4; ++ks) {
-#pragma unroll
-      for (int np = 0; np < 4; ++np) {
-        uint32_t b[4];
-        frag_b_cols(vb, ks * 16, np, lane, b);
-        mma16816(oacc[2 * np], pf[ks], b[0], b[1]);
-        mma16816(oacc[2 * np + 1], pf[ks], b[2], b[3]);
-      }
-    }
-  }
-  if (!warp_active) return;
-  l0 += __shfl_xor_sync(0xffffffffu, l0, 1); l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
-  l1 += __shfl_xor_sync(0xffffffffu, l1, 1); l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
-  const float inv0 = 1.f / l0, inv1 = 1.f / l1;
-#pragma unroll
-  for (int nt = 0; nt < 8; ++nt) {
-    oacc[nt][0] *= inv0; oacc[nt][1] *= inv0; oacc[nt][2] *= inv1; oacc[nt][3] *= inv1;
-  }
-  store_acc_bf16(sQ, wrow0, lane, oacc, 1.0f, o + (int64_t)seq * S * H * HD + h * HD, (int64_t)H * HD, q0, S);
-  if (lse != nullptr && (lane & 3) == 0) {
-    const int r0 = q0 + wrow0 + (lane >> 2);
-    float* L = lse + ((int64_t)seq * H + h) * S;
-    if (r0 < S) L[r0] = m0 * scale + logf(l0);
-    if (r0 + 8 < S) L[r0 + 8] = m1 * scale + logf(l1);
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// backward, part 0:  D[seq,h,row] = sum_d dO * O
+// backward pre-pass:  D[seq,h,row] = sum_d dO * O
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) attn_bwd_prep_kernel(const bf16* __restrict__ o, const bf16* __restrict__ d_o,
                                                             float* __restrict__ D, long n_chunks, int S, int H) {
@@ -257,239 +43,6 @@ __global__ void __launch_bounds__(256) attn_bwd_prep_kernel(const bf16* __restri
     const int r = (int)(row % S);
     D[(seq * H + h) * S + r] = v;
   }
-}
-
-// ------------------------------------------------------------------------------------------------
-// backward, part 1:  dK, dV   (CTA = 64 keys of one (seq, head); loops over query tiles)
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) attn_bwd_dkv_kernel(const bf16* __restrict__ qkv, const bf16* __restrict__ d_o,
-                                                           const float* __restrict__ lse, const float* __restrict__ Dv,
-                                                           bf16* __restrict__ dqkv, int S, int H, float scale) {
-  pdl_grid_sync();
-  extern __shared__ __align__(1024) uint8_t smem_dkv[];
-  uint8_t* sK = smem_dkv;                      // 8 KB (reused to stage dK)
-  uint8_t* sV = sK + TQ * 128;                 // 8 KB (reused to stage dV)
-  uint8_t* sQ = sV + TQ * 128;                 // 2 x 8 KB
-  uint8_t* sdO = sQ + 2 * TQ * 128;            // 2 x 8 KB
-  float* sL = reinterpret_cast<float*>(sdO + 2 * TQ * 128);  // 2 x 64
-  float* sD = sL + 2 * TQ;                                    // 2 x 64
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int k0 = blockIdx.x * TQ, h = blockIdx.y, seq = blockIdx.z;
-  const int64_t ld = 3 * (int64_t)H * HD, ldo = (int64_t)H * HD;
-  const bf16* base = qkv + (int64_t)seq * S * ld;
-  const bf16* gq = base + h * HD;
-  const bf16* gk = base + (H + h) * HD;
-  const bf16* gv = base + (2 * H + h) * HD;
-  const bf16* gdo = d_o + (int64_t)seq * S * ldo + h * HD;
-  const float* gL = lse + ((int64_t)seq * H + h) * S;
-  const float* gD = Dv + ((int64_t)seq * H + h) * S;
-  const uint32_t sKa = smem_u32(sK), sVa = smem_u32(sV), sQa = smem_u32(sQ), sdOa = smem_u32(sdO);
-  const int nq = (S + TQ - 1) / TQ;
-
-  auto load_q_tile = [&](int t) {
-    const int buf = t & 1;
-    load_tile(sQa + buf * TQ * 128, gq, ld, t * TQ, S);
-    load_tile(sdOa + buf * TQ * 128, gdo, ldo, t * TQ, S);
-    if (threadIdx.x < TQ) {
-      const int r = t * TQ + threadIdx.x;
-      sL[buf * TQ + threadIdx.x] = r < S ? gL[r] * LOG2E : INFINITY;   // +inf -> P = 0 for padded queries
-      sD[buf * TQ + threadIdx.x] = r < S ? gD[r] : 0.f;
-    }
-  };
-  load_tile(sKa, gk, ld, k0, S);
-  load_tile(sVa, gv, ld, k0, S);
-  load_q_tile(0);
-  cp_async_commit();
-
-  const int wrow0 = warp * 16;
-  const float sl2 = scale * LOG2E;
-  uint32_t kf[4][4], vf[4][4];
-  float dk[8][4], dv[8][4];
-#pragma unroll
-  for (int i = 0; i < 8; ++i)
-#pragma unroll
-    for (int j = 0; j < 4; ++j) { dk[i][j] = 0.f; dv[i][j] = 0.f; }
-
-  for (int t = 0; t < nq; ++t) {
-    cp_async_wait<0>();
-    __syncthreads();
-    if (t + 1 < nq) {
-      load_q_tile(t + 1);
-      cp_async_commit();
-    }
-    if (t == 0) {
-#pragma unroll
-      for (int ks = 0; ks < 4; ++ks) {
-        frag_a(sKa, wrow0, ks, lane, kf[ks]);
-        frag_a(sVa, wrow0, ks, lane, vf[ks]);
-      }
-    }
-    const uint32_t qb = sQa + (t & 1) * TQ * 128, dob = sdOa + (t & 1) * TQ * 128;
-    const float* L = sL + (t & 1) * TQ;
-    const float* Dq = sD + (t & 1) * TQ;
-#pragma unroll
-    for (int half = 0; half < 2; ++half) {
-      const int qh = half * 32;
-      float st[4][4], dp[4][4];
-#pragma unroll
-      for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) { st[i][j] = 0.f; dp[i][j] = 0.f; }
-      // S^T = K_w Q^T   and   dP^T = V_w dO^T       (16 keys x 32 queries)
-#pragma unroll
-      for (int ks = 0; ks < 4; ++ks) {
-#pragma unroll
-        for (int np = 0; np < 2; ++np) {
-          uint32_t b[4];
-          frag_b_rows(qb, qh + np * 16, ks, lane, b);
-          mma16816(st[2 * np], kf[ks], b[0], b[1]);
-          mma16816(st[2 * np + 1], kf[ks], b[2], b[3]);
-          frag_b_rows(dob, qh + np * 16, ks, lane, b);
-          mma16816(dp[2 * np], vf[ks], b[0], b[1]);
-          mma16816(dp[2 * np + 1], vf[ks], b[2], b[3]);
-        }
-      }
-      uint32_t pf[2][4], dsf[2][4];
-#pragma unroll
-      for (int nt = 0; nt < 4; ++nt) {
-        const int qc = qh + nt * 8 + (lane & 3) * 2;
-        const float L0 = L[qc], L1 = L[qc + 1], D0 = Dq[qc], D1 = Dq[qc + 1];
-        const float p0 = exp2f(st[nt][0] * sl2 - L0), p1 = exp2f(st[nt][1] * sl2 - L1);
-        const float p2 = exp2f(st[nt][2] * sl2 - L0), p3 = exp2f(st[nt][3] * sl2 - L1);
-        pf[nt >> 1][(nt & 1) * 2 + 0] = pack_bf16x2(p0, p1);
-        pf[nt >> 1][(nt & 1) * 2 + 1] = pack_bf16x2(p2, p3);
-        dsf[nt >> 1][(nt & 1) * 2 + 0] = pack_bf16x2(p0 * (dp[nt][0] - D0), p1 * (dp[nt][1] - D1));
-        dsf[nt >> 1][(nt & 1) * 2 + 1] = pack_bf16x2(p2 * (dp[nt][2] - D0), p3 * (dp[nt][3] - D1));
-      }
-      // dV += P^T dO ;  dK += dS^T Q        (contraction over the 32 queries)
-#pragma unroll
-      for (int ks = 0; ks < 2; ++ks) {
-#pragma unroll
-        for (int np = 0; np < 4; ++np) {
-          uint32_t b[4];
-          frag_b_cols(dob, qh + ks * 16, np, lane, b);
-          mma16816(dv[2 * np], pf[ks], b[0], b[1]);
-          mma16816(dv[2 * np + 1], pf[ks], b[2], b[3]);
-          frag_b_cols(qb, qh + ks * 16, np, lane, b);
-          mma16816(dk[2 * np], dsf[ks], b[0], b[1]);
-          mma16816(dk[2 * np + 1], dsf[ks], b[2], b[3]);
-        }
-      }
-    }
-  }
-  // all K/V fragments were taken in iteration 0; each warp re-uses its own 16 rows of sK / sV as staging
-  bf16* gdk = dqkv + (int64_t)seq * S * ld + (H + h) * HD;
-  bf16* gdv = dqkv + (int64_t)seq * S * ld + (2 * H + h) * HD;
-  __syncwarp();
-  store_acc_bf16(sK, wrow0, lane, dk, scale, gdk, ld, k0, S);
-  store_acc_bf16(sV, wrow0, lane, dv, 1.0f, gdv, ld, k0, S);
-}
-
-// ------------------------------------------------------------------------------------------------
-// backward, part 2:  dQ   (CTA = 64 queries of one (seq, head); loops over key tiles)
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) attn_bwd_dq_kernel(const bf16* __restrict__ qkv, const bf16* __restrict__ d_o,
-                                                          const float* __restrict__ lse, const float* __restrict__ Dv,
-                                                          bf16* __restrict__ dqkv, int S, int H, float scale) {
-  pdl_grid_sync();
-  extern __shared__ __align__(1024) uint8_t smem_dq[];
-  uint8_t* sQ = smem_dq;                 // 8 KB (reused to stage dQ)
-  uint8_t* sdO = sQ + TQ * 128;          // 8 KB
-  uint8_t* sK = sdO + TQ * 128;          // 2 x 8 KB
-  uint8_t* sV = sK + 2 * TQ * 128;       // 2 x 8 KB
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int q0 = blockIdx.x * TQ, h = blockIdx.y, seq = blockIdx.z;
-  const int64_t ld = 3 * (int64_t)H * HD, ldo = (int64_t)H * HD;
-  const bf16* base = qkv + (int64_t)seq * S * ld;
-  const bf16* gq = base + h * HD;
-  const bf16* gk = base + (H + h) * HD;
-  const bf16* gv = base + (2 * H + h) * HD;
-  const bf16* gdo = d_o + (int64_t)seq * S * ldo + h * HD;
-  const uint32_t sQa = smem_u32(sQ), sdOa = smem_u32(sdO), sKa = smem_u32(sK), sVa = smem_u32(sV);
-  const int nkv = (S + TQ - 1) / TQ;
-
-  load_tile(sQa, gq, ld, q0, S);
-  load_tile(sdOa, gdo, ldo, q0, S);
-  load_tile(sKa, gk, ld, 0, S);
-  load_tile(sVa, gv, ld, 0, S);
-  cp_async_commit();
-
-  const int wrow0 = warp * 16;
-  const bool warp_active = (q0 + wrow0) < S;
-  const float sl2 = scale * LOG2E;
-  const int r0 = q0 + wrow0 + (lane >> 2);
-  const float* gL = lse + ((int64_t)seq * H + h) * S;
-  const float* gD = Dv + ((int64_t)seq * H + h) * S;
-  const float L0 = r0 < S ? gL[r0] * LOG2E : INFINITY, L1 = r0 + 8 < S ? gL[r0 + 8] * LOG2E : INFINITY;
-  const float D0 = r0 < S ? gD[r0] : 0.f, D1 = r0 + 8 < S ? gD[r0 + 8] : 0.f;
-  uint32_t qf[4][4], dof[4][4];
-  float dq[8][4];
-#pragma unroll
-  for (int i = 0; i < 8; ++i)
-#pragma unroll
-    for (int j = 0; j < 4; ++j) dq[i][j] = 0.f;
-
-  for (int j = 0; j < nkv; ++j) {
-    cp_async_wait<0>();
-    __syncthreads();
-    if (j + 1 < nkv) {
-      load_tile(sKa + ((j + 1) & 1) * TQ * 128, gk, ld, (j + 1) * TQ, S);
-      load_tile(sVa + ((j + 1) & 1) * TQ * 128, gv, ld, (j + 1) * TQ, S);
-      cp_async_commit();
-    }
-    if (!warp_active) continue;
-    if (j == 0) {
-#pragma unroll
-      for (int ks = 0; ks < 4; ++ks) {
-        frag_a(sQa, wrow0, ks, lane, qf[ks]);
-        frag_a(sdOa, wrow0, ks, lane, dof[ks]);
-      }
-    }
-    const uint32_t kb = sKa + (j & 1) * TQ * 128, vb = sVa + (j & 1) * TQ * 128;
-    float s[8][4], dp[8][4];
-#pragma unroll
-    for (int i = 0; i < 8; ++i)
-#pragma unroll
-      for (int jj = 0; jj < 4; ++jj) { s[i][jj] = 0.f; dp[i][jj] = 0.f; }
-#pragma unroll
-    for (int ks = 0; ks < 4; ++ks) {
-#pragma unroll
-      for (int np = 0; np < 4; ++np) {
-        uint32_t b[4];
-        frag_b_rows(kb, np * 16, ks, lane, b);
-        mma16816(s[2 * np], qf[ks], b[0], b[1]);
-        mma16816(s[2 * np + 1], qf[ks], b[2], b[3]);
-        frag_b_rows(vb, np * 16, ks, lane, b);
-        mma16816(dp[2 * np], dof[ks], b[0], b[1]);
-        mma16816(dp[2 * np + 1], dof[ks], b[2], b[3]);
-      }
-    }
-    uint32_t dsf[4][4];
-    const int kbase = j * TQ + (lane & 3) * 2;
-#pragma unroll
-    for (int nt = 0; nt < 8; ++nt) {
-      const int key = kbase + nt * 8;
-      float p0 = exp2f(s[nt][0] * sl2 - L0), p1 = exp2f(s[nt][1] * sl2 - L0);
-      float p2 = exp2f(s[nt][2] * sl2 - L1), p3 = exp2f(s[nt][3] * sl2 - L1);
-      if (key >= S) { p0 = 0.f; p2 = 0.f; }
-      if (key + 1 >= S) { p1 = 0.f; p3 = 0.f; }
-      dsf[nt >> 1][(nt & 1) * 2 + 0] = pack_bf16x2(p0 * (dp[nt][0] - D0), p1 * (dp[nt][1] - D0));
-      dsf[nt >> 1][(nt & 1) * 2 + 1] = pack_bf16x2(p2 * (dp[nt][2] - D1), p3 * (dp[nt][3] - D1));
-    }
-#pragma unroll
-    for (int ks = 0; ks < 4; ++ks) {
-#pragma unroll
-      for (int np = 0; np < 4; ++np) {
-        uint32_t b[4];
-        frag_b_cols(kb, ks * 16, np, lane, b);
-        mma16816(dq[2 * np], dsf[ks], b[0], b[1]);
-        mma16816(dq[2 * np + 1], dsf[ks], b[2], b[3]);
-      }
-    }
-  }
-  if (!warp_active) return;
-  __syncwarp();
-  store_acc_bf16(sQ, wrow0, lane, dq, scale, dqkv + (int64_t)seq * S * ld + h * HD, ld, q0, S);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -563,15 +116,6 @@ int launch_attn_bwd_tc(const void* qkv, const void* d_o, const float* lse, const
 int launch_attn_fwd_long_tc(const void* qkv, void* o, float* lse, int n_seq, int S, int H, float scale, cudaStream_t stream);
 int launch_attn_bwd_long_tc(const void* qkv, const void* d_o, const float* lse, const float* Dv, void* dqkv, float* dbias, int n_seq, int S,
                             int H, float scale, cudaStream_t stream);
-// UB_ATTN_LONG_TC=0: fall back to the mma.sync kernels below for S beyond the short-sequence tcgen05 kernels (debugging only)
-static bool use_long_tc() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("UB_ATTN_LONG_TC");
-    v = e ? atoi(e) : 1;
-  }
-  return v != 0;
-}
 }
 using namespace ub;
 
@@ -580,25 +124,12 @@ extern "C" int ub_attn_fwd(const void* qkv, void* o, float* lse, int n_seq, int 
   UB_REQUIRE(n_seq > 0 && S > 0 && H > 0, "attn_fwd: bad shape n_seq=%d S=%d H=%d", n_seq, S, H);
   UB_REQUIRE(n_seq <= 65535 && H <= 65535, "attn_fwd: grid too large");
   // inference over short sequences (the teacher's 197-token frames): tcgen05 / TMEM kernel
-  static int use_tc = -1;
-  if (use_tc < 0) {
-    const char* e = getenv("UB_ATTN_TC");
-    use_tc = e ? atoi(e) : 1;
-  }
-  if (use_tc && lse == nullptr && S <= 240) return   // (K and V for NK <= 240 padded keys fit the 227 KB smem budget twice)
+  if (lse == nullptr && S <= 240) return   // (K and V for NK <= 240 padded keys fit the 227 KB smem budget twice)
     launch_attn_fwd_tc(qkv, o, n_seq, S, H, scale, (cudaStream_t)stream);
   // training forward (LSE kept for the backward) over the student's <= 320 visible tokens: two-chunk tcgen05 kernel
-  static int use_tc_lse = -1;
-  if (use_tc_lse < 0) {
-    const char* e = getenv("UB_ATTN_FWD_LSE_TC");
-    use_tc_lse = e ? atoi(e) : 1;
-  }
-  if (use_tc_lse && lse != nullptr && S <= 320) return launch_attn_fwd_lse_tc(qkv, o, lse, n_seq, S, H, scale, (cudaStream_t)stream);
+  if (lse != nullptr && S <= 320) return launch_attn_fwd_lse_tc(qkv, o, lse, n_seq, S, H, scale, (cudaStream_t)stream);
   // everything longer (stage-2 / stage-3 all-token passes, S = 1568): streamed-KV tcgen05 kernel, with or without LSE
-  if (use_long_tc()) return launch_attn_fwd_long_tc(qkv, o, lse, n_seq, S, H, scale, (cudaStream_t)stream);
-  dim3 grid((S + TQ - 1) / TQ, H, n_seq);
-  UB_LAUNCH(attn_fwd_kernel, grid, 128, 0, (cudaStream_t)stream, (const bf16*)qkv, (bf16*)o, lse, S, H, scale);
-  return check_launch("attn_fwd_kernel");
+  return launch_attn_fwd_long_tc(qkv, o, lse, n_seq, S, H, scale, (cudaStream_t)stream);
 }
 
 extern "C" int ub_attn_bwd(const void* qkv, const void* o, const void* d_o, const float* lse, float* D_ws, void* dqkv, float* dbias,
@@ -613,30 +144,8 @@ extern "C" int ub_attn_bwd(const void* qkv, const void* o, const void* d_o, cons
     if (check_launch("attn_bwd_prep_kernel")) return 1;
   }
   // short sequences (the student's <= 320 visible tokens): single-pass tcgen05 / TMEM kernel
-  static int use_tc = -1;
-  if (use_tc < 0) {
-    const char* e = getenv("UB_ATTN_BWD_TC");
-    use_tc = e ? atoi(e) : 1;
-  }
-  if (use_tc && S <= 320) return launch_attn_bwd_tc(qkv, d_o, lse, D_ws, dqkv, dbias, n_seq, S, H, scale, st);
-  if (use_long_tc()) return launch_attn_bwd_long_tc(qkv, d_o, lse, D_ws, dqkv, dbias, n_seq, S, H, scale, st);
-  dim3 grid((S + TQ - 1) / TQ, H, n_seq);
-  constexpr int SMEM_DKV = 6 * TQ * 128 + 4 * TQ * 4;
-  constexpr int SMEM_DQ = 6 * TQ * 128;
-  static bool configured = false;
-  if (!configured) {
-    cudaError_t e1 = cudaFuncSetAttribute(attn_bwd_dkv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_DKV);
-    cudaError_t e2 = cudaFuncSetAttribute(attn_bwd_dq_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_DQ);
-    UB_REQUIRE(e1 == cudaSuccess && e2 == cudaSuccess, "attn_bwd: cudaFuncSetAttribute failed");
-    configured = true;
-  }
-  UB_LAUNCH(attn_bwd_dkv_kernel, grid, 128, SMEM_DKV, st, (const bf16*)qkv, (const bf16*)d_o, lse, D_ws, (bf16*)dqkv, S, H, scale);
-  if (check_launch("attn_bwd_dkv_kernel")) return 1;
-  UB_LAUNCH(attn_bwd_dq_kernel, grid, 128, SMEM_DQ, st, (const bf16*)qkv, (const bf16*)d_o, lse, D_ws, (bf16*)dqkv, S, H, scale);
-  if (check_launch("attn_bwd_dq_kernel")) return 1;
-  if (dbias != nullptr)        // the mma.sync fallback has no fused bias gradient: one column-sum pass over dqkv, key third skipped
-    return ub_colsum_bf16(dqkv, 3 * (int64_t)H * 64, dbias, n_seq * S, 3 * H * 64, H * 64, 2 * H * 64, stream);
-  return 0;
+  if (S <= 320) return launch_attn_bwd_tc(qkv, d_o, lse, D_ws, dqkv, dbias, n_seq, S, H, scale, st);
+  return launch_attn_bwd_long_tc(qkv, d_o, lse, D_ws, dqkv, dbias, n_seq, S, H, scale, st);
 }
 
 extern "C" int ub_cls_attn(const void* qkv, float* out, int n_seq, int S, int H, float scale, void* stream) {

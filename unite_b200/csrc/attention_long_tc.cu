@@ -320,19 +320,8 @@ attn_long_tc_kernel(const __grid_constant__ CUtensorMap tmStat, const __grid_con
         atomicAdd(bias_dst + 2 * lane + 1, c1);
       }
     };
-    // The TMEM read port (64 B/clk/SM) bounds every mode (4 B of scores per (query, key) pair forward, 8 B backward), with the
-    // MUFU (16 ex2/clk/SM) right behind it.  -DUB_AL_PINGPONG makes the score loads of the two warpgroups strictly alternate
-    // (named barriers 2 / 3); measured on B200 at S = 1568 it changes nothing (575 vs 584 us forward), so it is off: what
+    // The TMEM read port (64 B/clk/SM) bounds every mode (4 B of scores per (query, key) pair forward, 8 B backward); what
     // mattered was taking the score MMAs off each warpgroup's critical path (two score sets, issued one chunk ahead).
-    auto my_turn = [&]() {
-      if (g == 0) asm volatile("bar.sync 2, 256;" ::: "memory"); else asm volatile("bar.sync 3, 256;" ::: "memory");
-    };
-    auto pass_turn = [&]() {
-      if (g == 0) asm volatile("bar.arrive 3, 256;" ::: "memory"); else asm volatile("bar.arrive 2, 256;" ::: "memory");
-    };
-#ifdef UB_AL_PINGPONG
-    if (g == 1) asm volatile("bar.arrive 2, 256;" ::: "memory");      // warpgroup A goes first
-#endif
     uint32_t ci = 0;
     int ui = 0;
     for (int u = blockIdx.x; u < n_units; u += gridDim.x, ++ui) {
@@ -355,15 +344,9 @@ attn_long_tc_kernel(const __grid_constant__ CUtensorMap tmStat, const __grid_con
         if (MODE == AL_FWD) {
           const int kvalid = min(NC, p.S - c * NC);
           uint32_t sv[NC];
-#ifdef UB_AL_PINGPONG
-          my_turn();
-#endif
 #pragma unroll
           for (int q = 0; q < NC / 32; ++q) tmem_ld_32x32(t_set + q * 32, *reinterpret_cast<uint32_t(*)[32]>(&sv[q * 32]));
           tmem_ld_wait();
-#ifdef UB_AL_PINGPONG
-          pass_turn();
-#endif
           float m4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
           if (kvalid == NC) {
 #pragma unroll
@@ -422,15 +405,9 @@ attn_long_tc_kernel(const __grid_constant__ CUtensorMap tmStat, const __grid_con
           // set = {S [0,32) | dP [32,64)}; P / dS (bf16, 16 columns each) are written over the first half of S / dP
           uint32_t sv[32], dv[32];
           if (MODE == AL_DKV) mbar_wait(&ld_full[stage], (ci / NSTG) & 1u);
-#ifdef UB_AL_PINGPONG
-          my_turn();
-#endif
           tmem_ld_32x32(t_set, sv);
           tmem_ld_32x32(t_set + 32, dv);
           tmem_ld_wait();
-#ifdef UB_AL_PINGPONG
-          pass_turn();
-#endif
           uint32_t pk[16], dk[16];
           if (MODE == AL_DQ) {
             const int kvalid = min(NC, p.S - c * NC);
@@ -490,9 +467,6 @@ attn_long_tc_kernel(const __grid_constant__ CUtensorMap tmStat, const __grid_con
       if (lane == 0) mbar_arrive(&acc_free[g]);
     }
     if (lane == 0) tma_store_wait_read<0>();
-#ifdef UB_AL_PINGPONG
-    if (g == 0) my_turn();                      // takes warpgroup B's last hand-over
-#endif
   }
   tc_fence_before();
   __syncthreads();

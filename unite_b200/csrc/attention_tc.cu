@@ -1,4 +1,4 @@
-// tcgen05 / TMEM fused attention forward for short sequences (S <= 256, head_dim 64, no LSE): the teacher's
+// tcgen05 / TMEM fused attention forward for short sequences (S <= 240, head_dim 64, no LSE): the teacher's
 // per-frame 197-token attention (clip.py:40-52, 12 layers x 3072 (frame, head) pairs per step).
 //
 // One persistent CTA per SM walks (sequence, head) items; per item the whole K and V of the head sit in smem
@@ -12,7 +12,6 @@
 // row sums of P [192, 208) — produced by the tensor core too (P x ones, N = 16), so the softmax threads spend their
 // FP32 issue slots on exactly one max, one FFMA and one ex2 per score.
 #include "common.cuh"
-#include <cstdlib>
 #include <mutex>
 #include <unordered_map>
 #include "../../include/unite_b200.h"
@@ -32,11 +31,7 @@ struct AttnTcParams {
 constexpr int ONES_BYTES = 16 * 4 * 128;   // [16 rows (N)] x [256 keys (K)] bf16, K-major: 4 k-blocks of 16 x 128 B
 // register-resident kernels (NKT > 0): the first ATC_NH0 32-key blocks of a score row are turned into P while the rest is still
 // being read; their P lives in the tile's spare columns [NKT, NKT + 16 * ATC_NH0) instead of over the scores
-#ifndef UB_ATTN_TC_ONE_LOAD
 constexpr int ATC_NH0(int nkt) { return (nkt / 32) / 2; }
-#else
-constexpr int ATC_NH0(int) { return 0; }
-#endif
 // TMEM column (within the tile) of the bf16 P operand of key step k (16 keys = 8 columns)
 UB_DEVINL constexpr uint32_t atc_p_col(int nkt, int k) { return nkt > 0 && k < 2 * ATC_NH0(nkt) ? (uint32_t)(nkt + k * 8) : (uint32_t)(k * 8); }
 
@@ -187,7 +182,6 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
           constexpr int NH0 = ATC_NH0(NKT);                 // 32-column loads of the first half
           static_assert(TAIL == 0 || TAIL == 16, "NKT must be a multiple of 16");
           static_assert(NH0 * 32 <= NKT - 16 && NKT + NH0 * 16 <= 256, "first half: unmasked, and its P must fit the spare columns");
-#ifndef UB_ATTN_TC_ONE_LOAD
           float mb1;
           auto exp32 = [&](const uint32_t (&v)[32], int c) {         // keys [32 c, 32 c + 32) -> bf16 P
             uint32_t pk[16];
@@ -264,48 +258,6 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
             }
             tmem_st_32x8(t_row + NFULL * 16, pk);
           }
-#else
-          uint32_t sv[NKT];
-#pragma unroll
-          for (int c = 0; c < NFULL; ++c) tmem_ld_32x32(t_row + c * 32, *reinterpret_cast<uint32_t(*)[32]>(&sv[c * 32]));
-          if constexpr (TAIL) tmem_ld_32x16(t_row + NFULL * 32, *reinterpret_cast<uint32_t(*)[16]>(&sv[NFULL * 32]));
-          tmem_ld_wait();
-          float m4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
-#pragma unroll
-          for (int i = 0; i < NKT - 16; ++i) m4[i & 3] = fmaxf(m4[i & 3], __uint_as_float(sv[i]));
-#pragma unroll
-          for (int i = NKT - 16; i < NKT; ++i)
-            if (i < S) m4[i & 3] = fmaxf(m4[i & 3], __uint_as_float(sv[i]));
-          const float mb1 = fmaxf(fmaxf(m4[0], m4[1]), fmaxf(m4[2], m4[3])) * sl2;
-          if (t == 0) asm volatile("bar.sync 2, 256;" ::: "memory"); else asm volatile("bar.sync 3, 256;" ::: "memory");
-#pragma unroll
-          for (int c = 0; c < NKT / 32; ++c) {
-            uint32_t pk[16];
-#pragma unroll
-            for (int i = 0; i < 16; ++i) {
-              const int k0 = c * 32 + 2 * i;
-              float p0 = fast_exp2(fmaf(__uint_as_float(sv[k0]), sl2, -mb1));
-              float p1 = fast_exp2(fmaf(__uint_as_float(sv[k0 + 1]), sl2, -mb1));
-              if (k0 >= NKT - 16) {
-                if (k0 >= S) p0 = 0.f;
-                if (k0 + 1 >= S) p1 = 0.f;
-              }
-              pk[i] = pack_bf16x2(p0, p1);
-            }
-            tmem_st_32x16(t_row + c * 16, pk);
-          }
-          if constexpr (TAIL) {
-            uint32_t pk[8];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-              const int k0 = NFULL * 32 + 2 * i;
-              const float p0 = (k0 < S) ? fast_exp2(fmaf(__uint_as_float(sv[k0]), sl2, -mb1)) : 0.f;
-              const float p1 = (k0 + 1 < S) ? fast_exp2(fmaf(__uint_as_float(sv[k0 + 1]), sl2, -mb1)) : 0.f;
-              pk[i] = pack_bf16x2(p0, p1);
-            }
-            tmem_st_32x8(t_row + NFULL * 16, pk);
-          }
-#endif
           if (t == 0) asm volatile("bar.arrive 3, 256;" ::: "memory"); else asm volatile("bar.arrive 2, 256;" ::: "memory");
         } else {
         // ---- pass 1: row maximum over the valid keys (only the chunk that straddles S pays for masking)
@@ -480,7 +432,7 @@ int make_tmap_3d_bf16(CUtensorMap* out, const void* base, int64_t d2, int64_t d1
   return 0;
 }
 
-// used by ub_attn_fwd (attention.cu) when S <= 256 and no LSE is requested
+// used by ub_attn_fwd (attention.cu) when S <= 240 and no LSE is requested
 int launch_attn_fwd_tc(const void* qkv, void* o, int n_seq, int S, int H, float scale, cudaStream_t stream) {
   AttnTcParams p;
   p.n_seq = n_seq; p.S = S; p.H = H;
@@ -499,12 +451,7 @@ int launch_attn_fwd_tc(const void* qkv, void* o, int n_seq, int S, int H, float 
   const int smem = 2 * (p.RB * 128 + 2 * p.NK * 128) + 8 * 4096 + ONES_BYTES + 12 * 8 + 16;
   const int items = n_seq * H;
   const int grid = items < sm_count() ? items : sm_count();
-  static int use_regs = -1;
-  if (use_regs < 0) {
-    const char* e = getenv("UB_ATTN_TC_REGS");
-    use_regs = e ? atoi(e) : 1;
-  }
-  if (p.NK == 208 && use_regs) {      // the teacher's 197-token frames (224^2 / 16^2 patches + CLS)
+  if (p.NK == 208) {  // the teacher's 197-token frames (224^2 / 16^2 patches + CLS)
     static int configured208 = 0;
     if (configured208 < smem) {
       cudaError_t e = cudaFuncSetAttribute(attn_fwd_tc_kernel<208>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
