@@ -204,6 +204,12 @@ UB_API int ub_l2norm_rows(float* x, int rows, int D, void* stream);
  *   ub_cast_scale_bf16  out = bf16(x * row_scale[row / rows_per_scale]).
  * ---------------------------------------------------------------------------------------------- */
 UB_API int ub_patchify(const float* x, void* out, int B, int T, int H, int W, int tubelet, void* stream);
+/* the same rows of the clip mixed as timm's batch-mode Mixup mixes it (stage-2 mixup_fn, engine_for_finetuning.py:86-87); x is
+ * not written.  mix: DEVICE fp32 {apply, lam, 1 - lam, use_cutmix, t0, t1, h0, h1, w0, w1} (1 - lam computed in double, then
+ * rounded).  apply == 0: ub_patchify.  cutmix: clip b takes clip B-1-b's values inside the half-open box [t0,t1) x [h0,h1) x
+ * [w0,w1) of the T, H, W axes.  mixup: lam * x_b + (1 - lam) * x_{B-1-b}, both products and the sum rounded on their own in fp32
+ * (bit-identical to torch's in-place mix).  B must be even. */
+UB_API int ub_patchify_mix(const float* x, void* out, const float* mix, int B, int T, int H, int W, int tubelet, void* stream);
 /* decoded uint8 frames [B,T,H,W,3] -> the same rows, with ToTensor + tensor_normalize(mean, std) applied on the way
  * (src/datasets/kinetics_sparse.py:236-243, 434-451); mean3 / std3 are HOST pointers to 3 floats.                     */
 UB_API int ub_patchify_u8(const uint8_t* x, void* out, const float* mean3, const float* std3, int B, int T, int H, int W,
@@ -305,6 +311,12 @@ UB_API int ub_linear_small_bwd(const float* x, const float* W, const float* dout
                                int C, int D, void* stream);
 UB_API int ub_softmax_ce(const float* logits, const int* labels, const float* weights, float scale, float* loss_acc,
                          float* dlogits, int B, int C, void* stream);
+/* soft-target CE of batch-mode mixup with label smoothing (timm SoftTargetCrossEntropy of mixup_target, run_stage2.py:702):
+ * t_bc = lam (c == y_b ? on : off) + (1 - lam) (c == y_{B-1-b} ? on : off), off = s / C, on = 1 - s + off; mix: DEVICE fp32
+ * {lam, on, off}.  loss_acc += scale * sum_b sum_c -t_bc log_softmax_c;  dlogits = scale * (softmax * sum_c t_bc - t).
+ * lam = 1: label smoothing alone (LabelSmoothingCrossEntropy(s), CrossEntropyLoss(label_smoothing=s)). */
+UB_API int ub_soft_target_ce(const float* logits, const int* labels, const float* mix, float scale, float* loss_acc,
+                             float* dlogits, int B, int C, void* stream);
 UB_API int ub_clip_zero_shot(const float* img_feat, const float* text_feat, float* probs, int B, int T, int C, int D,
                              void* stream);
 UB_API int ub_pseudo_label_fusion(const float* logits_full, const float* clip_probs, float threshold, int conf_weighted,

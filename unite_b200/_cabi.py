@@ -90,6 +90,7 @@ SIGNATURES = {
     "ub_dec_tail_bwd": (C.c_int, [_P, _P, _P, _F, _P, _F, _I, _I, _P, _P, _P, _I, _I, _P]),
     "ub_l2norm_rows": (C.c_int, [_P, _I, _I, _P]),
     "ub_patchify": (C.c_int, [_P, _P, _I, _I, _I, _I, _I, _P]),
+    "ub_patchify_mix": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "ub_patchify_u8": (C.c_int, [_P, _P, C.POINTER(C.c_float), C.POINTER(C.c_float), _I, _I, _I, _I, _I, _P]),
     "ub_resize_patchify": (C.c_int, [_P, _I, C.POINTER(C.c_float), C.POINTER(C.c_float), _P, _L, _I, _I, _I, _I, _I, _I, _I, _P]),
     "ub_mask_select": (C.c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
@@ -110,6 +111,7 @@ SIGNATURES = {
     "ub_linear_small_fwd": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _P]),
     "ub_linear_small_bwd": (C.c_int, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _P]),
     "ub_softmax_ce": (C.c_int, [_P, _P, _P, _F, _P, _P, _I, _I, _P]),
+    "ub_soft_target_ce": (C.c_int, [_P, _P, _P, _F, _P, _P, _I, _I, _P]),
     "ub_clip_zero_shot": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _P]),
     "ub_pseudo_label_fusion": (C.c_int, [_P, _P, _F, _I, _P, _P, _P, _P, _I, _I, _P]),
 }

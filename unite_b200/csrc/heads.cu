@@ -6,6 +6,7 @@
 //                            stage-3 `src_classifier = nn.Linear(768, C)` (run_stage3.py:1193)
 //   ub_softmax_ce            (weighted) cross-entropy forward + gradient: engine_for_finetuning.py:39,
 //                            run_stage3.py:486 (source CE), :606-615 (confidence-weighted target CE)
+//   ub_soft_target_ce        stage-2 mixup / label-smoothing loss + gradient (run_stage2.py:702), target built on the fly
 //   ub_clip_zero_shot        utils.clip_infer after encode_image (utils.py:62-68): per-frame softmax(100 cos) mean over frames
 //   ub_pseudo_label_fusion   selection_strategy 'clip_matchORconf' (run_stage3.py:489-490, 556-587): argmax / max-softmax of
 //                            the student, match-or-exactly-one-confident selection, per-sample loss weights
@@ -111,6 +112,41 @@ __global__ void __launch_bounds__(256) softmax_ce_kernel(const float* __restrict
   if (lane == 0 && loss_acc != nullptr) atomicAdd(loss_acc, w * (lse - l[y]));
   if (dlogits != nullptr)
     for (int c = lane; c < C; c += 32) dlogits[(int64_t)b * C + c] = w * (expf(l[c] - lse) - (c == y ? 1.0f : 0.0f));
+}
+
+// Soft-target cross-entropy of batch-mode mixup (timm SoftTargetCrossEntropy(mixup_target(...)), run_stage2.py:702 with mixup):
+//   t_bc = lam * (c == y_b ? on : off) + (1 - lam) * (c == y_{B-1-b} ? on : off)      mix (device fp32) = {lam, on, off}
+//   loss_acc += scale * sum_b sum_c -t_bc * log_softmax(logits_b)_c;  dlogits[b,c] = scale * (softmax_bc * sum_c t_bc - t_bc)
+// The [B,C] target is never stored.  lam = 1 is label smoothing alone (LabelSmoothingCrossEntropy, CrossEntropyLoss(label_smoothing)).
+// One warp per sample, like softmax_ce.
+__global__ void __launch_bounds__(256) soft_target_ce_kernel(const float* __restrict__ logits, const int* __restrict__ labels,
+                                                             const float* __restrict__ mix, float scale, float* __restrict__ loss_acc,
+                                                             float* __restrict__ dlogits, int B, int C) {
+  pdl_grid_sync();
+  const int b = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (b >= B) return;
+  const float lam = mix[0], on = mix[1], off = mix[2], lam1 = 1.0f - lam;
+  const int y = labels[b], y2 = labels[B - 1 - b];
+  const float* l = logits + (int64_t)b * C;
+  float mx = -INFINITY;
+  for (int c = lane; c < C; c += 32) mx = fmaxf(mx, l[c]);
+  mx = warp_max(mx);
+  float se = 0.f, st = 0.f;
+  for (int c = lane; c < C; c += 32) {
+    se += expf(l[c] - mx);
+    st += lam * (c == y ? on : off) + lam1 * (c == y2 ? on : off);
+  }
+  se = warp_sum(se);
+  st = warp_sum(st);
+  const float lse = mx + logf(se);
+  float loss = 0.f;
+  for (int c = lane; c < C; c += 32) {
+    const float t = lam * (c == y ? on : off) + lam1 * (c == y2 ? on : off);
+    loss += t * (lse - l[c]);
+    if (dlogits != nullptr) dlogits[(int64_t)b * C + c] = scale * (expf(l[c] - lse) * st - t);
+  }
+  loss = warp_sum(loss);
+  if (lane == 0 && loss_acc != nullptr) atomicAdd(loss_acc, scale * loss);
 }
 
 // probs[b, c] = mean_t softmax_c(100 * <img[b*T+t]/|.|, txt[c]/|.|>)   one block per clip, one warp per frame, C <= 32*? (loop)
@@ -228,6 +264,13 @@ extern "C" int ub_softmax_ce(const float* logits, const int* labels, const float
   UB_REQUIRE(logits && labels && B > 0 && C > 0, "softmax_ce: bad arguments");
   UB_LAUNCH(softmax_ce_kernel, (B + 7) / 8, 256, 0, (cudaStream_t)stream, logits, labels, weights, scale, loss_acc, dlogits, B, C);
   return check_launch("softmax_ce_kernel");
+}
+
+extern "C" int ub_soft_target_ce(const float* logits, const int* labels, const float* mix, float scale, float* loss_acc, float* dlogits,
+                                 int B, int C, void* stream) {
+  UB_REQUIRE(logits && labels && mix && B > 0 && C > 0, "soft_target_ce: bad arguments");
+  UB_LAUNCH(soft_target_ce_kernel, (B + 7) / 8, 256, 0, (cudaStream_t)stream, logits, labels, mix, scale, loss_acc, dlogits, B, C);
+  return check_launch("soft_target_ce_kernel");
 }
 
 extern "C" int ub_clip_zero_shot(const float* img_feat, const float* text_feat, float* probs, int B, int T, int C, int D,

@@ -2,6 +2,7 @@
 //
 //   ub_patchify      fp32 clip -> bf16 im2col rows (the A operand of the stride==kernel Conv3d as a GEMM)
 //                    clip.py:123-128,146 (teacher conv1), modeling_finetune.py:165-174 (student PatchEmbed.proj)
+//   ub_patchify_mix  the same rows of the batch-mode mixup / cutmix of the clip (stage-2 mixup_fn), x left untouched
 //   ub_mask_select   attention-guided visible-token selection, bit-exact
 //                    run_stage1.py:379-387 (multinomial == top-N_vis of attn/q, q ~ Exp(1) supplied by the caller)
 //                    utils.py:89-120 get_greedy_masks (k committee members take ranks i, i+k, ...; q == NULL)
@@ -39,6 +40,78 @@ __global__ void __launch_bounds__(256) patchify_kernel(const float* __restrict__
     bf16* dst = out + tok * (long)(runs_per_tok * 16) + run * 16;
     stg_v4(dst, o0);
     stg_v4(dst + 8, o1);
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
+// patchify_mix: ub_patchify of the clip mixed as timm's batch-mode Mixup._mix_batch mixes it (run_stage2.py's mixup_fn,
+// engine_for_finetuning.py:86-87), in one pass that never writes x — so a graph replayed over a resident input buffer mixes the
+// clip afresh on every replay instead of mixing its own output again.
+//   mix (device fp32) = {apply, lam, 1 - lam, use_cutmix, t0, t1, h0, h1, w0, w1}
+//   apply == 0: copy.  cutmix: inside the half-open box [t0,t1) x [h0,h1) x [w0,w1) of the (T, H, W) axes, clip b takes clip
+//   B-1-b's value.  mixup: lam * x_b + (1 - lam) * x_{B-1-b} with each product and the sum rounded on their own (no FMA) — what
+//   x.mul_(lam).add_(x.flip(0).mul_(1 - lam)) computes in fp32, so the rows are bit-identical to patchify(torch-mixed clip).
+// One thread moves the same (token, c, kt, kh) run of clips b and B-1-b (b < B/2, B even): every input byte is read once.
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) patchify_mix_kernel(const float* __restrict__ x, bf16* __restrict__ out,
+                                                           const float* __restrict__ mix, int B, int T, int H, int W, int tub,
+                                                           long total_runs) {
+  pdl_grid_sync();
+  const bool apply = mix[0] != 0.f, cut = mix[3] != 0.f;
+  const float lam = mix[1], lam1 = mix[2];
+  const int t0 = (int)mix[4], t1 = (int)mix[5], h0 = (int)mix[6], h1 = (int)mix[7], w0 = (int)mix[8], w1 = (int)mix[9];
+  const int gh = H / 16, gw = W / 16, Tp = T / tub;
+  const int runs_per_tok = 3 * tub * 16;
+  const long toks_per_clip = (long)Tp * gh * gw;
+  const long clip_elems = 3L * T * H * W;
+  for (long id = (long)blockIdx.x * blockDim.x + threadIdx.x; id < total_runs; id += (long)gridDim.x * blockDim.x) {
+    const int run = (int)(id % runs_per_tok);
+    const long tok = id / runs_per_tok;                       // token of the first half of the batch
+    const int kh = run % 16, kt = (run / 16) % tub, c = run / (16 * tub);
+    const int pw = (int)(tok % gw), ph = (int)((tok / gw) % gh), tp = (int)((tok / ((long)gw * gh)) % Tp);
+    const int b = (int)(tok / toks_per_clip);
+    const int t = tp * tub + kt, h = ph * 16 + kh;
+    const long mirror = (long)(B - 1 - 2 * b);                // clip B-1-b is `mirror` clips further on
+    const float* sa = x + ((((long)b * 3 + c) * T + t) * H + h) * W + pw * 16;
+    const float* sb = sa + mirror * clip_elems;
+    float a[16], m[16];
+#pragma unroll
+    for (int i = 0; i < 16; i += 4) {
+      *reinterpret_cast<float4*>(&a[i]) = *reinterpret_cast<const float4*>(sa + i);
+      *reinterpret_cast<float4*>(&m[i]) = *reinterpret_cast<const float4*>(sb + i);
+    }
+    if (apply) {
+      if (cut) {
+        if (t >= t0 && t < t1 && h >= h0 && h < h1) {
+#pragma unroll
+          for (int i = 0; i < 16; ++i) {
+            const int w = pw * 16 + i;
+            if (w >= w0 && w < w1) { const float s = a[i]; a[i] = m[i]; m[i] = s; }
+          }
+        }
+      } else {
+#pragma unroll
+        for (int i = 0; i < 16; ++i) {
+          const float va = a[i], vm = m[i];
+          a[i] = __fadd_rn(__fmul_rn(va, lam), __fmul_rn(vm, lam1));
+          m[i] = __fadd_rn(__fmul_rn(vm, lam), __fmul_rn(va, lam1));
+        }
+      }
+    }
+    uint4 o[4];
+#pragma unroll
+    for (int i = 0; i < 2; ++i) {
+      o[i].x = pack_bf16x2(a[8 * i], a[8 * i + 1]); o[i].y = pack_bf16x2(a[8 * i + 2], a[8 * i + 3]);
+      o[i].z = pack_bf16x2(a[8 * i + 4], a[8 * i + 5]); o[i].w = pack_bf16x2(a[8 * i + 6], a[8 * i + 7]);
+      o[2 + i].x = pack_bf16x2(m[8 * i], m[8 * i + 1]); o[2 + i].y = pack_bf16x2(m[8 * i + 2], m[8 * i + 3]);
+      o[2 + i].z = pack_bf16x2(m[8 * i + 4], m[8 * i + 5]); o[2 + i].w = pack_bf16x2(m[8 * i + 6], m[8 * i + 7]);
+    }
+    bf16* da = out + tok * (long)(runs_per_tok * 16) + run * 16;
+    bf16* db = da + mirror * toks_per_clip * (long)(runs_per_tok * 16);
+    stg_v4(da, o[0]);
+    stg_v4(da + 8, o[1]);
+    stg_v4(db, o[2]);
+    stg_v4(db + 8, o[3]);
   }
 }
 
@@ -380,6 +453,16 @@ extern "C" int ub_patchify(const float* x, void* out, int B, int T, int H, int W
   const long runs = tokens * 3 * tubelet * 16;
   UB_LAUNCH(patchify_kernel, flat_grid(runs, 256), 256, 0, (cudaStream_t)stream, x, (bf16*)out, B, T, H, W, tubelet, runs);
   return check_launch("patchify_kernel");
+}
+
+extern "C" int ub_patchify_mix(const float* x, void* out, const float* mix, int B, int T, int H, int W, int tubelet, void* stream) {
+  UB_REQUIRE(x && out && mix, "patchify_mix: null pointer");
+  UB_REQUIRE(B > 0 && B % 2 == 0, "patchify_mix: the batch must be even to pair clip b with clip B-1-b (B=%d)", B);
+  UB_REQUIRE(T > 0 && tubelet > 0 && T % tubelet == 0, "patchify_mix: bad temporal shape T=%d tubelet=%d", T, tubelet);
+  UB_REQUIRE(H % 16 == 0 && W % 16 == 0 && H > 0 && W > 0, "patchify_mix: H, W must be multiples of the 16-pixel patch (H=%d W=%d)", H, W);
+  const long runs = (long)(B / 2) * (T / tubelet) * (H / 16) * (W / 16) * 3 * tubelet * 16;
+  UB_LAUNCH(patchify_mix_kernel, flat_grid(runs, 256), 256, 0, (cudaStream_t)stream, x, (bf16*)out, mix, B, T, H, W, tubelet, runs);
+  return check_launch("patchify_mix_kernel");
 }
 
 extern "C" int ub_patchify_u8(const uint8_t* x, void* out, const float* mean3, const float* std3, int B, int T, int H, int W,

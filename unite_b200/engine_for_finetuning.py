@@ -1,10 +1,13 @@
 """Stage-2 supervised fine-tuning step with the reference's `train_one_epoch` signature
-(src/engines/engine_for_finetuning.py:48-54; non-DeepSpeed branch :116-127, no mixup).
+(src/engines/engine_for_finetuning.py:48-54; non-DeepSpeed branch :116-127).
 
-    loss = CE(model(samples), targets) / update_freq          engine_for_finetuning.py:37-40, :119
+    samples, targets = mixup_fn(samples, targets)             engine_for_finetuning.py:86-87 (when mixup_fn is given)
+    loss = criterion(model(samples), targets) / update_freq   engine_for_finetuning.py:37-40, :119
     backward every micro-step, optimizer every update_freq     :120-126
-The loss and its gradient come from one fused kernel (ub_softmax_ce); the model's backward is the explicit one in
-finetune_core.py; gradients accumulate in the parameter arena across micro-steps like `.grad` does in torch.
+The loss and its gradient come from one fused kernel: ub_softmax_ce for CrossEntropyLoss(), ub_soft_target_ce for the mixup
+and label-smoothing criteria (mixup.resolve_loss).  Mixup / cutmix are drawn on the host exactly as timm draws them and applied
+on the device inside the im2col (ub_patchify_mix), so the caller's clip is never written.  The model's backward is the explicit
+one in finetune_core.py; gradients accumulate in the parameter arena across micro-steps like `.grad` does in torch.
 """
 import math
 import sys
@@ -14,6 +17,7 @@ import torch
 
 from . import ops
 from .engine import FusedAdamW, require_fused_optimizer
+from .mixup import NO_MIX, MixBuffer, draw, resolve_loss
 
 
 def train_class_batch(model, samples, target, criterion):
@@ -34,17 +38,22 @@ def _default_optimizer(net):
     return opt
 
 
-def finetune_step(model, samples, targets, loss_acc, scale=1.0, grad_sync=None):
+def finetune_step(model, samples, targets, loss_acc, scale=1.0, grad_sync=None, mix=None):
     """One micro-step: forward, CE, backward.  Adds scale * mean CE to loss_acc (fp32 [1]).  Returns logits.
     grad_sync: pass the model's GradSync on the micro-step that is followed by the optimizer step — its range all-reduces then
-    overlap this backward."""
+    overlap this backward.
+    mix: None (plain CE), or a mixup.MixBuffer holding this step's draw on the device: the clip is mixed on its way into the
+    im2col (mix.clip, None for label smoothing alone) and the loss is the soft-target CE of the mixed, smoothed target."""
     net = model.module if hasattr(model, "module") else model
     core = net.core()
     dp = core.drop_path.draw(samples.shape[0]) if net.training else None       # modeling_finetune.py:42-50 (device-side draws)
-    logits, state = core.run_forward(samples, dp, save=True)
+    logits, state = core.run_forward(samples, dp, save=True, mix=None if mix is None else mix.clip)
     B = logits.shape[0]
     dlogits = torch.empty_like(logits)
-    ops.softmax_ce(logits, targets.to(torch.int32), None, scale / B, loss_acc, dlogits)
+    if mix is None:
+        ops.softmax_ce(logits, targets.to(torch.int32), None, scale / B, loss_acc, dlogits)
+    else:
+        ops.soft_target_ce(logits, targets.to(torch.int32), mix.target, scale / B, loss_acc, dlogits)
     core.run_backward(state, dlogits, grad_sync=grad_sync)
     return logits
 
@@ -71,11 +80,13 @@ class Stage2Engine:
         self.stats = torch.zeros(3, device=dev)             # running sums: loss, correct predictions, grad-norm
         self.graphs = GraphReplay()
         self.logits = None
+        self._mix_bufs = {}                                 # loss kind -> MixBuffer (fixed addresses the graphs read)
+        self._mix = None                                    # the buffer of the current step, None for plain CE
 
     def _body(self, samples, targets):
         self.optimizer.zero_grad()
         self.loss.zero_()
-        logits = finetune_step(self.model, samples, targets, self.loss, scale=1.0, grad_sync=self.grad_sync)
+        logits = finetune_step(self.model, samples, targets, self.loss, scale=1.0, grad_sync=self.grad_sync, mix=self._mix)
         if self.grad_sync is not None:
             self.grad_sync.all_reduce(self.core.arena.grads)
         self.optimizer.step_dev(max_norm=self.max_norm)
@@ -83,15 +94,27 @@ class Stage2Engine:
         self.stats += torch.cat([self.loss, (logits.argmax(-1) == targets).sum().float().view(1), self.optimizer.grad_norm(scale)])
         self.logits = logits
 
-    def step(self, samples, targets, private_inputs=False):
+    def step(self, samples, targets, private_inputs=False, mix=None, smoothing=None):
         """samples fp32 [B,3,T,H,W], targets integer [B], both on the device.  Returns the device loss tensor [1].
-        private_inputs: the batch lives in fresh tensors every step (a loader), so the graph keeps its own static inputs."""
+        private_inputs: the batch lives in fresh tensors every step (a loader), so the graph keeps its own static inputs.
+        smoothing None: plain CE.  smoothing s: soft-target CE with label smoothing s, and with mix (a mixup.MixDraw, NO_MIX for a
+        batch the draw left unmixed) the clip is mixed as drawn.  The draw is uploaded to device memory before the step, so every
+        replay of the one graph per loss kind reads its own draw."""
+        if mix is not None and smoothing is None:
+            raise ValueError("Stage2Engine.step: a mixup draw needs the soft-target loss (pass smoothing=)")
         scale = 1.0 / self.grad_sync.world if self.grad_sync is not None else 1.0
         self.optimizer.prepare_step(grad_scale=scale)
+        kind = "ce" if smoothing is None else ("mix" if mix is not None else "smooth")
+        self._mix = None
+        if kind != "ce":
+            if kind not in self._mix_bufs:
+                self._mix_bufs[kind] = MixBuffer(self.core.arena.device, mix_clips=kind == "mix")
+            self._mix = self._mix_bufs[kind]
+            self._mix.upload((mix or NO_MIX).packed(smoothing, self.core.C))
         if not self.use_graph:
             self._body(samples, targets)
             return self.loss
-        key = (tuple(samples.shape), samples.dtype, targets.dtype, float(self.max_norm or 0.0), bool(self.net.training))
+        key = (tuple(samples.shape), samples.dtype, targets.dtype, float(self.max_norm or 0.0), bool(self.net.training), kind)
         self.logits = self.graphs.run(key, (samples, targets), self._body, state_fn=lambda: self.logits, private=private_inputs)
         return self.loss
 
@@ -109,22 +132,25 @@ def train_one_epoch(model: torch.nn.Module, criterion=None, data_loader: Iterabl
                     loss_scaler=None, max_norm: float = 0, model_ema=None, mixup_fn=None, log_writer=None, start_steps=None,
                     lr_schedule_values=None, wd_schedule_values=None, num_training_steps_per_epoch=None, update_freq=None,
                     num_epochs=None, train_head_only=False, wandb_run=None, args=None):
-    if mixup_fn is not None or model_ema is not None or train_head_only:
-        raise NotImplementedError("mixup / EMA / head-only training are off in the shipped stage-2 config")
-    if criterion is not None and not (isinstance(criterion, torch.nn.CrossEntropyLoss) and criterion.label_smoothing == 0.0
-                                      and criterion.weight is None and criterion.reduction == "mean"):
-        raise NotImplementedError("the fused stage-2 loss is nn.CrossEntropyLoss() (run_stage2.py:702 without mixup / smoothing)")
+    """mixup_fn: a mixup.Mixup (or the reference's timm Mixup) in batch mode, drawn once per loader batch; criterion: see
+    mixup.resolve_loss.  With mixup_fn the returned dict has no class_acc (the reference logs None there)."""
+    if model_ema is not None or train_head_only:
+        raise NotImplementedError("model EMA and head-only training are not implemented in the fused stage-2 loop")
+    smoothing = resolve_loss(criterion, mixup_fn)
     model.train(True)
     net = model.module if hasattr(model, "module") else model
     core = net.core()
     dev = core.arena.device
+    if mixup_fn is not None and mixup_fn.num_classes != core.C:
+        raise ValueError(f"mixup_fn.num_classes={mixup_fn.num_classes} differs from the model's {core.C} classes")
     update_freq = update_freq or 1
     start_steps = start_steps or 0
     optimizer = require_fused_optimizer(optimizer, core.arena, "train_one_epoch") or _default_optimizer(net)
     gs = getattr(model, "grad_sync", None)
     if update_freq == 1:
         return _train_one_epoch_graphed(model, net, data_loader, optimizer, gs, max_norm, start_steps, lr_schedule_values,
-                                        wd_schedule_values, num_training_steps_per_epoch)
+                                        wd_schedule_values, num_training_steps_per_epoch, mixup_fn, smoothing)
+    mix = None if smoothing is None else MixBuffer(dev, mix_clips=mixup_fn is not None)
     loss_sum = torch.zeros(1, device=dev)
     loss_acc = torch.zeros(1, device=dev)
     correct = torch.zeros(1, device=dev)
@@ -145,11 +171,14 @@ def train_one_epoch(model: torch.nn.Module, criterion=None, data_loader: Iterabl
                     group["lr"] = lr_schedule_values[min(it, len(lr_schedule_values) - 1)] * group.get("lr_scale", 1.0)
                 if wd_schedule_values is not None and group["weight_decay"] > 0:
                     group["weight_decay"] = wd_schedule_values[min(it, len(wd_schedule_values) - 1)]
+        if mix is not None:
+            mix.upload((draw(mixup_fn, samples.shape) if mixup_fn is not None else NO_MIX).packed(smoothing, core.C))
         samples = samples.to(dev, non_blocking=True)
         targets = targets.to(dev, non_blocking=True)
         loss_acc.zero_()
         last_micro = (data_iter_step + 1) % update_freq == 0
-        logits = finetune_step(model, samples, targets, loss_acc, scale=1.0 / update_freq, grad_sync=gs if last_micro else None)
+        logits = finetune_step(model, samples, targets, loss_acc, scale=1.0 / update_freq, grad_sync=gs if last_micro else None,
+                               mix=mix)
         loss_sum += loss_acc * update_freq
         correct += (logits.argmax(-1) == targets).sum()
         seen += samples.shape[0]
@@ -166,12 +195,15 @@ def train_one_epoch(model: torch.nn.Module, criterion=None, data_loader: Iterabl
         sys.exit(1)
     lrs = [g["lr"] for g in optimizer.param_groups]
     wds = [g["weight_decay"] for g in optimizer.param_groups if g["weight_decay"] > 0]
-    return {"loss": loss_avg, "class_acc": (correct / max(seen, 1)).item(), "loss_scale": 1.0, "lr": max(lrs), "min_lr": min(lrs),
-            "weight_decay": wds[0] if wds else None, "grad_norm": (gn_sum / max(1, n_updates)).item()}
+    stats = {"loss": loss_avg, "class_acc": (correct / max(seen, 1)).item(), "loss_scale": 1.0, "lr": max(lrs), "min_lr": min(lrs),
+             "weight_decay": wds[0] if wds else None, "grad_norm": (gn_sum / max(1, n_updates)).item()}
+    if mixup_fn is not None:
+        del stats["class_acc"]
+    return stats
 
 
 def _train_one_epoch_graphed(model, net, data_loader, optimizer, gs, max_norm, start_steps, lr_schedule_values, wd_schedule_values,
-                             num_training_steps_per_epoch):
+                             num_training_steps_per_epoch, mixup_fn=None, smoothing=None):
     """update_freq == 1 (the shipped stage-2 recipe): every loader batch is one whole update, run through Stage2Engine (CUDA-graph
     replay).  Same schedule handling and return dict as the general loop above."""
     eng = _stage2_engine(model, net, optimizer, gs)
@@ -188,7 +220,9 @@ def _train_one_epoch_graphed(model, net, data_loader, optimizer, gs, max_norm, s
                 group["lr"] = lr_schedule_values[min(it, len(lr_schedule_values) - 1)] * group.get("lr_scale", 1.0)
             if wd_schedule_values is not None and group["weight_decay"] > 0:
                 group["weight_decay"] = wd_schedule_values[min(it, len(wd_schedule_values) - 1)]
-        eng.step(batch[0].to(dev, non_blocking=True), batch[1].to(dev, non_blocking=True), private_inputs=True)
+        mix = draw(mixup_fn, batch[0].shape) if mixup_fn is not None else None
+        eng.step(batch[0].to(dev, non_blocking=True), batch[1].to(dev, non_blocking=True), private_inputs=True, mix=mix,
+                 smoothing=smoothing)
         seen += batch[0].shape[0]
         n += 1
     loss_sum, correct, gn_sum = eng.stats.tolist()
@@ -198,8 +232,11 @@ def _train_one_epoch_graphed(model, net, data_loader, optimizer, gs, max_norm, s
         sys.exit(1)
     lrs = [g["lr"] for g in optimizer.param_groups]
     wds = [g["weight_decay"] for g in optimizer.param_groups if g["weight_decay"] > 0]
-    return {"loss": loss_avg, "class_acc": correct / max(seen, 1), "loss_scale": 1.0, "lr": max(lrs), "min_lr": min(lrs),
-            "weight_decay": wds[0] if wds else None, "grad_norm": gn_sum / max(1, n)}
+    stats = {"loss": loss_avg, "class_acc": correct / max(seen, 1), "loss_scale": 1.0, "lr": max(lrs), "min_lr": min(lrs),
+             "weight_decay": wds[0] if wds else None, "grad_norm": gn_sum / max(1, n)}
+    if mixup_fn is not None:
+        del stats["class_acc"]                                                     # the reference's class_acc = None under mixup
+    return stats
 
 
 # ---------------------------------------------------------------------------------------------------------------------

@@ -53,11 +53,16 @@ class FinetuneCore:
             self._pos_full[B] = self.pos.repeat(B, 1).contiguous()
         return self._pos_full[B]
 
-    def run_forward(self, x, dp, save):
+    def run_forward(self, x, dp, save, mix=None):
+        """mix: None, or the device draw of batch-mode mixup / cutmix (mixup.MixBuffer.clip): the trunk then sees the mixed clip,
+        mixed on the way into the im2col (x itself is not written)."""
         self.sync_shadow()
         B, dev, a = x.shape[0], x.device, self.arena
         patches = torch.empty(B * self.N, 3 * self.tubelet * 256, device=dev, dtype=BF16)
-        ops.patchify(x.contiguous(), patches, self.tubelet)
+        if mix is None:
+            ops.patchify(x.contiguous(), patches, self.tubelet)
+        else:
+            ops.patchify_mix(x.contiguous(), patches, mix, self.tubelet)
         ws = self.trunk.forward(patches, self._pos_rows(B), B, self.N, self.depth, save, dp)
         pooled = torch.empty(B, self.D, device=dev, dtype=F32)
         ops.meanpool_fwd(ws.x_at(self.depth).view(B, self.N, self.D), pooled)                     # x.mean(1)

@@ -284,6 +284,20 @@ def patchify(x, out, tubelet):
     return out
 
 
+@_instrument("patchify_mix", 1)
+def patchify_mix(x, out, mix, tubelet):
+    """patchify of the batch-mode mixup / cutmix of x, x untouched.  mix: device fp32 [10] (see ub_patchify_mix; built by
+    unite_b200.mixup)."""
+    B, Cc, T, H, W = x.shape
+    if Cc != 3:
+        raise _cabi.UBError("patchify_mix: 3 input channels expected")
+    if mix.numel() < 10:
+        raise _cabi.UBError("patchify_mix: mix must hold 10 floats")
+    check(lib.ub_patchify_mix(_p(x, F32, "videos"), _p(out, BF16, "patches"), _p(mix, F32, "mix"), B, T, H, W, tubelet, _stream()),
+          "ub_patchify_mix")
+    return out
+
+
 IMAGENET_MEAN, IMAGENET_STD = (0.485, 0.456, 0.406), (0.229, 0.224, 0.225)      # kinetics_sparse.py:241-243
 
 
@@ -456,6 +470,16 @@ def softmax_ce(logits, labels, weights, scale, loss_acc, dlogits):
     B, Cc = logits.shape
     check(lib.ub_softmax_ce(_p(logits, F32, "logits"), _p(labels, I32, "labels"), _p(weights, F32, "weights"), scale,
                             _p(loss_acc, F32, "loss_acc"), _p(dlogits, F32, "dlogits"), B, Cc, _stream()), "ub_softmax_ce")
+
+
+@_instrument("soft_target_ce", 1)
+def soft_target_ce(logits, labels, mix, scale, loss_acc, dlogits):
+    """Soft-target CE of the mixup target built on the device from labels and mix = device fp32 [lam, on, off]."""
+    B, Cc = logits.shape
+    if mix.numel() < 3:
+        raise _cabi.UBError("soft_target_ce: mix must hold lam, on, off")
+    check(lib.ub_soft_target_ce(_p(logits, F32, "logits"), _p(labels, I32, "labels"), _p(mix, F32, "mix"), scale,
+                                _p(loss_acc, F32, "loss_acc"), _p(dlogits, F32, "dlogits"), B, Cc, _stream()), "ub_soft_target_ce")
 
 
 @_instrument("clip_zero_shot", 1)
