@@ -1,6 +1,6 @@
 #!/bin/bash
 # usage: tools/attn_sweep.sh [LOG]  (default build/attn_sweep.log) ; each attention shape in its own process + timeout, then
-# the adversarial forward inputs; prints every line that is not an OK
+# the per-row kernel tests against the fp64 reference (slow paths included); prints every line that is not an OK
 cd "$(dirname "$0")/.."
 L=${1:-build/attn_sweep.log}
 mkdir -p "$(dirname "$L")"
@@ -10,7 +10,7 @@ for shp in "2 17 2" "3 128 4" "2 160 3" "4 197 12" "2 256 3" "3 288 5" "2 300 3"
   timeout 90 python tools/attn_bwd_check.py $shp >> $L 2>&1
   echo "rc=$?" >> $L
 done
-echo "=== adversarial" >> $L
-timeout 90 python tools/attn_fwd_adv.py >> $L 2>&1
+echo "=== tests/test_attention_kernels_gpu.py" >> $L
+timeout 600 python -m pytest -q -m gpu tests/test_attention_kernels_gpu.py >> $L 2>&1
 echo "rc=$?" >> $L
 grep -v " OK$" $L
