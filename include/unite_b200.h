@@ -253,6 +253,12 @@ UB_API int ub_adamw_seg(float* p, const float* g, float* m, float* v, void* w_bf
 UB_API int ub_sumsq_seg(const float* g, int64_t n, const int32_t* seg_end4, int n_seg, const float* hyper, float* out,
                         void* stream);
 UB_API int ub_cast_bf16(const float* x, void* out, int64_t n, void* stream);
+/* Model EMA of the stage-2 loop (timm 0.4.12 ModelEma.update, called after every optimizer update at
+ * engine_for_finetuning.py:126-127): for every element of the fp32 arena, ema = fl(fl(ema * decay) + fl(p * one_minus_decay)),
+ * the two products and the sum rounded on their own (no FMA: bit-identical to torch's `ema_v * decay + (1. - decay) * model_v`
+ * in fp32), and ema_w16 = bf16 of the new ema, rounded as ub_cast_bf16 rounds.  The caller passes (float)decay and
+ * (float)(1.0 - decay), 1 - decay computed in double.  n: a positive multiple of 4.  p is only read. */
+UB_API int ub_ema_update(float* ema, void* ema_w16, const float* p, int64_t n, float decay, float one_minus_decay, void* stream);
 
 /* DropPath factors for one step (src/models/modeling_finetune.py:42-50 via timm drop_path; rates = linspace(0, drop_path, depth),
  * :311): out fp32 [depth, 2, B] = floor(keep_l + u) / keep_l, u ~ U[0,1) from Philox4x32-10 keyed by `seed` with counter

@@ -103,6 +103,7 @@ SIGNATURES = {
     "ub_adamw_seg": (C.c_int, [_P, _P, _P, _P, _P, _L, _P, _I, _P, _P, _P]),
     "ub_sumsq_seg": (C.c_int, [_P, _L, _P, _I, _P, _P, _P]),
     "ub_cast_bf16": (C.c_int, [_P, _P, _L, _P]),
+    "ub_ema_update": (C.c_int, [_P, _P, _P, _L, _F, _F, _P]),
     "ub_drop_path_draw": (C.c_int, [_P, _P, _I, _I, C.c_uint64, _P, _P]),
     "ub_nvls_slots": (C.c_int, []),
     "ub_adamw_nvls": (C.c_int, [_P, _P, _P, _P, _P, _P, _L, _L, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _P]),

@@ -10,6 +10,7 @@ adapters as small composable steps; `load_student_from_ckpt` / `load_from_ckpt` 
     resize_pos_embed   temporal linear + spatial bicubic interpolation of `pos_embed`   run_stage1.py:553-588, run_stage2.py:394-434
     load_state_dict    prefix-aware, non-strict load with the reference's report        src/utils.py:554-599
     save_model / auto_load_model   `checkpoint-<tag>.pth` with model / optimizer / epoch  src/utils.py:689-776
+                                   (+ `model_ema`, the EMA model's state_dict, when a model EMA is given)
 The CLIP teacher's adapter (2-D -> 3-D conv inflation, positional-grid resize, clip.py:191-231) lives next to the
 teacher in unite_b200/clip.py.
 """
@@ -165,8 +166,16 @@ def _is_master() -> bool:
     return not (dist.is_available() and dist.is_initialized()) or dist.get_rank() == 0
 
 
-def save_model(output_dir: str, epoch, model_without_ddp, optimizer, loss_scaler=None, args=None, tag: Optional[str] = None) -> str:
-    """`checkpoint-<epoch or tag>.pth` = {model, optimizer, epoch, scaler, args}; written by rank 0 only."""
+def _ema_model(model_ema):
+    """The EMA's own model (timm's get_state_dict(model_ema) unwraps ModelEma.ema and a `.module` wrapper)."""
+    m = model_ema.ema if hasattr(model_ema, "ema") else model_ema
+    return m.module if hasattr(m, "module") else m
+
+
+def save_model(output_dir: str, epoch, model_without_ddp, optimizer, loss_scaler=None, args=None, tag: Optional[str] = None,
+               model_ema=None) -> str:
+    """`checkpoint-<epoch or tag>.pth` = {model, optimizer, epoch, scaler, args}, plus `model_ema` (the EMA model's state_dict)
+    when model_ema is given; written by rank 0 only."""
     path = os.path.join(output_dir, "checkpoint-%s.pth" % (tag if tag is not None else str(epoch)))
     if hasattr(optimizer, "consolidate"):
         optimizer.consolidate()        # collective: gathers the rank-sharded fp32 master weights / Adam moments (ddp.NvlsShardedStep)
@@ -174,12 +183,16 @@ def save_model(output_dir: str, epoch, model_without_ddp, optimizer, loss_scaler
         os.makedirs(output_dir, exist_ok=True)
         to_save = {"model": model_without_ddp.state_dict(), "optimizer": optimizer.state_dict(), "epoch": epoch, "args": args,
                    "scaler": loss_scaler.state_dict() if loss_scaler is not None and hasattr(loss_scaler, "state_dict") else {}}
+        if model_ema is not None:
+            to_save["model_ema"] = _ema_model(model_ema).state_dict()
         torch.save(to_save, path)
     return path
 
 
-def auto_load_model(output_dir: str, model_without_ddp, optimizer=None, loss_scaler=None, resume: str = "", auto_resume: bool = True):
+def auto_load_model(output_dir: str, model_without_ddp, optimizer=None, loss_scaler=None, resume: str = "", auto_resume: bool = True,
+                    model_ema=None):
     """Resume order of the reference: checkpoint-latest.pth, checkpoint-best.pth, the highest numbered checkpoint-<n>.pth.
+    model_ema: restored from the checkpoint's `model_ema` entry when there is one (its bf16 shadow refreshed).
     Returns the epoch to start from (0 when nothing was found)."""
     if not resume:
         for name in ("checkpoint-latest.pth", "checkpoint-best.pth"):
@@ -199,6 +212,12 @@ def auto_load_model(output_dir: str, model_without_ddp, optimizer=None, loss_sca
     core = getattr(model_without_ddp, "_core", None)
     if core is not None and hasattr(core, "sync_shadow"):
         core.sync_shadow(force=True)
+    if model_ema is not None and "model_ema" in ckpt:
+        ema = _ema_model(model_ema)
+        ema.load_state_dict(ckpt["model_ema"])
+        core = getattr(ema, "_core", None)
+        if core is not None and hasattr(core, "sync_shadow"):
+            core.sync_shadow(force=True)
     start = 0
     if optimizer is not None and "optimizer" in ckpt and "epoch" in ckpt:
         optimizer.load_state_dict(ckpt["optimizer"])

@@ -210,6 +210,27 @@ __global__ void __launch_bounds__(256) cast_bf16_kernel(const float4* __restrict
   }
 }
 
+// Model EMA (timm 0.4.12 ModelEma.update): ema = fl(fl(ema * decay) + fl(p * one_minus_decay)), each product and the sum rounded
+// on its own (no FMA), as torch evaluates `ema_v * decay + (1. - decay) * model_v` in fp32; the bf16 shadow of the new value is
+// written in the same pass, so the EMA model can be evaluated at any time without a cast pass.
+__global__ void __launch_bounds__(256) ema_update_kernel(float4* __restrict__ ema, uint2* __restrict__ ema_w16, const float4* __restrict__ p,
+                                                         long n4, float decay, float one_minus_decay) {
+  pdl_grid_sync();
+  for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long)gridDim.x * blockDim.x) {
+    float4 e = ema[i];
+    const float4 q = p[i];
+    e.x = __fadd_rn(__fmul_rn(e.x, decay), __fmul_rn(q.x, one_minus_decay));
+    e.y = __fadd_rn(__fmul_rn(e.y, decay), __fmul_rn(q.y, one_minus_decay));
+    e.z = __fadd_rn(__fmul_rn(e.z, decay), __fmul_rn(q.z, one_minus_decay));
+    e.w = __fadd_rn(__fmul_rn(e.w, decay), __fmul_rn(q.w, one_minus_decay));
+    ema[i] = e;
+    uint2 o;
+    o.x = pack_bf16x2(e.x, e.y);
+    o.y = pack_bf16x2(e.z, e.w);
+    ema_w16[i] = o;
+  }
+}
+
 static int flat_grid4(long n4) {
   long want = (n4 + 255) / 256;
   const long cap = (long)sm_count() * 8;
@@ -271,4 +292,12 @@ extern "C" int ub_cast_bf16(const float* x, void* out, int64_t n, void* stream) 
   UB_REQUIRE(x && out && n > 0 && n % 4 == 0, "cast_bf16: n=%lld must be a positive multiple of 4", (long long)n);
   UB_LAUNCH(cast_bf16_kernel, flat_grid4(n / 4), 256, 0, (cudaStream_t)stream, (const float4*)x, (uint2*)out, n / 4);
   return check_launch("cast_bf16_kernel");
+}
+
+extern "C" int ub_ema_update(float* ema, void* ema_w16, const float* p, int64_t n, float decay, float one_minus_decay, void* stream) {
+  UB_REQUIRE(ema && ema_w16 && p, "ema_update: null pointer");
+  UB_REQUIRE(n > 0 && n % 4 == 0, "ema_update: n=%lld must be a positive multiple of 4", (long long)n);
+  UB_LAUNCH(ema_update_kernel, flat_grid4(n / 4), 256, 0, (cudaStream_t)stream, (float4*)ema, (uint2*)ema_w16, (const float4*)p, n / 4,
+            decay, one_minus_decay);
+  return check_launch("ema_update_kernel");
 }

@@ -8,6 +8,9 @@ The loss and its gradient come from one fused kernel: ub_softmax_ce for CrossEnt
 and label-smoothing criteria (mixup.resolve_loss).  Mixup / cutmix are drawn on the host exactly as timm draws them and applied
 on the device inside the im2col (ub_patchify_mix), so the caller's clip is never written.  The model's backward is the explicit
 one in finetune_core.py; gradients accumulate in the parameter arena across micro-steps like `.grad` does in torch.
+    model_ema.update(model)                                   engine_for_finetuning.py:126-127 (after every optimizer update)
+With `model_ema` (ema.ModelEma or timm's ModelEma) the EMA arena is updated by one fused kernel (ub_ema_update) right after the
+optimizer, inside the CUDA graph of the step.
 """
 import math
 import sys
@@ -16,6 +19,7 @@ from typing import Iterable, Optional
 import torch
 
 from . import ops
+from .ema import resolve_model_ema
 from .engine import FusedAdamW, require_fused_optimizer
 from .mixup import NO_MIX, MixBuffer, draw, resolve_loss
 
@@ -64,13 +68,17 @@ class Stage2Engine:
     the ~750 launches of the all-token step then cost one launch.  DropPath draws come from the device-side generator, the
     optimizer's lr / wd / bias corrections from device memory (FusedAdamW.prepare_step), so nothing in the body depends on the
     host.  The running sums train_one_epoch reports (loss, correct predictions, grad-norm) are accumulated on the device inside
-    the step."""
+    the step.  model_ema (ema.ModelEma or timm's ModelEma): its arena is updated right after AdamW, in the same graph; every rank
+    of a data-parallel run updates its own EMA from the same replicated weights."""
 
-    def __init__(self, model, optimizer: FusedAdamW, grad_sync=None, use_graph: bool = False):
+    def __init__(self, model, optimizer: FusedAdamW, grad_sync=None, use_graph: bool = False, model_ema=None):
         from .engine import GraphReplay
+        self.ema = resolve_model_ema(model_ema, model)
         self.model = model
         self.net = model.module if hasattr(model, "module") else model
         self.core = self.net.core()
+        if self.ema is not None:
+            self.ema.ema_net.core()                         # the EMA's arena exists before any step is captured
         self.optimizer = require_fused_optimizer(optimizer, self.core.arena, "Stage2Engine")
         self.grad_sync = grad_sync
         self.use_graph = use_graph
@@ -90,6 +98,8 @@ class Stage2Engine:
         if self.grad_sync is not None:
             self.grad_sync.all_reduce(self.core.arena.grads)
         self.optimizer.step_dev(max_norm=self.max_norm)
+        if self.ema is not None:
+            self.ema.update(self.model)
         scale = 1.0 / self.grad_sync.world if self.grad_sync is not None else 1.0
         self.stats += torch.cat([self.loss, (logits.argmax(-1) == targets).sum().float().view(1), self.optimizer.grad_norm(scale)])
         self.logits = logits
@@ -115,15 +125,18 @@ class Stage2Engine:
             self._body(samples, targets)
             return self.loss
         key = (tuple(samples.shape), samples.dtype, targets.dtype, float(self.max_norm or 0.0), bool(self.net.training), kind)
+        if self.ema is not None:
+            key += (("ema", self.ema.decay),)               # the decay is a launch argument recorded in the graph
         self.logits = self.graphs.run(key, (samples, targets), self._body, state_fn=lambda: self.logits, private=private_inputs)
         return self.loss
 
 
-def _stage2_engine(model, net, optimizer, gs):
+def _stage2_engine(model, net, optimizer, gs, model_ema=None):
     held = net.__dict__.get("_ub_stage2_engine")
-    if held is None or held.optimizer is not optimizer or held.grad_sync is not gs:
+    held_ema = None if held is None or held.ema is None else held.ema.source
+    if held is None or held.optimizer is not optimizer or held.grad_sync is not gs or held_ema is not model_ema:
         import os
-        held = Stage2Engine(model, optimizer, grad_sync=gs, use_graph=os.environ.get("UB_NO_GRAPH", "0") != "1")
+        held = Stage2Engine(model, optimizer, grad_sync=gs, use_graph=os.environ.get("UB_NO_GRAPH", "0") != "1", model_ema=model_ema)
         net.__dict__["_ub_stage2_engine"] = held
     return held
 
@@ -133,9 +146,12 @@ def train_one_epoch(model: torch.nn.Module, criterion=None, data_loader: Iterabl
                     lr_schedule_values=None, wd_schedule_values=None, num_training_steps_per_epoch=None, update_freq=None,
                     num_epochs=None, train_head_only=False, wandb_run=None, args=None):
     """mixup_fn: a mixup.Mixup (or the reference's timm Mixup) in batch mode, drawn once per loader batch; criterion: see
-    mixup.resolve_loss.  With mixup_fn the returned dict has no class_acc (the reference logs None there)."""
-    if model_ema is not None or train_head_only:
-        raise NotImplementedError("model EMA and head-only training are not implemented in the fused stage-2 loop")
+    mixup.resolve_loss.  With mixup_fn the returned dict has no class_acc (the reference logs None there).
+    model_ema: an ema.ModelEma (or the reference's timm ModelEma) of this model, updated once per optimizer update (see
+    ema.resolve_model_ema for what is refused)."""
+    ema = resolve_model_ema(model_ema, model)
+    if train_head_only:
+        raise NotImplementedError("head-only training is not implemented in the fused stage-2 loop")
     smoothing = resolve_loss(criterion, mixup_fn)
     model.train(True)
     net = model.module if hasattr(model, "module") else model
@@ -149,7 +165,7 @@ def train_one_epoch(model: torch.nn.Module, criterion=None, data_loader: Iterabl
     gs = getattr(model, "grad_sync", None)
     if update_freq == 1:
         return _train_one_epoch_graphed(model, net, data_loader, optimizer, gs, max_norm, start_steps, lr_schedule_values,
-                                        wd_schedule_values, num_training_steps_per_epoch, mixup_fn, smoothing)
+                                        wd_schedule_values, num_training_steps_per_epoch, mixup_fn, smoothing, model_ema)
     mix = None if smoothing is None else MixBuffer(dev, mix_clips=mixup_fn is not None)
     loss_sum = torch.zeros(1, device=dev)
     loss_acc = torch.zeros(1, device=dev)
@@ -188,6 +204,8 @@ def train_one_epoch(model: torch.nn.Module, criterion=None, data_loader: Iterabl
             gn_sum += optimizer.grad_norm(scale)
             n_updates += 1
             optimizer.zero_grad()
+            if ema is not None:
+                ema.update(model)                                                  # engine_for_finetuning.py:126-127
     n = max(1, data_iter_step + 1)
     loss_avg = (loss_sum / n).item()
     if not math.isfinite(loss_avg):
@@ -203,10 +221,10 @@ def train_one_epoch(model: torch.nn.Module, criterion=None, data_loader: Iterabl
 
 
 def _train_one_epoch_graphed(model, net, data_loader, optimizer, gs, max_norm, start_steps, lr_schedule_values, wd_schedule_values,
-                             num_training_steps_per_epoch, mixup_fn=None, smoothing=None):
+                             num_training_steps_per_epoch, mixup_fn=None, smoothing=None, model_ema=None):
     """update_freq == 1 (the shipped stage-2 recipe): every loader batch is one whole update, run through Stage2Engine (CUDA-graph
     replay).  Same schedule handling and return dict as the general loop above."""
-    eng = _stage2_engine(model, net, optimizer, gs)
+    eng = _stage2_engine(model, net, optimizer, gs, model_ema)
     eng.max_norm = float(max_norm) if max_norm else None
     eng.stats.zero_()
     dev = eng.core.arena.device

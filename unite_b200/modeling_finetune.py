@@ -6,6 +6,7 @@ state_dict keys/shapes, so checkpoints and driver code (`model.patch_embed.patch
 `no_weight_decay()`) carry over.  The modules hold parameters only — the arithmetic is in vit_core.ViTTrunk
 and runs on the CUDA kernels; calling forward without a GPU raises.
 """
+from copy import deepcopy
 from functools import partial
 
 import numpy as np
@@ -170,6 +171,17 @@ class VisionTransformer(nn.Module):
             from .finetune_core import FinetuneCore
             self._core = FinetuneCore(self, dev)
         return self._core
+
+    def __deepcopy__(self, memo):
+        """A copy with its own parameters and no compute core (timm's ModelEma deep-copies the model, often after its arena
+        exists): the copy builds its own arena on first use and never shares the source's arena, bf16 shadow, tensor maps or
+        the engine / optimizer cached on the model (`_ub_*`).  Each parameter is cloned on its own (nn.Parameter.__deepcopy__),
+        so a parameter that is a view into the source's arena becomes a standalone tensor."""
+        new = self.__class__.__new__(self.__class__)
+        memo[id(self)] = new
+        state = {k: (None if k == "_core" else deepcopy(v, memo)) for k, v in self.__dict__.items() if not k.startswith("_ub_")}
+        new.__setstate__(state)
+        return new
 
     def _apply(self, fn, *a, **k):
         if self._core is not None:

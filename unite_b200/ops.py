@@ -434,6 +434,17 @@ def cast_bf16(x, out):
     check(lib.ub_cast_bf16(_p(x, F32, "x"), _p(out, BF16, "out"), x.numel(), _stream()), "ub_cast_bf16")
 
 
+@_instrument("ema_update", 1)
+def ema_update(ema_params, ema_w16, params, decay):
+    """ema_params = ema_params * decay + (1 - decay) * params in fp32 (timm ModelEma.update, bit for bit), and ema_w16 = its bf16
+    shadow, in one pass.  decay is rounded to fp32 and 1 - decay is computed in double first, as torch does with the scalars."""
+    n = ema_params.numel()
+    if params.numel() != n or ema_w16.numel() != n:
+        raise _cabi.UBError(f"ema_update: ema {n}, shadow {ema_w16.numel()} and params {params.numel()} elements differ")
+    check(lib.ub_ema_update(_p(ema_params, F32, "ema_params"), _p(ema_w16, BF16, "ema_w16"), _p(params, F32, "params"), n, float(decay),
+                            float(1.0 - decay), _stream()), "ub_ema_update")
+
+
 @_instrument("meanpool_fwd", 1)
 def meanpool_fwd(x, out):
     B, N, D = x.shape
