@@ -170,7 +170,7 @@ def test_graph_replayed_step_matches_an_eager_step():
     p0 = eng.core.arena.params.clone()
     eng.step(videos, q)                                           # captured, then replayed
     torch.cuda.synchronize()
-    assert len(eng._graphs) == 1
+    assert len(eng.graphs._graphs) == 1
     loss_g, mask_g = eng.loss.clone(), eng.last["mask"].clone()
     out_g, grads_g = eng.last["outputs"].clone(), eng.core.arena.grads.clone()
     eng.core.arena.params.copy_(p0)

@@ -90,7 +90,7 @@ def test_cuda_graph_step_draws_fresh_drop_path_factors_on_every_replay():
     for s in range(6):                                                            # 2 eager warm-up steps, then capture + replays
         losses.append(eng.step(videos, q).clone())
         torch.cuda.synchronize()
-    assert len(eng._graphs) == 1, "the DropPath step was not captured in a CUDA graph"
+    assert len(eng.graphs._graphs) == 1, "the DropPath step was not captured in a CUDA graph"
     n_draws = int(eng.drop_path.step.item())
     assert n_draws == 6, f"{n_draws} draws for 6 steps (capture itself must not consume a draw)"
     student2 = build_student(scfg, drop_path_rate=0.5)
@@ -486,7 +486,7 @@ def test_four_training_steps_track_the_oracle_with_torch_adamw():
         rel = abs(loss - ref["loss"].item()) / abs(ref["loss"].item())
         print(f"step {it}: loss {loss:.6f} vs {ref['loss'].item():.6f} ({rel:.1e})")
         assert rel < LOSS_TOL, (it, loss, ref["loss"].item())
-    assert len(eng._graphs) >= 1
+    assert len(eng.graphs._graphs) >= 1
     sd = student.state_dict()
     worst, worst_cos = 0.0, 1.0
     for k, p in ps.items():

@@ -1,7 +1,7 @@
 """A/B/A/B runs of bench.py on ONE box (boxes of the pool differ by +-2 %, so two settings are only comparable when they
 alternate on the same GPU).
 
-    python tools/ab_bench.py --a "" --b "UB_SIDE_WGRAD=2" [--rounds 2] [--steps 20] [--gpus 1]
+    python tools/ab_bench.py --a "" --b "UB_MULTI_WGRAD=0" [--rounds 2] [--steps 20] [--gpus 1]
 
 Each run is a fresh process (`bench.py --no-cpu-baseline`, UB_BENCH_U8=0 unless the setting says otherwise); prints one line per
 run and the per-setting medians of ms/step (device-resident) and of the e2e ms/step.  Takes ~15 s per single-GPU run.

@@ -159,7 +159,7 @@ def main():
     line = dict(
         metric="clips/sec (stage-1 step, ViT-B/16 student 8x224^2, CLIP ViT-L/14 teacher at 196 px)", value=round(clips_s, 2),
         unit="clips/s", ms_per_step=round(ms_step, 3), batch=B, steps=args.steps, warmup_steps_run=n_warm, cuda_graph=True,
-        graphs_captured=len(eng._graphs), drop_path=DROP_PATH, loss=round(loss.item(), 5),
+        graphs_captured=len(eng.graphs._graphs), drop_path=DROP_PATH, loss=round(loss.item(), 5),
         f_alg_gflop_per_clip={k: round(v, 1) for k, v in F.items()},
         mfu=dict(tflops=round(clips_s * F["total"] / 1e3, 1), of_nominal_2250=round(clips_s * F["total"] / 1e3 / NOMINAL_BF16_TFLOPS, 4)),
         teacher_forward=dict(ms=round(ms_teacher, 3), share_of_step=round(ms_teacher / ms_step, 4),

@@ -13,6 +13,8 @@ Nothing in the step reads a device value on the host: the loss and grad-norm sta
 """
 import math
 import os
+import sys
+import warnings
 from typing import Optional
 
 import torch
@@ -208,12 +210,13 @@ _ASYNC_ZERO = os.environ.get("UB_ASYNC_ZERO", "1") != "0"
 
 
 class GraphReplay:
-    """CUDA-graph plumbing shared by the stage-2 and stage-3 engines (Stage1Engine.step carries the same logic inline): the first
-    two steps of an input signature run eagerly (lazy attribute setting, workspace allocation, NCCL initialisation), then the
-    step body is captured once per set of persistent input buffers — callers that cycle through a few resident buffers get one
-    graph per buffer set, bound directly to them; past `max_graphs` sets the inputs are copied into one more graph that owns
-    private static inputs.  All graphs share one memory pool (they never run concurrently).  The body must be free of host
-    synchronisation and read its per-step scalars from device memory (FusedAdamW.prepare_step / step_dev)."""
+    """CUDA-graph plumbing of the step engines: the first two steps of an input signature run eagerly (lazy attribute setting,
+    workspace allocation, NCCL initialisation), then the step body is captured once per set of persistent input buffers — callers
+    that cycle through a few resident buffers (the staging ring of train_one_epoch, bench.py's resident batches) get one graph per
+    buffer set, bound directly to them, and no device-to-device copy into a static input per step; past `max_graphs` sets
+    (UB_MAX_GRAPHS, default 6; 0: always) the inputs are copied into one more graph that owns private static inputs.  All graphs
+    share one memory pool (they never run concurrently).  The body must be free of host synchronisation and read its per-step
+    scalars from device memory (FusedAdamW.prepare_step / step_dev)."""
 
     def __init__(self, max_graphs: Optional[int] = None):
         self.max_graphs = int(os.environ.get("UB_MAX_GRAPHS", "6")) if max_graphs is None else max_graphs
@@ -277,7 +280,95 @@ def require_fused_optimizer(optimizer, arena, what: str):
     return optimizer
 
 
-class Stage1Engine:
+class StepEngine:
+    """The data-parallel update shared by Stage1Engine, Stage2Engine and Stage3Engine.  Everything is read from the engine's
+    attributes when it is called (core, optimizer, grad_sync, nvls, max_norm, graphs), so a caller may swap any of them between
+    steps (bench.py's parity gate runs forward_backward with grad_sync = None)."""
+
+    @property
+    def grad_scale(self) -> float:
+        """The arena holds the SUM of every rank's gradients; AdamW and the reported grad-norm take 1 / world of it."""
+        return 1.0 / self.grad_sync.world if self.grad_sync is not None else 1.0
+
+    def _fused_step(self):
+        """N > 1: the all-reduce -> AdamW pair becomes ONE kernel over NVSwitch multicast (ddp.NvlsShardedStep) when the box
+        offers it; UB_DDP_NVLS=0 (or a box without multicast) keeps NCCL range all-reduces overlapped with backward (None)."""
+        gs = self.grad_sync
+        if gs is None or getattr(gs, "world", 1) <= 1 or self.core.arena.device.type != "cuda" \
+                or os.environ.get("UB_DDP_NVLS", "1") == "0" or not self.optimizer.plain_two_groups:
+            return None
+        from .ddp import NvlsShardedStep
+        try:
+            return NvlsShardedStep(self.core.arena, self.optimizer, gs.pg)
+        except Exception as e:                          # no multicast / symmetric memory on this box: NCCL path
+            if os.environ.get("UB_DDP_NVLS") == "1":
+                raise
+            warnings.warn(f"unite_b200: NVLS fused optimizer step unavailable ({type(e).__name__}: {e}); using NCCL all-reduce")
+            return None
+
+    def set_optimizer(self, optimizer: "FusedAdamW"):
+        """Swap in a caller-built FusedAdamW over the same arena (train_one_epoch's `optimizer` argument); the fused data-parallel
+        step, if active, is re-bound to it (its gradient-norm accumulator lives in symmetric memory)."""
+        if optimizer is self.optimizer:
+            return
+        require_fused_optimizer(optimizer, self.core.arena, f"{type(self).__name__}.set_optimizer")
+        if self.nvls is not None:
+            if not optimizer.plain_two_groups:
+                raise NotImplementedError("the fused NVLink step updates the plain [decay | no-decay] layout; layer-decay groups or "
+                                          "frozen parameters need UB_DDP_NVLS=0 (NCCL all-reduce + ub_adamw_seg)")
+            self.nvls.opt = optimizer
+            optimizer.gnorm_sq = self.optimizer.gnorm_sq
+            optimizer._sharded = self.nvls
+        self.optimizer = optimizer
+        self.graphs.clear()                     # captured graphs hold the old optimizer's buffers
+
+    def _backward_hook(self):
+        """Who is told, block by block, that a prefix of the gradient arena is final: the fused NVLink step (copy-engine pushes
+        to the owning ranks) or the NCCL path (range all-reduces); both overlap the rest of backward.  With clip_grad the fused
+        step needs the summed gradient first (NvlsShardedStep.step_dev_clipped), so nothing is pushed early."""
+        if self.nvls is not None:
+            return self.nvls if (self.nvls.early_push and not self.max_norm) else None
+        return self.grad_sync
+
+    def _update(self):
+        """After backward: reduce-scatter + AdamW + shadow all-gather in one kernel (the fused NVLink step), or the NCCL
+        all-reduce followed by grad-norm + AdamW.  Reads the scalars of the optimizer's last prepare_step."""
+        if self.nvls is not None:
+            if self.max_norm:
+                self.nvls.step_dev_clipped(self.max_norm)
+            else:
+                self.nvls.step_dev()
+            return
+        if self.grad_sync is not None:
+            self.grad_sync.all_reduce(self.core.arena.grads)
+        self.optimizer.step_dev(max_norm=self.max_norm)
+
+
+def apply_schedule(optimizer, it: int, lr_schedule_values=None, wd_schedule_values=None):
+    """Step `it` of the per-step lr / weight-decay schedules into the optimizer's param_groups: lr times the group's lr_scale
+    (layer decay), weight decay only in the groups that decay."""
+    for group in optimizer.param_groups:
+        if lr_schedule_values is not None:
+            group["lr"] = lr_schedule_values[min(it, len(lr_schedule_values) - 1)] * group.get("lr_scale", 1.0)
+        if wd_schedule_values is not None and group["weight_decay"] > 0:
+            group["weight_decay"] = wd_schedule_values[min(it, len(wd_schedule_values) - 1)]
+
+
+def schedule_stats(optimizer) -> dict:
+    """The lr / min_lr / weight_decay entries of the dict train_one_epoch returns."""
+    lrs = [g["lr"] for g in optimizer.param_groups]
+    wds = [g["weight_decay"] for g in optimizer.param_groups if g["weight_decay"] > 0]
+    return {"lr": max(lrs), "min_lr": min(lrs), "weight_decay": wds[0] if wds else None}
+
+
+def exit_if_not_finite(loss: float):
+    """A non-finite loss stops training, as the reference's loops do."""
+    if not math.isfinite(loss):
+        print("Loss is {}, stopping training".format(loss))
+        sys.exit(1)
+
+
+class Stage1Engine(StepEngine):
     def __init__(self, student: AdaptationVisionTransformer, teacher: ClipVisionTransformer, mask_ratio: float = 0.8,
                  lr: float = 1.5e-4, weight_decay: float = 0.05, betas=(0.9, 0.95), eps: float = 1e-8, grad_sync=None,
                  use_graph: bool = False, clip_loss_type: str = "l2", optimizer: Optional[FusedAdamW] = None):
@@ -291,28 +382,14 @@ class Stage1Engine:
         self.clip_loss_data = "mixed"         # 'source' / 'target': only the first B_s / the remaining clips enter the loss (:418-423)
         self.n_source = None                  # B_s of the current batch (needed when clip_loss_data != 'mixed')
         self.max_norm = None                  # clip_grad of the reference's loss_scaler call (run_stage1.py:451-455); None / 0 = off
-        self._graphs = {}
-        self._graph_count, self._graph_pool = {}, None
-        self.max_graphs_per_shape = int(os.environ.get("UB_MAX_GRAPHS", "6"))   # 0: always copy into private static inputs
-        self._eager_steps = {}
+        self.graphs = GraphReplay()
+        self._graphs = self.graphs._graphs    # the same dict: bench.py counts and drops a stage-1 engine's graphs through it
         self.core = student.core()
         self.core.sync_shadow(force=True)
         self.optimizer = require_fused_optimizer(optimizer, self.core.arena, "Stage1Engine") or \
             FusedAdamW(self.core.arena, lr, weight_decay, betas, eps)
         self.grad_sync = grad_sync            # unite_b200.ddp.GradSync or None
-        # N > 1: the all-reduce -> AdamW pair becomes ONE kernel over NVSwitch multicast (ddp.NvlsShardedStep) when the box
-        # offers it; UB_DDP_NVLS=0 (or a box without multicast) keeps NCCL range all-reduces overlapped with backward
-        self.nvls = None
-        if grad_sync is not None and getattr(grad_sync, "world", 1) > 1 and self.core.arena.device.type == "cuda" \
-                and os.environ.get("UB_DDP_NVLS", "1") != "0" and self.optimizer.plain_two_groups:
-            from .ddp import NvlsShardedStep
-            try:
-                self.nvls = NvlsShardedStep(self.core.arena, self.optimizer, grad_sync.pg)
-            except Exception as e:                      # no multicast / symmetric memory on this box: NCCL path
-                if os.environ.get("UB_DDP_NVLS") == "1":
-                    raise
-                import warnings
-                warnings.warn(f"unite_b200: NVLS fused optimizer step unavailable ({type(e).__name__}: {e}); using NCCL all-reduce")
+        self.nvls = self._fused_step()
         # the resolution the teacher sees (train_one_epoch's clip_input_resolution): a clip of another size is resized for the
         # teacher only (bicubic, on the device); the student always patchifies the clip as it comes
         self.teacher_resolution = teacher.input_resolution
@@ -322,23 +399,6 @@ class Stage1Engine:
         self.loss = torch.zeros(1, device=self.core.arena.device, dtype=F32)
         self.last = {}
         self.drop_path = self.core.drop_path       # vit_core.DropPathSource: device-side draws, one launch per step
-
-    def set_optimizer(self, optimizer: "FusedAdamW"):
-        """Swap in a caller-built FusedAdamW over the same arena (train_one_epoch's `optimizer` argument); the fused data-parallel
-        step, if active, is re-bound to it (its gradient-norm accumulator lives in symmetric memory)."""
-        if optimizer is self.optimizer:
-            return
-        require_fused_optimizer(optimizer, self.core.arena, "Stage1Engine.set_optimizer")
-        if self.nvls is not None:
-            if not optimizer.plain_two_groups:
-                raise NotImplementedError("the fused NVLink step updates the plain [decay | no-decay] layout; layer-decay groups or "
-                                          "frozen parameters need UB_DDP_NVLS=0 (NCCL all-reduce + ub_adamw_seg)")
-            self.nvls.opt = optimizer
-            optimizer.gnorm_sq = self.optimizer.gnorm_sq
-            optimizer._sharded = self.nvls
-        self.optimizer = optimizer
-        self._graphs.clear()                    # captured graphs hold the old optimizer's buffers
-        self._graph_count.clear()
 
     @property
     def share_patches(self) -> bool:
@@ -460,14 +520,6 @@ class Stage1Engine:
         self.last = dict(attn=attn, mask=mask.view(B, Tp * P).bool(), vis_idx=vis_idx[0], targets=targets, outputs=x_clip)
         return self.loss
 
-    def _backward_hook(self):
-        """Who is told, block by block, that a prefix of the gradient arena is final: the fused NVLink step (copy-engine pushes
-        to the owning ranks) or the NCCL path (range all-reduces); both overlap the rest of backward.  With clip_grad the fused
-        step needs the summed gradient first (NvlsShardedStep.step_dev_clipped), so nothing is pushed early."""
-        if self.nvls is not None:
-            return self.nvls if (self.nvls.early_push and not self.max_norm) else None
-        return self.grad_sync
-
     def _loss_clips(self, B):
         """Clip range [lo, hi) of the batch that enters the alignment loss (run_stage1.py:418-423); None = all ('mixed')."""
         if self.clip_loss_data == "mixed":
@@ -499,79 +551,18 @@ class Stage1Engine:
         else:
             self.optimizer.zero_grad()
         self.forward_backward(videos, q, None, grads_ready=zeroed)
-        if self.nvls is not None:
-            if self.max_norm:
-                self.nvls.step_dev_clipped(self.max_norm)
-            else:
-                self.nvls.step_dev()                    # reduce-scatter + AdamW + shadow all-gather, one kernel
-            return
-        if self.grad_sync is not None:
-            self.grad_sync.all_reduce(self.core.arena.grads)
-        self.optimizer.step_dev(max_norm=self.max_norm)
+        self._update()
 
     def step(self, videos, q, dp=None):
-        graphable = self.use_graph and dp is None
-        if not graphable:
+        self.optimizer.prepare_step(grad_scale=self.grad_scale)
+        if not self.use_graph or dp is not None:
+            # eager (bench.py's instrumented per-op step too): the arena fill stays in line, ahead of the step
             self.optimizer.zero_grad()
-            loss = self.forward_backward(videos, q, dp)
-            if self.nvls is not None:
-                self.optimizer.prepare_step(grad_scale=1.0 / self.nvls.world)
-                if self.max_norm:
-                    self.nvls.step_dev_clipped(self.max_norm)
-                else:
-                    self.nvls.step_dev()
-                return loss
-            scale = 1.0
-            if self.grad_sync is not None:
-                scale = self.grad_sync.all_reduce(self.core.arena.grads)
-            self.optimizer.step(grad_scale=scale, max_norm=self.max_norm)
-            return loss
+            self.forward_backward(videos, q, dp)
+            self._update()
+            return self.loss
         shape_key = (tuple(videos.shape), videos.dtype, tuple(q.shape), self.clip_loss_type, float(self.max_norm or 0.0),
                      self.clip_loss_data, self.n_source if self.clip_loss_data != "mixed" else None, bool(self.student.training))
-        scale = 1.0 / self.grad_sync.world if self.grad_sync is not None else 1.0
-        self.optimizer.prepare_step(grad_scale=scale)
-        n = self._eager_steps.get(shape_key, 0)
-        if n < 2:                                       # warm-up: lazy attribute setting, workspace allocation, NCCL init
-            self._eager_steps[shape_key] = n + 1
-            self._step_body_dev(videos, q)
-            return self.loss
-        # A graph is bound to the addresses of its inputs.  Callers that cycle through a few persistent device buffers (the
-        # staging ring of train_one_epoch, bench.py's resident batches) get one graph PER BUFFER PAIR, bound directly to those
-        # buffers (a reference is kept, so the addresses stay theirs) — all graphs share one memory pool, they never run
-        # concurrently — and no 154 MB device-to-device copy into a static input is needed per step.  Past max_graphs_per_shape
-        # distinct buffers, inputs are copied into one more graph that owns private static inputs (the general case).
-        buf_key = shape_key + (videos.data_ptr(), q.data_ptr())
-        if buf_key not in self._graphs:
-            private = self._graph_count.get(shape_key, 0) >= self.max_graphs_per_shape
-            if private:
-                buf_key = shape_key + ("private",)
-            if buf_key not in self._graphs:
-                sv, sq = (torch.empty_like(videos), torch.empty_like(q)) if private else (videos, q)
-                if private:
-                    sv.copy_(videos); sq.copy_(q)
-                torch.cuda.synchronize()
-                g = torch.cuda.CUDAGraph()
-                n0 = ops.LAUNCHES
-                # UB_SIDE_WGRAD=2: capture on a high-priority stream so that the kernel nodes of the critical path outrank the
-                # low-priority side stream of the weight-gradient GEMMs (vit_core._SIDE_WGRAD_FINE)
-                cap_stream = None
-                if os.environ.get("UB_SIDE_WGRAD", "0") == "2":
-                    if getattr(self, "_hi_stream", None) is None:
-                        self._hi_stream = torch.cuda.Stream(device=self.core.arena.device, priority=-1)
-                    cap_stream = self._hi_stream
-                with torch.cuda.graph(g, pool=self._graph_pool, stream=cap_stream):
-                    self._step_body_dev(sv, sq)
-                if self._graph_pool is None:
-                    self._graph_pool = g.pool()
-                n_kernels = ops.LAUNCHES - n0           # kernels of ours recorded in the graph (capture executes nothing)
-                ops.LAUNCHES = n0
-                self._graphs[buf_key] = (g, sv, sq, n_kernels, self.last)     # `last` = this graph's own mask / target / output tensors
-                self._graph_count[shape_key] = self._graph_count.get(shape_key, 0) + 1
-        g, sv, sq, n_kernels, self.last = self._graphs[buf_key]
-        ops.LAUNCHES += n_kernels                       # every replay launches all of them
-        if videos.data_ptr() != sv.data_ptr():
-            sv.copy_(videos, non_blocking=True)
-        if q.data_ptr() != sq.data_ptr():
-            sq.copy_(q, non_blocking=True)
-        g.replay()
+        # `last` = the mask / target / output tensors of the graph just replayed
+        self.last = self.graphs.run(shape_key, (videos, q), self._step_body_dev, state_fn=lambda: self.last)
         return self.loss

@@ -12,15 +12,15 @@ one in finetune_core.py; gradients accumulate in the parameter arena across micr
 With `model_ema` (ema.ModelEma or timm's ModelEma) the EMA arena is updated by one fused kernel (ub_ema_update) right after the
 optimizer, inside the CUDA graph of the step.
 """
-import math
-import sys
+import os
 from typing import Iterable, Optional
 
 import torch
 
 from . import ops
 from .ema import resolve_model_ema
-from .engine import FusedAdamW, require_fused_optimizer
+from .engine import (FusedAdamW, GraphReplay, StepEngine, apply_schedule, exit_if_not_finite, require_fused_optimizer,
+                     schedule_stats)
 from .mixup import NO_MIX, MixBuffer, draw, resolve_loss
 
 
@@ -62,7 +62,7 @@ def finetune_step(model, samples, targets, loss_acc, scale=1.0, grad_sync=None, 
     return logits
 
 
-class Stage2Engine:
+class Stage2Engine(StepEngine):
     """One whole stage-2 update (update_freq == 1): zero the gradient arena, forward, CE, backward, gradient all-reduce, grad-norm +
     layer-decay AdamW — engine_for_finetuning.py:116-127 — replayed from a CUDA graph after two eager steps (engine.GraphReplay):
     the ~750 launches of the all-token step then cost one launch.  DropPath draws come from the device-side generator, the
@@ -72,7 +72,6 @@ class Stage2Engine:
     of a data-parallel run updates its own EMA from the same replicated weights."""
 
     def __init__(self, model, optimizer: FusedAdamW, grad_sync=None, use_graph: bool = False, model_ema=None):
-        from .engine import GraphReplay
         self.ema = resolve_model_ema(model_ema, model)
         self.model = model
         self.net = model.module if hasattr(model, "module") else model
@@ -81,6 +80,7 @@ class Stage2Engine:
             self.ema.ema_net.core()                         # the EMA's arena exists before any step is captured
         self.optimizer = require_fused_optimizer(optimizer, self.core.arena, "Stage2Engine")
         self.grad_sync = grad_sync
+        self.nvls = None                                    # the update is the NCCL all-reduce + ub_adamw_seg
         self.use_graph = use_graph
         self.max_norm = None
         dev = self.core.arena.device
@@ -94,14 +94,12 @@ class Stage2Engine:
     def _body(self, samples, targets):
         self.optimizer.zero_grad()
         self.loss.zero_()
-        logits = finetune_step(self.model, samples, targets, self.loss, scale=1.0, grad_sync=self.grad_sync, mix=self._mix)
-        if self.grad_sync is not None:
-            self.grad_sync.all_reduce(self.core.arena.grads)
-        self.optimizer.step_dev(max_norm=self.max_norm)
+        logits = finetune_step(self.model, samples, targets, self.loss, scale=1.0, grad_sync=self._backward_hook(), mix=self._mix)
+        self._update()
         if self.ema is not None:
             self.ema.update(self.model)
-        scale = 1.0 / self.grad_sync.world if self.grad_sync is not None else 1.0
-        self.stats += torch.cat([self.loss, (logits.argmax(-1) == targets).sum().float().view(1), self.optimizer.grad_norm(scale)])
+        self.stats += torch.cat([self.loss, (logits.argmax(-1) == targets).sum().float().view(1),
+                                 self.optimizer.grad_norm(self.grad_scale)])
         self.logits = logits
 
     def step(self, samples, targets, private_inputs=False, mix=None, smoothing=None):
@@ -112,8 +110,7 @@ class Stage2Engine:
         replay of the one graph per loss kind reads its own draw."""
         if mix is not None and smoothing is None:
             raise ValueError("Stage2Engine.step: a mixup draw needs the soft-target loss (pass smoothing=)")
-        scale = 1.0 / self.grad_sync.world if self.grad_sync is not None else 1.0
-        self.optimizer.prepare_step(grad_scale=scale)
+        self.optimizer.prepare_step(grad_scale=self.grad_scale)
         kind = "ce" if smoothing is None else ("mix" if mix is not None else "smooth")
         self._mix = None
         if kind != "ce":
@@ -135,7 +132,6 @@ def _stage2_engine(model, net, optimizer, gs, model_ema=None):
     held = net.__dict__.get("_ub_stage2_engine")
     held_ema = None if held is None or held.ema is None else held.ema.source
     if held is None or held.optimizer is not optimizer or held.grad_sync is not gs or held_ema is not model_ema:
-        import os
         held = Stage2Engine(model, optimizer, grad_sync=gs, use_graph=os.environ.get("UB_NO_GRAPH", "0") != "1", model_ema=model_ema)
         net.__dict__["_ub_stage2_engine"] = held
     return held
@@ -180,13 +176,8 @@ def train_one_epoch(model: torch.nn.Module, criterion=None, data_loader: Iterabl
         step = data_iter_step // update_freq
         if num_training_steps_per_epoch is not None and step >= num_training_steps_per_epoch:
             continue                                                               # engine_for_finetuning.py:71-72
-        it = start_steps + step
-        if data_iter_step % update_freq == 0:
-            for group in optimizer.param_groups:                                   # engine_for_finetuning.py:76-81
-                if lr_schedule_values is not None:
-                    group["lr"] = lr_schedule_values[min(it, len(lr_schedule_values) - 1)] * group.get("lr_scale", 1.0)
-                if wd_schedule_values is not None and group["weight_decay"] > 0:
-                    group["weight_decay"] = wd_schedule_values[min(it, len(wd_schedule_values) - 1)]
+        if data_iter_step % update_freq == 0:                                      # engine_for_finetuning.py:76-81
+            apply_schedule(optimizer, start_steps + step, lr_schedule_values, wd_schedule_values)
         if mix is not None:
             mix.upload((draw(mixup_fn, samples.shape) if mixup_fn is not None else NO_MIX).packed(smoothing, core.C))
         samples = samples.to(dev, non_blocking=True)
@@ -208,13 +199,9 @@ def train_one_epoch(model: torch.nn.Module, criterion=None, data_loader: Iterabl
                 ema.update(model)                                                  # engine_for_finetuning.py:126-127
     n = max(1, data_iter_step + 1)
     loss_avg = (loss_sum / n).item()
-    if not math.isfinite(loss_avg):
-        print("Loss is {}, stopping training".format(loss_avg))
-        sys.exit(1)
-    lrs = [g["lr"] for g in optimizer.param_groups]
-    wds = [g["weight_decay"] for g in optimizer.param_groups if g["weight_decay"] > 0]
-    stats = {"loss": loss_avg, "class_acc": (correct / max(seen, 1)).item(), "loss_scale": 1.0, "lr": max(lrs), "min_lr": min(lrs),
-             "weight_decay": wds[0] if wds else None, "grad_norm": (gn_sum / max(1, n_updates)).item()}
+    exit_if_not_finite(loss_avg)
+    stats = {"loss": loss_avg, "class_acc": (correct / max(seen, 1)).item(), "loss_scale": 1.0, **schedule_stats(optimizer),
+             "grad_norm": (gn_sum / max(1, n_updates)).item()}
     if mixup_fn is not None:
         del stats["class_acc"]
     return stats
@@ -232,12 +219,7 @@ def _train_one_epoch_graphed(model, net, data_loader, optimizer, gs, max_norm, s
     for data_iter_step, batch in enumerate(data_loader):
         if num_training_steps_per_epoch is not None and data_iter_step >= num_training_steps_per_epoch:
             continue                                                               # engine_for_finetuning.py:71-72
-        it = start_steps + data_iter_step
-        for group in optimizer.param_groups:                                       # engine_for_finetuning.py:76-81
-            if lr_schedule_values is not None:
-                group["lr"] = lr_schedule_values[min(it, len(lr_schedule_values) - 1)] * group.get("lr_scale", 1.0)
-            if wd_schedule_values is not None and group["weight_decay"] > 0:
-                group["weight_decay"] = wd_schedule_values[min(it, len(wd_schedule_values) - 1)]
+        apply_schedule(optimizer, start_steps + data_iter_step, lr_schedule_values, wd_schedule_values)   # :76-81
         mix = draw(mixup_fn, batch[0].shape) if mixup_fn is not None else None
         eng.step(batch[0].to(dev, non_blocking=True), batch[1].to(dev, non_blocking=True), private_inputs=True, mix=mix,
                  smoothing=smoothing)
@@ -245,13 +227,9 @@ def _train_one_epoch_graphed(model, net, data_loader, optimizer, gs, max_norm, s
         n += 1
     loss_sum, correct, gn_sum = eng.stats.tolist()
     loss_avg = loss_sum / max(1, n)
-    if not math.isfinite(loss_avg):
-        print("Loss is {}, stopping training".format(loss_avg))
-        sys.exit(1)
-    lrs = [g["lr"] for g in optimizer.param_groups]
-    wds = [g["weight_decay"] for g in optimizer.param_groups if g["weight_decay"] > 0]
-    stats = {"loss": loss_avg, "class_acc": correct / max(seen, 1), "loss_scale": 1.0, "lr": max(lrs), "min_lr": min(lrs),
-             "weight_decay": wds[0] if wds else None, "grad_norm": gn_sum / max(1, n)}
+    exit_if_not_finite(loss_avg)
+    stats = {"loss": loss_avg, "class_acc": correct / max(seen, 1), "loss_scale": 1.0, **schedule_stats(optimizer),
+             "grad_norm": gn_sum / max(1, n)}
     if mixup_fn is not None:
         del stats["class_acc"]                                                     # the reference's class_acc = None under mixup
     return stats

@@ -9,13 +9,11 @@ Batches are `(videos, mask_placeholder, labels[, noise])`; without `noise` the E
 bicubic, when it differs from the clip's); None (the default here) means the teacher's own input_resolution, the only side its
 positional embedding fits.  A CLIP ViT-L/14 teacher behind a 16-pixel student at 224 px needs 196.
 """
-import math
-import sys
 from typing import Iterable, Optional
 
 import torch
 
-from .engine import Stage1Engine, require_fused_optimizer
+from .engine import Stage1Engine, apply_schedule, exit_if_not_finite, require_fused_optimizer, schedule_stats
 
 _IO = {}          # per device: copy stream, device staging ring, pinned loss read-back slots
 
@@ -130,9 +128,7 @@ def train_one_epoch(model: torch.nn.Module, data_loader: Iterable, data_loader_t
             loss_ev[slot] = None
             if eng.nvls is not None:
                 eng.nvls.raise_if(int(pin_err[slot][0]))                       # a peer stalled inside the fused data-parallel step
-            if not math.isfinite(last_loss):
-                print("Loss is {}, stopping training".format(last_loss))
-                sys.exit(1)
+            exit_if_not_finite(last_loss)                                      # run_stage1.py:447-449
 
     it_loader = iter(data_loader)
     nxt = next(it_loader, None)
@@ -141,12 +137,7 @@ def train_one_epoch(model: torch.nn.Module, data_loader: Iterable, data_loader_t
     while staged is not None:
         videos, noise, ev, slots, eng.n_source = staged
         nxt = next(it_loader, None)
-        it = start_steps + step
-        for group in opt.param_groups:                                         # run_stage1.py:326-338
-            if lr_schedule_values is not None:
-                group["lr"] = lr_schedule_values[min(it, len(lr_schedule_values) - 1)] * group.get("lr_scale", 1.0)
-            if wd_schedule_values is not None and group["weight_decay"] > 0:
-                group["weight_decay"] = wd_schedule_values[min(it, len(wd_schedule_values) - 1)]
+        apply_schedule(opt, start_steps + step, lr_schedule_values, wd_schedule_values)   # run_stage1.py:326-338
         torch.cuda.current_stream(dev).wait_event(ev)
         if noise is None:
             # fp32 clips are [B,3,T,H,W]; decoded uint8 frames are [B,T,H,W,3]
@@ -162,7 +153,7 @@ def train_one_epoch(model: torch.nn.Module, data_loader: Iterable, data_loader_t
             if sl is not None:
                 ring_free[sl[0]][sl[1]] = done
         loss_sum += loss
-        gn_sum += opt.grad_norm(1.0 / (eng.grad_sync.world if eng.grad_sync is not None else 1))
+        gn_sum += opt.grad_norm(eng.grad_scale)
         n += 1
         if log_freq and (step + 1) % log_freq == 0:
             slot = (step // log_freq) & 1
@@ -182,10 +173,5 @@ def train_one_epoch(model: torch.nn.Module, data_loader: Iterable, data_loader_t
         torch.distributed.all_reduce(stats)                                    # utils.py:239-241 (epoch-end meter sync)
         stats /= torch.distributed.get_world_size()
     loss_avg, gn_avg = stats.tolist()
-    if not math.isfinite(loss_avg):
-        print("Loss is {}, stopping training".format(loss_avg))
-        sys.exit(1)
-    lrs = [g["lr"] for g in opt.param_groups]
-    wds = [g["weight_decay"] for g in opt.param_groups if g["weight_decay"] > 0]
-    return {"loss": loss_avg, "loss_clip": loss_avg, "loss_scale": 1.0, "lr": max(lrs), "min_lr": min(lrs),
-            "weight_decay": wds[0] if wds else None, "grad_norm": gn_avg}
+    exit_if_not_finite(loss_avg)
+    return {"loss": loss_avg, "loss_clip": loss_avg, "loss_scale": 1.0, **schedule_stats(opt), "grad_norm": gn_avg}

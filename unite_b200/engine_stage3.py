@@ -14,21 +14,19 @@ The OpenAI-CLIP image/text towers of `clip_infer` are not available offline: the
 (clip.VisionTransformer.cls_features) and a caller-supplied text matrix [n_classes, 512] stand in (SURVEY.md §8(c)).
 No host synchronisation: |sel| never leaves the device — tgt_ratio*|sel|/B_t*mean_sel(w*CE) == tgt_ratio/B_t * sum_b sel_b*w_b*CE_b.
 """
-from typing import Optional
+import os
+from typing import Iterable, Optional
 
 import torch
 
-import math
-import sys
-from typing import Iterable
-
 from . import ops
-from .engine import FusedAdamW, require_fused_optimizer
+from .engine import (FusedAdamW, GraphReplay, StepEngine, apply_schedule, exit_if_not_finite, require_fused_optimizer,
+                     schedule_stats)
 
 BF16, F32, I32, U8 = torch.bfloat16, torch.float32, torch.int32, torch.uint8
 
 
-class Stage3Engine:
+class Stage3Engine(StepEngine):
     def __init__(self, student, teacher, cls_weight: torch.Tensor, cls_bias: torch.Tensor, text_features: torch.Tensor,
                  mask_ratio: float = 0.8, k: int = 2, clip_threshold: float = 0.5, src_ratio: float = 1.0, tgt_ratio: float = 1.0,
                  conf_weighted: bool = True, lr: float = 1e-4, weight_decay: float = 0.05, betas=(0.9, 0.999), grad_sync=None,
@@ -36,7 +34,6 @@ class Stage3Engine:
         """use_graph: after two eager steps of a batch signature the whole step (the five forwards, both backwards, the gradient
         exchange and AdamW: ~900 launches) is captured in a CUDA graph and replayed (engine.GraphReplay); nothing in it reads a
         device value on the host, DropPath factors and optimizer scalars come from device memory."""
-        from .engine import GraphReplay
         if teacher.patch_size != 16:
             # the zero-shot head stands the teacher's CLS embedding in for OpenAI CLIP's image tower against a 512-wide text
             # matrix; which stand-in a ViT-L/14 teacher should provide is not settled
@@ -58,18 +55,7 @@ class Stage3Engine:
         self.grad_sync = grad_sync
         # N > 1: the same fused NVLink step as stage 1 (the student's arena is the same; src_classifier is a separate, frozen
         # module, run_stage3.py:1193/:1264): gradient pushes overlapped with the step's last backward, then ub_adamw_nvls
-        self.nvls = None
-        import os
-        if grad_sync is not None and getattr(grad_sync, "world", 1) > 1 and dev.type == "cuda" \
-                and os.environ.get("UB_DDP_NVLS", "1") != "0" and self.optimizer.plain_two_groups:
-            from .ddp import NvlsShardedStep
-            try:
-                self.nvls = NvlsShardedStep(self.core.arena, self.optimizer, grad_sync.pg)
-            except Exception as e:                      # no multicast / symmetric memory on this box: NCCL path
-                if os.environ.get("UB_DDP_NVLS") == "1":
-                    raise
-                import warnings
-                warnings.warn(f"unite_b200: NVLS fused optimizer step unavailable ({type(e).__name__}: {e}); using NCCL all-reduce")
+        self.nvls = self._fused_step()
         self.loss = torch.zeros(1, device=dev, dtype=F32)
         self.loss_s = torch.zeros(1, device=dev, dtype=F32)
         self.loss_t = torch.zeros(1, device=dev, dtype=F32)
@@ -166,10 +152,7 @@ class Stage3Engine:
         dl_t = torch.empty(Bt, C, device=dev, dtype=F32)
         ops.softmax_ce(logits_masked[k - 1], pseudo, weight, self.tgt_ratio / Bt, self.loss_t, dl_t)
         # the step's LAST backward: every gradient range it completes is final, so the NCCL range all-reduces overlap it
-        hook = self.grad_sync
-        if self.nvls is not None:
-            hook = self.nvls if (self.nvls.early_push and not self.max_norm) else None
-        self._backward_from_logits(st_m, pooled_m, dl_t, T * n_vis, grad_sync=hook)
+        self._backward_from_logits(st_m, pooled_m, dl_t, T * n_vis, grad_sync=self._backward_hook())
         self.loss.copy_(self.loss_s + self.loss_t)
         self.last = dict(attn=attn, masks=mask.view(k, frames, P).bool(), logits_s=logits_s, logits_full_t=logits_full_t,
                          logits_masked=logits_masked, clip_probs=clip_probs, sel_mask=sel.bool(), pseudo=pseudo, msp=msp)
@@ -178,20 +161,11 @@ class Stage3Engine:
     def _step_body_dev(self, videos_s, labels_s, videos_t, videos_t_aug):
         self.optimizer.zero_grad()
         self.forward_backward(videos_s, labels_s, videos_t, videos_t_aug)
-        if self.nvls is not None:
-            if self.max_norm:
-                self.nvls.step_dev_clipped(self.max_norm)
-            else:
-                self.nvls.step_dev()
-            return
-        if self.grad_sync is not None:
-            self.grad_sync.all_reduce(self.core.arena.grads)
-        self.optimizer.step_dev(max_norm=self.max_norm)
+        self._update()
 
     def step(self, videos_s, labels_s, videos_t, videos_t_aug=None, private_inputs=False):
         """One update.  private_inputs: the batch lives in fresh tensors every step (a loader), so a graph keeps its own inputs."""
-        world = self.nvls.world if self.nvls is not None else (self.grad_sync.world if self.grad_sync is not None else 1)
-        self.optimizer.prepare_step(grad_scale=1.0 / world)
+        self.optimizer.prepare_step(grad_scale=self.grad_scale)
         if videos_t_aug is videos_t:
             videos_t_aug = None
         if not self.use_graph:
@@ -224,18 +198,12 @@ def _engine_for(model, teacher_model, src_classifier, optimizer, mask_ratio, arg
                            tgt_ratio=float(getattr(args, "class_loss_tgt_ratio", 1.0)),
                            conf_weighted=bool(getattr(args, "conf_weighted_loss", True)), grad_sync=gs,
                            optimizer=require_fused_optimizer(optimizer, student.core().arena, "train_one_epoch"),
-                           use_graph=__import__("os").environ.get("UB_NO_GRAPH", "0") != "1")
+                           use_graph=os.environ.get("UB_NO_GRAPH", "0") != "1")
         student.__dict__["_ub_stage3_engine"] = (teacher, cls, eng)
         return eng
     eng = held[2]
-    if optimizer is not None and optimizer is not eng.optimizer:
-        new = require_fused_optimizer(optimizer, eng.core.arena, "train_one_epoch")
-        if eng.nvls is not None:
-            if not new.plain_two_groups:
-                raise NotImplementedError("the fused NVLink step updates the plain [decay | no-decay] layout (UB_DDP_NVLS=0 otherwise)")
-            eng.nvls.opt, new.gnorm_sq, new._sharded = new, eng.optimizer.gnorm_sq, eng.nvls
-        eng.optimizer = new
-        eng.graphs.clear()                      # captured graphs hold the old optimizer's buffers
+    if optimizer is not None:
+        eng.set_optimizer(require_fused_optimizer(optimizer, eng.core.arena, "train_one_epoch"))
     eng.mask_ratio = mask_ratio
     return eng
 
@@ -274,12 +242,7 @@ def train_one_epoch(model: torch.nn.Module, data_loader: Iterable, data_loader_t
     it_target = iter(data_loader_train_target)
     dual = bool(getattr(args, "return_aug_for_val", True))
     for step, batch in enumerate(data_loader):
-        it = start_steps + step
-        for group in opt.param_groups:                                           # run_stage3.py:383-396
-            if lr_schedule_values is not None:
-                group["lr"] = lr_schedule_values[min(it, len(lr_schedule_values) - 1)] * group.get("lr_scale", 1.0)
-            if wd_schedule_values is not None and group["weight_decay"] > 0:
-                group["weight_decay"] = wd_schedule_values[min(it, len(wd_schedule_values) - 1)]
+        apply_schedule(opt, start_steps + step, lr_schedule_values, wd_schedule_values)   # run_stage3.py:383-396
         videos_s, labels_s = batch[0], batch[1]
         try:
             tb = next(it_target)
@@ -290,8 +253,7 @@ def train_one_epoch(model: torch.nn.Module, data_loader: Iterable, data_loader_t
         videos_t_aug = tb[1].to(dev, non_blocking=True) if dual else None
         loss = eng.step(videos_s.to(dev, non_blocking=True), labels_s.to(dev, non_blocking=True), videos_t, videos_t_aug,
                         private_inputs=True)
-        scale = 1.0 / eng.grad_sync.world if eng.grad_sync is not None else 1.0
-        acc += torch.cat([loss, eng.loss_s, eng.loss_t, opt.grad_norm(scale)])
+        acc += torch.cat([loss, eng.loss_s, eng.loss_t, opt.grad_norm(eng.grad_scale)])
         n += 1
         if lr_scheduler is not None:
             lr_scheduler.step_update(start_steps + step)
@@ -300,10 +262,6 @@ def train_one_epoch(model: torch.nn.Module, data_loader: Iterable, data_loader_t
         torch.distributed.all_reduce(stats)                                      # metric_logger.synchronize_between_processes (:705)
         stats /= torch.distributed.get_world_size()
     loss_avg, ls_avg, lt_avg, gn_avg = stats.tolist()
-    if not math.isfinite(loss_avg):
-        print("Loss is {}, stopping training".format(loss_avg))
-        sys.exit(1)
-    lrs = [g["lr"] for g in opt.param_groups]
-    wds = [g["weight_decay"] for g in opt.param_groups if g["weight_decay"] > 0]
-    return {"loss": loss_avg, "loss_class": ls_avg, "loss_class_t": lt_avg, "loss_scale": 1.0, "lr": max(lrs), "min_lr": min(lrs),
-            "weight_decay": wds[0] if wds else None, "grad_norm": gn_avg}
+    exit_if_not_finite(loss_avg)                                                 # :640-642
+    return {"loss": loss_avg, "loss_class": ls_avg, "loss_class_t": lt_avg, "loss_scale": 1.0, **schedule_stats(opt),
+            "grad_norm": gn_avg}

@@ -25,25 +25,9 @@ from .arena import ParamArena
 BF16, F32 = torch.bfloat16, torch.float32
 
 
-# measured on B200 (round 1): no gain — every GEMM is a persistent one-CTA-per-SM grid, so two of them cannot share SMs and
-# the tails they could fill are short; kept as an option (UB_SIDE_WGRAD=1)
-_SIDE_WGRAD = os.environ.get("UB_SIDE_WGRAD", "0") in ("1", "2")
-# UB_SIDE_WGRAD=2 (end of round 1; one measurement: correct, 18.48 ms vs 17.6-18.0 ms default -> no gain as written): the
-# side-stream weight-gradient GEMMs become
-# NON-persistent single-CTA grids with finer split-K (work items of ~24 k-blocks) while the step itself is captured on a
-# high-priority stream (engine.Stage1Engine), so the block scheduler fills idle SMs with weight-gradient CTAs and hands every SM
-# back to the critical path at the next CTA boundary.  The persistent form could not do that: its CTAs keep an SM for their
-# whole static tile list, which is why UB_SIDE_WGRAD=1 measured no gain.
-_SIDE_WGRAD_FINE = os.environ.get("UB_SIDE_WGRAD", "0") == "2"
 # fc1 bias gradient accumulated by the epilogue of the GEMM that produces d_pre (ub_gemm_epilogue.colsum_out) instead of a
 # separate column-sum pass over d_pre: 12 launches and 12 x 63 MB of reads fewer per ViT-B step
 _FUSE_COLSUM = os.environ.get("UB_FUSE_COLSUM", "0") == "1"
-# The bias-gradient column sums of d_pre / dqkv (24 launches, ~0.35 ms per ViT-B step) feed nothing before the optimizer.  Unlike
-# the weight-gradient GEMMs they are small CTAs (256 threads, 8 KB smem, ~32 registers); UB_SIDE_COLSUM=1 puts them on a side stream
-# so that they could run under the dgrad / wgrad GEMMs instead of between them.  Measured on B200 (A/B/A/B, 20 steps each): 17.63 /
-# 17.66 ms with, 17.71 / 17.52 ms without — no gain: a GEMM CTA holds ~227 KB of the SM's 228 KB of shared memory, so nothing
-# co-resides with it and the column sums still wait for a GEMM to drain.  Off by default.
-_SIDE_COLSUM = os.environ.get("UB_SIDE_COLSUM", "0") == "1"
 # q_bias / v_bias gradients accumulated by the attention backward kernels while they store dq / dv (ub_attn_bwd's dbias) instead
 # of a separate column-sum pass over dqkv: 12 launches fewer per ViT-B step.  UB_FUSE_QKV_BIAS=0 restores the separate pass.
 _FUSE_QKV_BIAS = os.environ.get("UB_FUSE_QKV_BIAS", "1") == "1"
@@ -134,7 +118,8 @@ class TrunkWorkspace:
             self.layers.append(L)
         if save:  # backward temporaries, shared by all layers
             self.dx = torch.empty(M, D, device=dev, dtype=F32)
-            # consumed by the weight-gradient GEMMs, which run one layer behind on a side stream: two copies (layer parity)
+            # two copies (layer parity): block l's weight gradients are one launch at the END of its backward (UB_MULTI_WGRAD), and
+            # before it runs, block l's norm1 LayerNorm backward writes dxs_m of layer l-1, while the launch still reads layer l's
             self.dxs_m = [torch.empty(M, D, device=dev, dtype=BF16) for _ in range(2)]     # gradient entering the MLP branch
             self.dxs_a = [torch.empty(M, D, device=dev, dtype=BF16) for _ in range(2)]     # ... the attention branch
             self.d_pre2 = [torch.empty(M, hidden, device=dev, dtype=BF16) for _ in range(2)]
@@ -161,16 +146,6 @@ class ViTTrunk:
         self.scale = 64 ** -0.5
         self.sms = ops.lib.ub_sm_count() if torch.cuda.is_available() else 148
         self._ws: Dict = {}
-
-    def _colsum_stream(self):
-        if getattr(self, "_cs", None) is None:
-            self._cs = torch.cuda.Stream(device=self.arena.device)
-        return self._cs
-
-    def _side_stream(self):
-        if getattr(self, "_side", None) is None:
-            self._side = torch.cuda.Stream(device=self.arena.device, priority=0)     # lowest priority
-        return self._side
 
     # -- parameter access ---------------------------------------------------------------------
     def w(self, name):       # bf16 shadow (GEMM operand)
@@ -240,10 +215,6 @@ class ViTTrunk:
     # -- backward -----------------------------------------------------------------------------
     def _wgrad(self, dy, x_in, gw):
         """gw[out,in] += dy[M,out]^T @ x_in[M,in]  (contraction over tokens, both operands MN-major)."""
-        if _SIDE_WGRAD_FINE and dy.is_cuda:
-            kb = (dy.shape[0] + 63) // 64                                  # k-blocks of the token contraction
-            ops.gemm(dy, x_in, gw, a_t=True, b_t=True, accumulate=True, split_k=max(1, min(32, kb // 24)), tile_ctas=1, max_ctas=-1)
-            return
         ops.gemm(dy, x_in, gw, a_t=True, b_t=True, accumulate=True, split_k=_splits_for(gw.shape[0], gw.shape[1], self.sms))
 
     def backward(self, ws: TrunkWorkspace, tap_grads: Dict[int, callable], dx_init: bool = False, on_block_done=None):
@@ -257,59 +228,20 @@ class ViTTrunk:
         dp = ws.dp
         have_dx = dx_init
         nl = ws.n_layers
-        # Weight gradients are off the critical path (nothing reads them before the optimizer): they are issued on a side
-        # stream so their CTAs fill the SMs the dgrad / attention / LayerNorm chain leaves idle (wave tails, small grids).
-        side = self._side_stream() if (_SIDE_WGRAD and ws.dx.is_cuda) else None
-        main = torch.cuda.current_stream() if side is not None else None
-        side_done = {}
-
-        multi = _MULTI_WGRAD and side is None and ws.dx.is_cuda
+        multi = _MULTI_WGRAD and ws.dx.is_cuda
         pending = []                                    # this block's (dy, x, gw) triples, issued as one launch at its end
 
         def wgrad(dy, x_in, gw):
             if multi:
                 pending.append((dy, x_in, gw))
-                return
-            if side is None:
-                return self._wgrad(dy, x_in, gw)
-            ev = torch.cuda.Event()
-            ev.record(main)
-            side.wait_event(ev)
-            with torch.cuda.stream(side):
+            else:
                 self._wgrad(dy, x_in, gw)
-
-        def block_final(l):
-            if on_block_done is not None:
-                on_block_done(l)     # every gradient of block l is final: its arena range can be all-reduced
-
-        # column sums beside the GEMMs (see _SIDE_COLSUM): cs_done[par] = the side stream has finished reading the scratch of
-        # layer parity `par`; the main stream waits for it before a later layer overwrites that scratch
-        cs = self._colsum_stream() if (_SIDE_COLSUM and side is None and ws.dx.is_cuda) else None
-        cs_main = torch.cuda.current_stream() if cs is not None else None
-        cs_done = {}
-
-        def colsum(x, out, skip=(0, 0), par=None):
-            if cs is None:
-                return ops.colsum_bf16(x, out, skip=skip)
-            ev = torch.cuda.Event()
-            ev.record(cs_main)
-            cs.wait_event(ev)
-            with torch.cuda.stream(cs):
-                ops.colsum_bf16(x, out, skip=skip)
-                done = torch.cuda.Event()
-                done.record(cs)
-            cs_done[par] = done
 
         for l in reversed(range(nl)):
             L = ws.layer(l)
             b = f"blocks.{l}."
             par = l & 1
             dxs_m, dxs_a, d_pre, dqkv = ws.dxs_m[par], ws.dxs_a[par], ws.d_pre2[par], ws.dqkv2[par]
-            if cs is not None and par in cs_done:
-                cs_main.wait_event(cs_done.pop(par))     # layer l + 2's column sums are done with d_pre / dqkv of this parity
-            if side is not None and (l + 2) in side_done:
-                main.wait_event(side_done[l + 2])        # the scratch of this parity is free again
-                block_final(l + 2)
             s_mlp = None if dp is None else dp[l, 1]
             s_att = None if dp is None else dp[l, 0]
             # the producer of dxs also accumulates its column sums = the bias gradient of the Linear it feeds
@@ -321,7 +253,6 @@ class ViTTrunk:
                 ops.cast_scale_bf16(ws.dx, dxs_m, s_mlp, N)
                 ops.colsum_bf16(dxs_m, self.g(b + "mlp.fc2.bias"))
             # ---- MLP branch: x_out = x_mid + s * (gelu(h2 W1^T + b1) W2^T + b2)
-            # (each side-stream GEMM is enqueued AFTER the critical-path kernel it runs beside, so the latter gets the SMs first)
             # with _FUSE_COLSUM the fc1 bias gradient (column sums of d_pre) is accumulated by this GEMM's epilogue
             ops.gemm(dxs_m, self.w(b + "mlp.fc2.weight"), d_pre, b_t=True, act=ops.UB_ACT_DGELU, aux_in=L.pre,
                      colsum_out=self.g(b + "mlp.fc1.bias") if _FUSE_COLSUM else None)
@@ -329,7 +260,7 @@ class ViTTrunk:
             ops.gemm(d_pre, self.w(b + "mlp.fc1.weight"), ws.d_h, b_t=True)
             wgrad(d_pre, L.h2, self.g(b + "mlp.fc1.weight"))
             if not _FUSE_COLSUM:
-                colsum(d_pre, self.g(b + "mlp.fc1.bias"), par=par)
+                ops.colsum_bf16(d_pre, self.g(b + "mlp.fc1.bias"))
             ops.layernorm_bwd(ws.d_h, L.x_mid, self.p(b + "norm2.weight"), self.eps, ws.dx, ws.dx, dxs_a, s_att, N,
                               self.g(b + "norm2.weight"), self.g(b + "norm2.bias"), dsum=self.g(b + "attn.proj.bias"))
             # ---- attention branch: x_mid = x_in + s * (attn(h1) Wp^T + bp)
@@ -347,7 +278,7 @@ class ViTTrunk:
             ops.gemm(dqkv, self.w(b + "attn.qkv.weight"), ws.d_h, b_t=True)
             wgrad(dqkv, L.h1, self.g(b + "attn.qkv.weight"))
             if not _FUSE_QKV_BIAS:
-                colsum(dqkv, self.qkv_bias_grad(l), skip=(D, 2 * D), par=par)
+                ops.colsum_bf16(dqkv, self.qkv_bias_grad(l), skip=(D, 2 * D))
             # next consumer of dxs: block l-1's MLP branch (unless a tap re-emits it) or the patch embedding
             emit = (l - 1) not in tap_grads
             s_next = None if (dp is None or l == 0) else dp[l - 1, 1]
@@ -358,17 +289,8 @@ class ViTTrunk:
             if multi:
                 ops.gemm_wgrad_multi(pending, split_k=_multi_splits(pending, max(1, self.sms // 2)))
                 pending.clear()
-            if side is not None:
-                side_done[l] = torch.cuda.Event()
-                side_done[l].record(side)
-            else:
-                block_final(l)
-        if side is not None:
-            main.wait_stream(side)
-            for l in reversed(range(min(2, nl))):
-                block_final(l)
-        if cs is not None:
-            cs_main.wait_stream(cs)          # bias gradients are complete before anything downstream (all-reduce, optimizer) runs
+            if on_block_done is not None:
+                on_block_done(l)     # every gradient of block l is final: its arena range can be all-reduced
         # ---- patch embedding (Conv3d as GEMM): only weight and bias gradients exist
         gw = self.g("patch_embed.proj.weight")
         self._wgrad(ws.dxs_m[1], ws.patches, gw.view(D, -1))
