@@ -214,6 +214,11 @@ UB_API int ub_patchify_mix(const float* x, void* out, const float* mix, int B, i
  * (src/datasets/kinetics_sparse.py:236-243, 434-451); mean3 / std3 are HOST pointers to 3 floats.                     */
 UB_API int ub_patchify_u8(const uint8_t* x, void* out, const float* mean3, const float* std3, int B, int T, int H, int W,
                           int tubelet, void* stream);
+/* ub_patchify_mix of the frames ub_patchify_u8 reads: every byte normalised exactly as there, then mixed exactly as ub_patchify_mix
+ * mixes (mix: the same DEVICE draw), so the rows equal ub_patchify of the torch-mixed normalised clip.  x is not written;
+ * B even, H and W multiples of 16, x 16-byte aligned; mean3 / std3 are HOST pointers to 3 floats. */
+UB_API int ub_patchify_mix_u8(const uint8_t* x, void* out, const float* mix, const float* mean3, const float* std3, int B, int T, int H,
+                              int W, int tubelet, void* stream);
 /* resize + patchify for the teacher: fp32 clip [B,3,T,H,W] (x_is_u8 = 0) or decoded uint8 frames [B,T,H,W,3] (x_is_u8 = 1,
  * normalised with the HOST mean3 / std3 as ub_patchify_u8 does, before the resize) -> bicubic resize of every (c, t) plane to
  * R x R (torch interpolate mode="bicubic", align_corners=False, antialias=False; no resize when R == H == W) -> bf16 im2col rows

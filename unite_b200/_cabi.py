@@ -92,6 +92,7 @@ SIGNATURES = {
     "ub_patchify": (C.c_int, [_P, _P, _I, _I, _I, _I, _I, _P]),
     "ub_patchify_mix": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "ub_patchify_u8": (C.c_int, [_P, _P, C.POINTER(C.c_float), C.POINTER(C.c_float), _I, _I, _I, _I, _I, _P]),
+    "ub_patchify_mix_u8": (C.c_int, [_P, _P, _P, C.POINTER(C.c_float), C.POINTER(C.c_float), _I, _I, _I, _I, _I, _P]),
     "ub_resize_patchify": (C.c_int, [_P, _I, C.POINTER(C.c_float), C.POINTER(C.c_float), _P, _L, _I, _I, _I, _I, _I, _I, _I, _P]),
     "ub_mask_select": (C.c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "ub_gather_rows": (C.c_int, [_P, _P, _P, _L, _L, _I, _L, _P]),

@@ -3,6 +3,7 @@
 //   ub_patchify      fp32 clip -> bf16 im2col rows (the A operand of the stride==kernel Conv3d as a GEMM)
 //                    clip.py:123-128,146 (teacher conv1), modeling_finetune.py:165-174 (student PatchEmbed.proj)
 //   ub_patchify_mix  the same rows of the batch-mode mixup / cutmix of the clip (stage-2 mixup_fn), x left untouched
+//   ub_patchify_u8 / ub_patchify_mix_u8   the same two from decoded uint8 frames, normalised on the way
 //   ub_mask_select   attention-guided visible-token selection, bit-exact
 //                    run_stage1.py:379-387 (multinomial == top-N_vis of attn/q, q ~ Exp(1) supplied by the caller)
 //                    utils.py:89-120 get_greedy_masks (k committee members take ranks i, i+k, ...; q == NULL)
@@ -122,38 +123,132 @@ __global__ void __launch_bounds__(256) patchify_mix_kernel(const float* __restri
 // One thread = one (token, kt, kh) run of 16 pixels: 48 contiguous bytes in, three 32-byte runs out (one per channel).
 // The step then needs 38.5 MB of H2D per 32-clip batch instead of the 154 MB fp32 clip.
 // ------------------------------------------------------------------------------------------------
+// One run of the THWC frames: clip b, frame t, pixel row h, the 16 pixels from column w, of token `tok` at (kt, kh).
+struct U8Run {
+  long tok;
+  int b, t, h, w, kt, kh;
+};
+
+UB_DEVINL U8Run u8_run(long id, int T, int H, int W, int tub) {
+  const int gh = H / 16, gw = W / 16, Tp = T / tub;
+  const int runs_per_tok = tub * 16;          // (kt, kh)
+  U8Run r;
+  const int run = (int)(id % runs_per_tok);
+  r.tok = id / runs_per_tok;
+  r.kh = run % 16;
+  r.kt = run / 16;
+  const int pw = (int)(r.tok % gw), ph = (int)((r.tok / gw) % gh), tp = (int)((r.tok / ((long)gw * gh)) % Tp);
+  r.b = (int)(r.tok / ((long)gw * gh * Tp));
+  r.t = tp * tub + r.kt;
+  r.h = ph * 16 + r.kh;
+  r.w = pw * 16;
+  return r;
+}
+
+// byte offset of the run's first pixel in x, and element offset of its channel-0 segment in the im2col rows
+UB_DEVINL long u8_src(const U8Run& r, int T, int H, int W) { return ((((long)r.b * T + r.t) * H + r.h) * W + r.w) * 3; }
+UB_DEVINL long u8_dst(const U8Run& r, int tub) { return r.tok * (long)(3 * tub * 256) + r.kt * 256 + r.kh * 16; }
+
+// the run's 48 bytes (16 pixels x RGB), one 16-byte load per third
+UB_DEVINL void u8_load(const uint8_t* src, uint32_t* w) {
+  *reinterpret_cast<uint4*>(&w[0]) = ldg_nc_v4(src);
+  *reinterpret_cast<uint4*>(&w[4]) = ldg_nc_v4(src + 16);
+  *reinterpret_cast<uint4*>(&w[8]) = ldg_nc_v4(src + 32);
+}
+
+// ToTensor + tensor_normalize of one byte: (u / 255 - mean) / std, each step an IEEE-rounded fp32 operation
+UB_DEVINL float u8_norm(uint8_t u, float mean, float sd) { return __fdiv_rn(__fsub_rn(__fdiv_rn((float)u, 255.0f), mean), sd); }
+
 __global__ void __launch_bounds__(256) patchify_u8_kernel(const uint8_t* __restrict__ x, bf16* __restrict__ out, float m0, float m1,
                                                           float m2, float s0, float s1, float s2, int B, int T, int H, int W, int tub,
                                                           long total_runs) {
   pdl_grid_sync();
-  const int gh = H / 16, gw = W / 16, Tp = T / tub;
-  const int runs_per_tok = tub * 16;          // (kt, kh)
-  const int feat = 3 * tub * 256;
   const float mean[3] = {m0, m1, m2}, sd[3] = {s0, s1, s2};
   for (long id = (long)blockIdx.x * blockDim.x + threadIdx.x; id < total_runs; id += (long)gridDim.x * blockDim.x) {
-    const int run = (int)(id % runs_per_tok);
-    const long tok = id / runs_per_tok;
-    const int kh = run % 16, kt = run / 16;
-    const int pw = (int)(tok % gw), ph = (int)((tok / gw) % gh), tp = (int)((tok / ((long)gw * gh)) % Tp);
-    const int b = (int)(tok / ((long)gw * gh * Tp));
-    const uint8_t* src = x + ((((long)b * T + (tp * tub + kt)) * H + (ph * 16 + kh)) * W + pw * 16) * 3;
+    const U8Run r = u8_run(id, T, H, W, tub);
     uint32_t w[12];
-    *reinterpret_cast<uint4*>(&w[0]) = ldg_nc_v4(src);
-    *reinterpret_cast<uint4*>(&w[4]) = ldg_nc_v4(src + 16);
-    *reinterpret_cast<uint4*>(&w[8]) = ldg_nc_v4(src + 32);
+    u8_load(x + u8_src(r, T, H, W), w);
     const uint8_t* by = reinterpret_cast<const uint8_t*>(w);
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
       uint32_t o[8];
 #pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        const float a = __fdiv_rn(__fsub_rn(__fdiv_rn((float)by[(2 * i) * 3 + c], 255.0f), mean[c]), sd[c]);
-        const float d = __fdiv_rn(__fsub_rn(__fdiv_rn((float)by[(2 * i + 1) * 3 + c], 255.0f), mean[c]), sd[c]);
-        o[i] = pack_bf16x2(a, d);
-      }
-      bf16* dst = out + tok * (long)feat + (long)c * (tub * 256) + kt * 256 + kh * 16;
+      for (int i = 0; i < 8; ++i)
+        o[i] = pack_bf16x2(u8_norm(by[(2 * i) * 3 + c], mean[c], sd[c]), u8_norm(by[(2 * i + 1) * 3 + c], mean[c], sd[c]));
+      bf16* dst = out + u8_dst(r, tub) + (long)c * (tub * 256);
       stg_v4(dst, make_uint4(o[0], o[1], o[2], o[3]));
       stg_v4(dst + 8, make_uint4(o[4], o[5], o[6], o[7]));
+    }
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
+// patchify_mix_u8: ub_patchify_mix of the frames ub_patchify_u8 normalises — every byte normalised as there, then mixed as there
+// (mixup and cutmix act on normalised values, as the reference's mixup_fn runs after its loader's tensor_normalize).
+// One thread takes the same (token, kt, kh) run of clips b and B-1-b (b < B/2): 2 x 48 bytes in, 6 x 32 bytes out.
+// A byte has 256 values per channel: each CTA normalises them once into a shared table (u8_norm, so every entry is bit-identical
+// to ub_patchify_u8's value) and looks the pixels up, instead of two IEEE divides per pixel.
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) patchify_mix_u8_kernel(const uint8_t* __restrict__ x, bf16* __restrict__ out,
+                                                              const float* __restrict__ mix, float m0, float m1, float m2, float s0,
+                                                              float s1, float s2, int B, int T, int H, int W, int tub, long total_runs) {
+  __shared__ float lut[3][256];
+  for (int i = threadIdx.x; i < 3 * 256; i += blockDim.x) {
+    const int c = i / 256;
+    lut[c][i % 256] = u8_norm((uint8_t)(i % 256), c == 0 ? m0 : (c == 1 ? m1 : m2), c == 0 ? s0 : (c == 1 ? s1 : s2));
+  }
+  __syncthreads();
+  pdl_grid_sync();
+  const bool apply = mix[0] != 0.f, cut = mix[3] != 0.f;
+  const float lam = mix[1], lam1 = mix[2];
+  const int t0 = (int)mix[4], t1 = (int)mix[5], h0 = (int)mix[6], h1 = (int)mix[7], w0 = (int)mix[8], w1 = (int)mix[9];
+  const long clip_bytes = 3L * T * H * W;
+  const long clip_rows = (long)(T / tub) * (H / 16) * (W / 16) * (3 * tub * 256);
+  for (long id = (long)blockIdx.x * blockDim.x + threadIdx.x; id < total_runs; id += (long)gridDim.x * blockDim.x) {
+    const U8Run r = u8_run(id, T, H, W, tub);                 // a run of the first half of the batch
+    const long mirror = (long)(B - 1 - 2 * r.b);              // clip B-1-b is `mirror` clips further on
+    const uint8_t* sa = x + u8_src(r, T, H, W);
+    uint32_t wa[12], wm[12];
+    u8_load(sa, wa);
+    u8_load(sa + mirror * clip_bytes, wm);
+    const uint8_t* ba = reinterpret_cast<const uint8_t*>(wa);
+    const uint8_t* bm = reinterpret_cast<const uint8_t*>(wm);
+    const bool in_box = apply && cut && r.t >= t0 && r.t < t1 && r.h >= h0 && r.h < h1;
+    bf16* da = out + u8_dst(r, tub);
+    bf16* db = da + mirror * clip_rows;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      float a[16], m[16];
+#pragma unroll
+      for (int i = 0; i < 16; ++i) {
+        a[i] = lut[c][ba[i * 3 + c]];
+        m[i] = lut[c][bm[i * 3 + c]];
+      }
+      if (in_box) {
+#pragma unroll
+        for (int i = 0; i < 16; ++i) {
+          const int w = r.w + i;
+          if (w >= w0 && w < w1) { const float s = a[i]; a[i] = m[i]; m[i] = s; }
+        }
+      } else if (apply && !cut) {
+#pragma unroll
+        for (int i = 0; i < 16; ++i) {
+          const float va = a[i], vm = m[i];
+          a[i] = __fadd_rn(__fmul_rn(va, lam), __fmul_rn(vm, lam1));
+          m[i] = __fadd_rn(__fmul_rn(vm, lam), __fmul_rn(va, lam1));
+        }
+      }
+      uint32_t oa[8], om[8];
+#pragma unroll
+      for (int i = 0; i < 8; ++i) {
+        oa[i] = pack_bf16x2(a[2 * i], a[2 * i + 1]);
+        om[i] = pack_bf16x2(m[2 * i], m[2 * i + 1]);
+      }
+      const long co = (long)c * (tub * 256);
+      stg_v4(da + co, make_uint4(oa[0], oa[1], oa[2], oa[3]));
+      stg_v4(da + co + 8, make_uint4(oa[4], oa[5], oa[6], oa[7]));
+      stg_v4(db + co, make_uint4(om[0], om[1], om[2], om[3]));
+      stg_v4(db + co + 8, make_uint4(om[4], om[5], om[6], om[7]));
     }
   }
 }
@@ -476,6 +571,20 @@ extern "C" int ub_patchify_u8(const uint8_t* x, void* out, const float* mean3, c
   UB_LAUNCH(patchify_u8_kernel, flat_grid(runs, 256), 256, 0, (cudaStream_t)stream, x, (bf16*)out, mean3[0], mean3[1], mean3[2], std3[0],
             std3[1], std3[2], B, T, H, W, tubelet, runs);
   return check_launch("patchify_u8_kernel");
+}
+
+extern "C" int ub_patchify_mix_u8(const uint8_t* x, void* out, const float* mix, const float* mean3, const float* std3, int B, int T, int H,
+                                  int W, int tubelet, void* stream) {
+  UB_REQUIRE(x && out && mix && mean3 && std3, "patchify_mix_u8: null pointer");
+  UB_REQUIRE(B > 0 && B % 2 == 0, "patchify_mix_u8: the batch must be even to pair clip b with clip B-1-b (B=%d)", B);
+  UB_REQUIRE(T > 0 && tubelet > 0 && T % tubelet == 0 && H > 0 && W > 0 && H % 16 == 0 && W % 16 == 0,
+             "patchify_mix_u8: bad shape B=%d T=%d H=%d W=%d tub=%d", B, T, H, W, tubelet);
+  UB_REQUIRE((reinterpret_cast<uintptr_t>(x) & 15) == 0, "patchify_mix_u8: input must be 16-byte aligned");
+  UB_REQUIRE(std3[0] != 0.f && std3[1] != 0.f && std3[2] != 0.f, "patchify_mix_u8: zero std");
+  const long runs = (long)(B / 2) * (T / tubelet) * (H / 16) * (W / 16) * tubelet * 16;
+  UB_LAUNCH(patchify_mix_u8_kernel, flat_grid(runs, 256), 256, 0, (cudaStream_t)stream, x, (bf16*)out, mix, mean3[0], mean3[1], mean3[2],
+            std3[0], std3[1], std3[2], B, T, H, W, tubelet, runs);
+  return check_launch("patchify_mix_u8_kernel");
 }
 
 extern "C" int ub_resize_patchify(const void* x, int x_is_u8, const float* mean3, const float* std3, void* out, int64_t ld_out, int B,

@@ -361,6 +361,21 @@ def schedule_stats(optimizer) -> dict:
     return {"lr": max(lrs), "min_lr": min(lrs), "weight_decay": wds[0] if wds else None}
 
 
+def frames_rows(frames: torch.Tensor, tubelet: int) -> torch.Tensor:
+    """Normalised bf16 im2col rows of decoded uint8 frames [B,T,H,W,3] for a Conv3d of temporal kernel `tubelet` and 16-pixel
+    patches (ops.patchify_u8)."""
+    B, T, H, W, _ = frames.shape
+    out = torch.empty(B * (T // tubelet) * (H // 16) * (W // 16), 3 * tubelet * 256, device=frames.device, dtype=BF16)
+    return ops.patchify_u8(frames, out, tubelet)
+
+
+def frames_carrier(frames: torch.Tensor) -> torch.Tensor:
+    """A zero-stride fp32 [B,3,T,H,W] view with the shape of the clip that uint8 frames [B,T,H,W,3] stand for: handed to a tower
+    together with the frames' im2col rows, it gives the shapes and never has its values read."""
+    B, T, H, W, _ = frames.shape
+    return torch.empty(1, device=frames.device, dtype=F32).expand(B, 3, T, H, W)
+
+
 def exit_if_not_finite(loss: float):
     """A non-finite loss stops training, as the reference's loops do."""
     if not math.isfinite(loss):
@@ -441,14 +456,12 @@ class Stage1Engine(StepEngine):
             T_ = videos.shape[1]
             ks, tub, p = teacher.kernel_size, self.student.encoder.patch_embed.tubelet_size, teacher.patch_size
             if p == 16 and not resize:
-                n_tok = lambda k: B * (T_ // k) * (H_ // 16) * (W_ // 16)
-                patches = ops.patchify_u8(videos, torch.empty(n_tok(ks), 3 * ks * 256, device=videos.device, dtype=BF16), ks)
+                patches = frames_rows(videos, ks)
             else:
                 patches = ops.resize_patchify(videos, torch.empty(B * (T_ // ks) * (R // p) ** 2, teacher.k_pad, device=videos.device,
                                                                   dtype=BF16), R, p, ks)
-            patches_s = patches if share else ops.patchify_u8(
-                videos, torch.empty(B * (T_ // tub) * (H_ // 16) * (W_ // 16), 3 * tub * 256, device=videos.device, dtype=BF16), tub)
-            videos = torch.empty(1, device=videos.device, dtype=F32).expand(B, 3, T_, H_, W_)
+            patches_s = patches if share else frames_rows(videos, tub)
+            videos = frames_carrier(videos)
         elif share:
             ks = teacher.kernel_size
             n_tok = B * (videos.shape[2] // ks) * (videos.shape[3] // 16) * (videos.shape[4] // 16)

@@ -8,6 +8,8 @@ The loss and its gradient come from one fused kernel: ub_softmax_ce for CrossEnt
 and label-smoothing criteria (mixup.resolve_loss).  Mixup / cutmix are drawn on the host exactly as timm draws them and applied
 on the device inside the im2col (ub_patchify_mix), so the caller's clip is never written.  The model's backward is the explicit
 one in finetune_core.py; gradients accumulate in the parameter arena across micro-steps like `.grad` does in torch.
+A batch may carry decoded uint8 frames [B,T,H,W,3] instead of the fp32 clip: they are normalised on the device inside the im2col
+(ub_patchify_u8, or ub_patchify_mix_u8 when mixed), a quarter of the host-to-device copy.
     model_ema.update(model)                                   engine_for_finetuning.py:126-127 (after every optimizer update)
 With `model_ema` (ema.ModelEma or timm's ModelEma) the EMA arena is updated by one fused kernel (ub_ema_update) right after the
 optimizer, inside the CUDA graph of the step.
@@ -48,6 +50,7 @@ def finetune_step(model, samples, targets, loss_acc, scale=1.0, grad_sync=None, 
     overlap this backward.
     mix: None (plain CE), or a mixup.MixBuffer holding this step's draw on the device: the clip is mixed on its way into the
     im2col (mix.clip, None for label smoothing alone) and the loss is the soft-target CE of the mixed, smoothed target."""
+    ops.clip_shape(samples, paired=mix is not None and mix.clip is not None)
     net = model.module if hasattr(model, "module") else model
     core = net.core()
     dp = core.drop_path.draw(samples.shape[0]) if net.training else None       # modeling_finetune.py:42-50 (device-side draws)
@@ -103,13 +106,15 @@ class Stage2Engine(StepEngine):
         self.logits = logits
 
     def step(self, samples, targets, private_inputs=False, mix=None, smoothing=None):
-        """samples fp32 [B,3,T,H,W], targets integer [B], both on the device.  Returns the device loss tensor [1].
+        """samples fp32 [B,3,T,H,W] or decoded uint8 frames [B,T,H,W,3] (normalised on the device), targets integer [B], both on
+        the device.  Returns the device loss tensor [1].
         private_inputs: the batch lives in fresh tensors every step (a loader), so the graph keeps its own static inputs.
         smoothing None: plain CE.  smoothing s: soft-target CE with label smoothing s, and with mix (a mixup.MixDraw, NO_MIX for a
         batch the draw left unmixed) the clip is mixed as drawn.  The draw is uploaded to device memory before the step, so every
         replay of the one graph per loss kind reads its own draw."""
         if mix is not None and smoothing is None:
             raise ValueError("Stage2Engine.step: a mixup draw needs the soft-target loss (pass smoothing=)")
+        ops.clip_shape(samples, paired=mix is not None)
         self.optimizer.prepare_step(grad_scale=self.grad_scale)
         kind = "ce" if smoothing is None else ("mix" if mix is not None else "smooth")
         self._mix = None
@@ -179,7 +184,7 @@ def train_one_epoch(model: torch.nn.Module, criterion=None, data_loader: Iterabl
         if data_iter_step % update_freq == 0:                                      # engine_for_finetuning.py:76-81
             apply_schedule(optimizer, start_steps + step, lr_schedule_values, wd_schedule_values)
         if mix is not None:
-            mix.upload((draw(mixup_fn, samples.shape) if mixup_fn is not None else NO_MIX).packed(smoothing, core.C))
+            mix.upload((draw(mixup_fn, ops.clip_shape(samples)) if mixup_fn is not None else NO_MIX).packed(smoothing, core.C))
         samples = samples.to(dev, non_blocking=True)
         targets = targets.to(dev, non_blocking=True)
         loss_acc.zero_()
@@ -220,7 +225,7 @@ def _train_one_epoch_graphed(model, net, data_loader, optimizer, gs, max_norm, s
         if num_training_steps_per_epoch is not None and data_iter_step >= num_training_steps_per_epoch:
             continue                                                               # engine_for_finetuning.py:71-72
         apply_schedule(optimizer, start_steps + data_iter_step, lr_schedule_values, wd_schedule_values)   # :76-81
-        mix = draw(mixup_fn, batch[0].shape) if mixup_fn is not None else None
+        mix = draw(mixup_fn, ops.clip_shape(batch[0])) if mixup_fn is not None else None
         eng.step(batch[0].to(dev, non_blocking=True), batch[1].to(dev, non_blocking=True), private_inputs=True, mix=mix,
                  smoothing=smoothing)
         seen += batch[0].shape[0]

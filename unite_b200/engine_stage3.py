@@ -20,10 +20,23 @@ from typing import Iterable, Optional
 import torch
 
 from . import ops
-from .engine import (FusedAdamW, GraphReplay, StepEngine, apply_schedule, exit_if_not_finite, require_fused_optimizer,
-                     schedule_stats)
+from .engine import (FusedAdamW, GraphReplay, StepEngine, apply_schedule, exit_if_not_finite, frames_carrier, frames_rows,
+                     require_fused_optimizer, schedule_stats)
 
 BF16, F32, I32, U8 = torch.bfloat16, torch.float32, torch.int32, torch.uint8
+
+
+def view_dtype(*views):
+    """The dtype shared by a step's source, target and augmented-target views (None entries skipped): fp32 clips or decoded
+    uint8 frames, never both in one step.  ValueError, before anything runs, for mixed dtypes or uint8 frames the device
+    normalisation cannot read (ops.clip_shape)."""
+    views = [v for v in views if v is not None]
+    dtypes = {v.dtype for v in views}
+    if len(dtypes) != 1:
+        raise ValueError(f"stage 3: the source, target and augmented-target views must share a dtype, got {[str(v.dtype) for v in views]}")
+    for v in views:
+        ops.clip_shape(v)
+    return views[0].dtype
 
 
 class Stage3Engine(StepEngine):
@@ -89,7 +102,11 @@ class Stage3Engine(StepEngine):
         the teacher attention and the masked committee views use it (`videos = cat([videos_s, videos_t_aug])`,
         run_stage3.py:413, :434-451, :499), while the full-token target pass and the zero-shot head see the plain view
         (:480, :557).  None = one view for everything.
-        dp_override: dict slot -> DropPath factors [depth,2,B] for the four forwards ('s', 't', 0..k-1) (tests)."""
+        dp_override: dict slot -> DropPath factors [depth,2,B] for the four forwards ('s', 't', 0..k-1) (tests).
+        Every view is an fp32 clip [B,3,T,H,W], or every view is decoded uint8 frames [B,T,H,W,3]: those are normalised on the
+        device inside the im2col (ub_patchify_u8), once per view for the teacher and, when its temporal kernel is the student's
+        tubelet, for the student too."""
+        u8 = view_dtype(videos_s, videos_t, videos_t_aug) == U8
         core, teacher, k = self.core, self.teacher, self.k
         dev = videos_s.device
         Bs, Bt, N = videos_s.shape[0], videos_t.shape[0], core.N
@@ -97,32 +114,41 @@ class Stage3Engine(StepEngine):
         dual = videos_t_aug is not None and videos_t_aug is not videos_t
         v_mask = videos_t_aug if dual else videos_t
         training = self.student.training
+        share = core.tubelet == teacher.kernel_size
 
         def dp_for(slot, B):
             if dp_override is not None:
                 return dp_override.get(slot)
             return core.drop_path.draw(B, slot=slot) if training else None          # model.train() covers every pass (:352)
 
+        def teacher_on(v):
+            # uint8 frames: the teacher reads their normalised rows and a shape carrier (as in Stage1Engine.forward_backward)
+            return teacher.forward_features(frames_carrier(v), frames_rows(v, teacher.kernel_size)) if u8 else teacher.forward_features(v)
+
+        def student_rows(v, teacher_rows):
+            # im2col rows the student reads: the teacher's when the kernels agree; None = run_forward patchifies the fp32 clip
+            return teacher_rows if share else (frames_rows(v, core.tubelet) if u8 else None)
+
         # ---- teacher on the target clips: attention map (augmented view) + CLS embedding for the zero-shot head (plain view)
-        _, attn, patches_m = teacher.forward_features(v_mask)
+        _, attn, patches_m = teacher_on(v_mask)
         frames, P = attn.shape
         T = frames // Bt
         if dual:
-            _, _, patches_t = teacher.forward_features(videos_t)
+            _, _, patches_t = teacher_on(videos_t)
         else:
             patches_t = patches_m
         img = teacher.cls_features(frames, P)                                      # [Bt*T, 512]
-        share = core.tubelet == teacher.kernel_size
         # ---- source clips, all tokens, with grad
         self.loss.zero_(); self.loss_s.zero_(); self.loss_t.zero_()
-        xs, _, st_s = core.run_forward(videos_s, self._all_visible(Bs, N, dev), None, dp_for("s", Bs), False, True, want_clip=False)
+        xs, _, st_s = core.run_forward(videos_s, self._all_visible(Bs, N, dev), frames_rows(videos_s, core.tubelet) if u8 else None,
+                                       dp_for("s", Bs), False, True, want_clip=False)
         pooled_s, logits_s = self._classify(xs)
         dl_s = torch.empty_like(logits_s)
         ops.softmax_ce(logits_s, labels_s.to(I32), None, self.src_ratio / Bs, self.loss_s, dl_s)
         self._backward_from_logits(st_s, pooled_s, dl_s, N)
         # ---- target clips, all tokens, no grad
-        xt, _, _ = core.run_forward(videos_t, self._all_visible(Bt, N, dev), patches_t if share else None, dp_for("t", Bt), False, False,
-                                    want_clip=False)
+        xt, _, _ = core.run_forward(videos_t, self._all_visible(Bt, N, dev), student_rows(videos_t, patches_t), dp_for("t", Bt), False,
+                                    False, want_clip=False)
         _, logits_full_t = self._classify(xt)
         # ---- committee masks and masked views
         n_vis = P - int(P * self.mask_ratio)
@@ -132,11 +158,12 @@ class Stage3Engine(StepEngine):
         logits_masked = torch.empty(k, Bt, C, device=dev, dtype=F32)
         base = (torch.arange(Bt, device=dev, dtype=I32) * N).view(Bt, 1)
         st_m = pooled_m = None
+        rows_m = student_rows(v_mask, patches_m)
         for m in range(k):
             grad = m == k - 1                                                      # only the last member trains (run_stage3.py:606)
             abs_rows = (vis[m] + base).reshape(-1).contiguous() if share else None
-            xm, _, st = core.run_forward(v_mask, vis[m].contiguous(), patches_m if share else None, dp_for(m, Bt), False, grad,
-                                         want_clip=False, abs_rows=abs_rows)
+            xm, _, st = core.run_forward(v_mask, vis[m].contiguous(), rows_m, dp_for(m, Bt), False, grad, want_clip=False,
+                                         abs_rows=abs_rows)
             pooled, lg = self._classify(xm)
             logits_masked[m].copy_(lg)
             if grad:
@@ -164,7 +191,9 @@ class Stage3Engine(StepEngine):
         self._update()
 
     def step(self, videos_s, labels_s, videos_t, videos_t_aug=None, private_inputs=False):
-        """One update.  private_inputs: the batch lives in fresh tensors every step (a loader), so a graph keeps its own inputs."""
+        """One update.  private_inputs: the batch lives in fresh tensors every step (a loader), so a graph keeps its own inputs.
+        The views are all fp32 clips or all decoded uint8 frames (see forward_backward)."""
+        dtype = view_dtype(videos_s, videos_t, videos_t_aug)
         self.optimizer.prepare_step(grad_scale=self.grad_scale)
         if videos_t_aug is videos_t:
             videos_t_aug = None
@@ -172,7 +201,7 @@ class Stage3Engine(StepEngine):
             self._step_body_dev(videos_s, labels_s, videos_t, videos_t_aug)
             return self.loss
         key = (tuple(videos_s.shape), tuple(videos_t.shape), videos_t_aug is not None, labels_s.dtype, float(self.max_norm or 0.0),
-               bool(self.student.training), self.mask_ratio)
+               bool(self.student.training), self.mask_ratio, dtype)
         self.last = self.graphs.run(key, (videos_s, labels_s, videos_t, videos_t_aug), self._step_body_dev,
                                     state_fn=lambda: self.last, private=private_inputs)
         return self.loss

@@ -8,7 +8,7 @@ from . import ops
 from .arena import ParamArena
 from .vit_core import DropPathSource, ViTTrunk
 
-BF16, F32 = torch.bfloat16, torch.float32
+BF16, F32, U8 = torch.bfloat16, torch.float32, torch.uint8
 
 
 class _FinetuneFn(torch.autograd.Function):
@@ -54,12 +54,18 @@ class FinetuneCore:
         return self._pos_full[B]
 
     def run_forward(self, x, dp, save, mix=None):
-        """mix: None, or the device draw of batch-mode mixup / cutmix (mixup.MixBuffer.clip): the trunk then sees the mixed clip,
+        """x: the fp32 clip [B,3,T,H,W], or decoded uint8 frames [B,T,H,W,3], normalised on the device (ops.patchify_u8).
+        mix: None, or the device draw of batch-mode mixup / cutmix (mixup.MixBuffer.clip): the trunk then sees the mixed clip,
         mixed on the way into the im2col (x itself is not written)."""
+        u8 = x.dtype == U8
         self.sync_shadow()
         B, dev, a = x.shape[0], x.device, self.arena
         patches = torch.empty(B * self.N, 3 * self.tubelet * 256, device=dev, dtype=BF16)
-        if mix is None:
+        if u8 and mix is None:
+            ops.patchify_u8(x, patches, self.tubelet)
+        elif u8:
+            ops.patchify_mix_u8(x, patches, mix, self.tubelet)
+        elif mix is None:
             ops.patchify(x.contiguous(), patches, self.tubelet)
         else:
             ops.patchify_mix(x.contiguous(), patches, mix, self.tubelet)

@@ -189,8 +189,11 @@ class VisionTransformer(nn.Module):
         return super()._apply(fn, *a, **k)
 
     def forward(self, x, drop_path_factors_=None):
-        """x [B,3,T,H,W] fp32 -> logits [B, num_classes] (modeling_finetune.py:356-383)."""
+        """x [B,3,T,H,W] fp32, or decoded uint8 frames [B,T,H,W,3] normalised on the device -> logits [B, num_classes]
+        (modeling_finetune.py:356-383)."""
+        from . import ops
         from .finetune_core import _FinetuneFn
+        ops.clip_shape(x)
         core = self.core()
         dp = drop_path_factors_
         if dp is None and self.training:

@@ -312,6 +312,39 @@ def patchify_u8(x, out, tubelet, mean=IMAGENET_MEAN, std=IMAGENET_STD):
     return out
 
 
+@_instrument("patchify_mix", 1)
+def patchify_mix_u8(x, out, mix, tubelet, mean=IMAGENET_MEAN, std=IMAGENET_STD):
+    """patchify_mix of the clip patchify_u8 normalises from x uint8 [B,T,H,W,3]: normalised, then mixed by the device draw mix
+    (fp32 [10], see patchify_mix); x untouched."""
+    if x.dim() != 5 or x.shape[-1] != 3 or not x.is_contiguous():
+        raise _cabi.UBError(f"patchify_mix_u8: contiguous uint8 [B,T,H,W,3] expected, got {tuple(x.shape)}")
+    if mix.numel() < 10:
+        raise _cabi.UBError("patchify_mix_u8: mix must hold 10 floats")
+    B, T, H, W, _ = x.shape
+    m3, s3 = (C.c_float * 3)(*mean), (C.c_float * 3)(*std)
+    check(lib.ub_patchify_mix_u8(_p(x, U8, "frames"), _p(out, BF16, "patches"), _p(mix, F32, "mix"), m3, s3, B, T, H, W, tubelet,
+                                 _stream()), "ub_patchify_mix_u8")
+    return out
+
+
+def clip_shape(x, paired=False):
+    """The [B,3,T,H,W] shape of the clip a batch stands for: an fp32 clip's own shape, or that of the clip decoded uint8 frames
+    [B,T,H,W,3] normalise to.  A uint8 batch that patchify_u8 / patchify_mix_u8 cannot read raises ValueError here, before any
+    launch: not contiguous [B,T,H,W,3], H or W not a multiple of 16, or (paired: clip b is mixed with clip B-1-b) an odd batch."""
+    if x.dtype != U8:
+        return tuple(x.shape)
+    if x.dim() != 5 or x.shape[-1] != 3:
+        raise ValueError(f"uint8 batches are decoded frames [B,T,H,W,3] (channels last); got shape {tuple(x.shape)}")
+    if not x.is_contiguous():
+        raise ValueError(f"uint8 frames must be contiguous; got shape {tuple(x.shape)} with strides {x.stride()}")
+    B, T, H, W, _ = x.shape
+    if H % 16 or W % 16:
+        raise ValueError(f"uint8 frames of {H}x{W} pixels: H and W must be multiples of the 16-pixel patch")
+    if paired and B % 2:
+        raise ValueError(f"mixup: the batch size must be even (clip b is mixed with clip B-1-b), got {B}")
+    return (B, 3, T, H, W)
+
+
 def padded_k(features: int) -> int:
     """Row pitch of resize_patchify's output: the im2col width rounded up to 64 elements (one GEMM K block; also keeps the
     rows 16-byte aligned for TMA, which 3*14*14 = 588 bf16 would not be)."""

@@ -11,6 +11,12 @@ Batches live in PINNED host memory (like DataLoader(pin_memory=True), run_stage1
 import torch
 
 
+def _clips(batch_size, num_frames, img_size, g, uint8):
+    if uint8:
+        return torch.randint(0, 256, (batch_size, num_frames, img_size, img_size, 3), generator=g, dtype=torch.uint8)
+    return torch.randn(batch_size, 3, num_frames, img_size, img_size, generator=g)
+
+
 class SyntheticStage1Loader:
     def __init__(self, batch_size, num_frames=8, img_size=224, steps=10, seed=0, rank=0, n_distinct=2, num_classes=12,
                  frames_per_token=1, pin=True, uint8=False):
@@ -22,10 +28,7 @@ class SyntheticStage1Loader:
         pin = pin and torch.cuda.is_available()
         HW = (img_size // 16) ** 2
         for _ in range(n_distinct):
-            if uint8:
-                v = torch.randint(0, 256, (batch_size, num_frames, img_size, img_size, 3), generator=g, dtype=torch.uint8)
-            else:
-                v = torch.randn(batch_size, 3, num_frames, img_size, img_size, generator=g)
+            v = _clips(batch_size, num_frames, img_size, g, uint8)
             q = torch.empty(batch_size * (num_frames // frames_per_token), HW).exponential_(1, generator=g)
             y = torch.randint(0, num_classes, (batch_size,), generator=g)
             if pin:
@@ -41,14 +44,16 @@ class SyntheticStage1Loader:
 
 
 class SyntheticStage2Loader:
-    """(clip, label, index, {}) batches of kinetics_sparse.py:159 (train mode), pinned."""
+    """(clip, label, index, {}) batches of kinetics_sparse.py:159 (train mode), pinned.  uint8=True: the clip is DECODED frames
+    uint8 [B,T,H,W,3], as in SyntheticStage1Loader; the engine normalises them on the device."""
 
-    def __init__(self, batch_size, num_frames=8, img_size=224, steps=10, seed=0, rank=0, n_distinct=2, num_classes=12, pin=True):
+    def __init__(self, batch_size, num_frames=8, img_size=224, steps=10, seed=0, rank=0, n_distinct=2, num_classes=12, pin=True,
+                 uint8=False):
         g = torch.Generator().manual_seed(seed + rank)
         pin = pin and torch.cuda.is_available()
         self.steps, self.batches = steps, []
         for _ in range(n_distinct):
-            v = torch.randn(batch_size, 3, num_frames, img_size, img_size, generator=g)
+            v = _clips(batch_size, num_frames, img_size, g, uint8)
             y = torch.randint(0, num_classes, (batch_size,), generator=g)
             self.batches.append((v.pin_memory() if pin else v, y, torch.arange(batch_size), {}))
 
@@ -65,7 +70,7 @@ class SyntheticStage3Loader:
     dual-view batch (vid, vid_aug, label, name) of validation mode with return_aug_for_val (kinetics_sparse.py:174-180) — the
     plain view feeds the full-token pass and the zero-shot head, the augmented one the teacher attention and the masked
     committee (run_stage3.py:405-413).  vid_aug = vid + small noise (a stand-in for RandAugment: a different tensor of the same
-    distribution)."""
+    distribution).  uint8=True: every view is DECODED frames uint8 [B,T,H,W,3], as in SyntheticStage1Loader."""
 
     class _Iter:
         def __init__(self, batches, steps):
@@ -79,16 +84,19 @@ class SyntheticStage3Loader:
                 yield self.batches[i % len(self.batches)]
 
     def __init__(self, batch_size_s, batch_size_t=None, num_frames=8, img_size=224, steps=10, seed=0, rank=0, n_distinct=2,
-                 num_classes=12, pin=True):
+                 num_classes=12, pin=True, uint8=False):
         g = torch.Generator().manual_seed(seed + rank)
         bt = batch_size_t or batch_size_s
         pin = pin and torch.cuda.is_available()
         src, tgt = [], []
         for i in range(n_distinct):
-            vs = torch.randn(batch_size_s, 3, num_frames, img_size, img_size, generator=g)
+            vs = _clips(batch_size_s, num_frames, img_size, g, uint8)
             ys = torch.randint(0, num_classes, (batch_size_s,), generator=g)
-            vt = torch.randn(bt, 3, num_frames, img_size, img_size, generator=g)
-            va = vt + 0.1 * torch.randn(bt, 3, num_frames, img_size, img_size, generator=g)
+            vt = _clips(bt, num_frames, img_size, g, uint8)
+            if uint8:
+                va = (vt.short() + torch.randint(-8, 9, vt.shape, generator=g, dtype=torch.int16)).clamp_(0, 255).to(torch.uint8)
+            else:
+                va = vt + 0.1 * torch.randn(bt, 3, num_frames, img_size, img_size, generator=g)
             yt = torch.randint(0, num_classes, (bt,), generator=g)
             if pin:
                 vs, vt, va = vs.pin_memory(), vt.pin_memory(), va.pin_memory()
