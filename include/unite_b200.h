@@ -76,19 +76,6 @@ typedef struct ub_gemm_epilogue {
    *   A: k + g * group_a_k, m - g * group_a_m        B: k + g * group_b_k, n + g * group_b_n        bias[n + g * group_bias]
    * (offsets in elements of the respective dimension; K is the per-group contraction length).  All 0 = ordinary GEMM.          */
   int32_t group_rows, group_a_k, group_a_m, group_b_k, group_b_n, group_bias;
-  /* Stream-K tail: scratch that lets the kernel cut the tiles of a partial LAST wave along K across all CTA pairs (e.g. 120 tiles
-   * of 256 x 256 on 74 pairs: 1.62 waves of work instead of 2 waves of time); a tile's pieces park fp32 partial accumulators here
-   * and the piece holding the tile's last k-block adds them and runs the epilogue, so results differ from the whole-tile schedule
-   * only by fp32 summation order.  Caller-owned, at least ub_gemm_sk_workspace_bytes() bytes, ZERO-FILLED ONCE when allocated (the
-   * kernel leaves its counters at zero), 16-byte aligned, and used by ONE stream at a time.  NULL = whole tiles only; with a
-   * workspace the cost model still decides per call whether the split is taken.  Measured on B200 (profiles/gemm_streamk_r02.md):
-   * bit-reproducible and within fp32 rounding of the whole-tile schedule, but 2-4 % SLOWER on the step's shapes — the partial
-   * last wave is not what bounds them (the pairs that remain active get the idle pairs' share of the L2 -> SM path) — so the
-   * Python front end passes a workspace only on request (ops.gemm(stream_k=True) / UB_GEMM_SK=1), and the default library is built
-   * WITHOUT the schedule (ub_gemm_sk_compiled() == 0: the field is ignored); -DUB_GEMM_STREAMK (libunite_b200_sk.so, loaded with
-   * UB_LIB_VARIANT=sk) compiles it in. */
-  void* sk_workspace;
-  int64_t sk_workspace_bytes;
   /* UB_ACT_DOT_AUX (bf16 out, N a multiple of 64): C = acc as usual, and in the same pass
    *   dot_out[((m / dot_seq_len) * (N / 64) + n / 64) * dot_seq_len + m % dot_seq_len] = sum over the 64 columns of head n / 64 of
    *   bf16(C[m, n]) * aux_in[m, n]
@@ -98,19 +85,6 @@ typedef struct ub_gemm_epilogue {
   int32_t dot_seq_len;
   int32_t reserved0;
 } ub_gemm_epilogue;
-
-/* bytes of ub_gemm_epilogue.sk_workspace that cover every shape on this device */
-UB_API int64_t ub_gemm_sk_workspace_bytes(void);
-/* 1 if this build of the library contains the stream-K tail (-DUB_GEMM_STREAMK: libunite_b200_sk.so), 0 if sk_workspace is ignored
- * (the default build: the schedule's bookkeeping costs the ordinary path 0.9 % of the step and no shape gains from it on B200) */
-UB_API int ub_gemm_sk_compiled(void);
-/* diagnostic: how many ub_gemm_bf16 calls of this process took the stream-K tail schedule */
-UB_API int64_t ub_gemm_sk_launches(void);
-/* Diagnostic (host only, no GPU needed): the stream-K plan the kernel follows for T tiles of KB k-blocks on U CTA pairs with a
- * fix-up charge of `overhead` k-blocks, and pair u's share of it:
- *   out[11] = {first split tile, split tiles, pairs in the split, whole tiles of u, partial piece (tile, kb0, kb1, slot),
- *              finishing piece (tile, kb0, pieces to add)};  tile = -1: no such piece.  Returns 1 if the tail is split, else 0. */
-UB_API int ub_gemm_sk_schedule(int T, int U, int KB, int overhead, int u, int32_t* out);
 
 /* a_mn_major / b_mn_major = 1: the operand is stored transposed, i.e. A is [K, lda>=M] / B is [K, ldb>=N]
  * row-major (used by weight-gradient GEMMs, where the contraction runs over tokens).                      */

@@ -27,21 +27,14 @@ def test_every_declared_symbol_is_exported_and_bound():
     assert sorted(_cabi.SIGNATURES) == declared
 
 
-def test_build_variants_export_the_same_abi_and_say_what_they_are():
-    """build() also produces libunite_b200_erf.so (-DUB_GELU_ERF) and libunite_b200_sk.so (-DUB_GEMM_STREAMK): same exported symbols
-    as the default library; only the stream-K build reports the schedule as compiled in (the default build ignores sk_workspace)."""
-    import ctypes as C
+def test_erf_build_exports_the_same_abi():
+    """build() also produces libunite_b200_erf.so (-DUB_GELU_ERF): the same exported symbols as the default library."""
     from unite_b200 import _cabi
     declared = _header_functions()
-    libdir = os.path.dirname(_cabi._LIB_PATH)
-    for variant, sk in (("erf", 0), ("sk", 1)):
-        path = os.path.join(libdir, f"libunite_b200_{variant}.so")
-        assert os.path.exists(path), f"build() did not produce {path}"
-        out = subprocess.run(["nm", "-D", "--defined-only", path], capture_output=True, text=True, check=True).stdout
-        assert sorted(set(re.findall(r" T (ub_\w+)", out))) == declared, variant
-        assert C.CDLL(path).ub_gemm_sk_compiled() == sk, variant
-    if not os.environ.get("UB_LIB_VARIANT"):
-        assert _cabi.lib.ub_gemm_sk_compiled() == 0
+    path = os.path.join(os.path.dirname(_cabi._LIB_PATH), "libunite_b200_erf.so")
+    assert os.path.exists(path), f"build() did not produce {path}"
+    out = subprocess.run(["nm", "-D", "--defined-only", path], capture_output=True, text=True, check=True).stdout
+    assert sorted(set(re.findall(r" T (ub_\w+)", out))) == declared
 
 
 def test_sass_uses_blackwell_tensor_and_tma_paths():

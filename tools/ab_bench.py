@@ -34,8 +34,8 @@ def run(setting, steps, warmup, gpus, port):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--a", default="", help='environment of setting A, e.g. "UB_PDL=0"')
-    ap.add_argument("--b", required=True, help='environment of setting B, e.g. "UB_PDL=1 UB_LIB_VARIANT=x"')
+    ap.add_argument("--a", default="", help='environment of setting A, e.g. "UB_ASYNC_ZERO=1"')
+    ap.add_argument("--b", required=True, help='environment of setting B, e.g. "UB_ASYNC_ZERO=0 UB_LIB_VARIANT=x"')
     ap.add_argument("--rounds", type=int, default=2)
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=4)

@@ -42,8 +42,6 @@ class GemmEpilogue(C.Structure):
         ("group_b_k", C.c_int32),
         ("group_b_n", C.c_int32),
         ("group_bias", C.c_int32),
-        ("sk_workspace", C.c_void_p),
-        ("sk_workspace_bytes", C.c_int64),
         ("dot_out", C.c_void_p),
         ("dot_seq_len", C.c_int32),
         ("reserved0", C.c_int32),
@@ -74,10 +72,6 @@ SIGNATURES = {
     "ub_sm_count": (C.c_int, []),
     "ub_set_sm_limit": (C.c_int, [_I]),
     "ub_gemm_cluster4_capacity": (C.c_int, []),
-    "ub_gemm_sk_workspace_bytes": (C.c_int64, []),
-    "ub_gemm_sk_compiled": (C.c_int, []),
-    "ub_gemm_sk_launches": (C.c_int64, []),
-    "ub_gemm_sk_schedule": (C.c_int, [_I, _I, _I, _I, _I, C.POINTER(C.c_int32)]),
     "ub_gemm_bf16": (C.c_int, [_P, _L, _I, _P, _L, _I, _P, _L, _I, _I, _I, C.POINTER(GemmEpilogue), _I, _P]),
     "ub_gemm_wgrad_multi": (C.c_int, [C.POINTER(GemmProblem), _I, _I, _I, _P]),
     "ub_attn_fwd": (C.c_int, [_P, _P, _P, _I, _I, _I, _F, _P]),

@@ -20,7 +20,6 @@ constexpr int HD = 64;          // head dim
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) attn_bwd_prep_kernel(const bf16* __restrict__ o, const bf16* __restrict__ d_o,
                                                             float* __restrict__ D, long n_chunks, int S, int H) {
-  pdl_grid_sync();
   // one thread = 8 consecutive channels (16 B of o and of d_o); 8 threads = one (row, head); 3 shuffles finish the dot product
   const long id = (long)blockIdx.x * blockDim.x + threadIdx.x;
   float v = 0.f;
@@ -50,7 +49,6 @@ __global__ void __launch_bounds__(256) attn_bwd_prep_kernel(const bf16* __restri
 //   out[seq, j] = 1/H * sum_h softmax_k(q_cls . k / sqrt(d))[j+1],   j in [0, S-1)
 // ------------------------------------------------------------------------------------------------
 __global__ void cls_attn_kernel(const bf16* __restrict__ qkv, float* __restrict__ out, int S, int H, float scale) {
-  pdl_grid_sync();
   extern __shared__ float s_probs[];  // [H][S]
   const int seq = blockIdx.x, h = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t ld = 3 * (int64_t)H * HD;

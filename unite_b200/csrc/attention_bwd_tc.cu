@@ -106,7 +106,6 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_grid_sync();     // everything above overlapped the previous kernel's tail; global memory is touched only below
   const int n_items = p.n_seq * p.H;
   const int nkt = p.nkt, nc = p.nc, total = p.nkt * p.nc;
   constexpr uint32_t TM_DV = 192, TM_DK = 256, TM_DQ = 320;

@@ -85,7 +85,6 @@ attn_fwd_lse_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_grid_sync();
   const int n_items = p.n_seq * p.H;
   const int nt = p.nt, nch = p.nch;
 

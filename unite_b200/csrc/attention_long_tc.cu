@@ -126,7 +126,6 @@ attn_long_tc_kernel(const __grid_constant__ CUtensorMap tmStat, const __grid_con
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_grid_sync();
   const int n_units = p.n_seq * p.H * p.npair;
   const int nchunk = p.nchunk;
 

@@ -86,7 +86,6 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_grid_sync();     // everything above overlapped the previous kernel's tail; global memory is touched only below
   const int n_items = p.n_seq * p.H;
   constexpr int SM_WARP0 = NKT ? 4 : 2;    // first softmax warp
 

@@ -27,37 +27,20 @@ int check_launch(const char* what);
   } while (0)
 
 int sm_count();
-bool pdl_enabled();   // programmatic dependent launch for every kernel of the library (UB_PDL=1 turns it on)
 
-// ----------------------------------------------------------------------------------------------
-// Programmatic dependent launch.  Every kernel of the library is launched with the programmatic-stream-serialization
-// attribute and calls pdl_grid_sync() before it touches global memory: its CTAs may be scheduled (and run their
-// prologue: barrier init, TMEM allocation, descriptor prefetch) while the previous kernel of the stream drains, but
-// read / write global memory only after that kernel has completed and flushed.  The trigger right after the wait lets
-// the NEXT kernel do the same behind this one.
-// ----------------------------------------------------------------------------------------------
-UB_DEVINL void pdl_grid_sync() {
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-#ifndef UB_PDL_NO_TRIGGER
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-}
+// Every kernel launch of the library goes through here: each argument is static_cast to the kernel's parameter type, so
+// that, for example, a void* may be passed for a float* parameter.
 template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args&&... args) {
+inline cudaError_t launch_kernel(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args&&... args) {
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = grid;
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = stream;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 #define UB_LAUNCH(kern, grid, block, smem, stream, ...) \
-  (void)ub::launch_pdl(kern, dim3(grid), dim3(block), (size_t)(smem), (cudaStream_t)(stream), __VA_ARGS__)
+  (void)ub::launch_kernel(kern, dim3(grid), dim3(block), (size_t)(smem), (cudaStream_t)(stream), __VA_ARGS__)
 
 // ----------------------------------------------------------------------------------------------
 // small math / packing

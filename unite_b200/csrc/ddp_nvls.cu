@@ -178,7 +178,6 @@ UB_DEVINL void nvls_segment(const NvlsStep& a, long lo, long hi, long tid, long 
 
 template <int kU, int kW>
 __global__ void __launch_bounds__(256) adamw_nvls_kernel(const NvlsStep a) {
-  pdl_grid_sync();
   __shared__ float s_part[8];
   __shared__ uint32_t s_epoch;
   __shared__ int s_abort;
@@ -236,7 +235,6 @@ __global__ void __launch_bounds__(256) adamw_nvls_kernel(const NvlsStep a) {
 // (all local HBM reads, rank order => bitwise reproducible), runs AdamW and stores the bf16 shadow to every rank.
 template <int kW>
 __global__ void __launch_bounds__(256) adamw_push_kernel(const NvlsStep a) {
-  pdl_grid_sync();
   __shared__ float s_part[8];
   __shared__ uint32_t s_epoch;
   __shared__ int s_abort;

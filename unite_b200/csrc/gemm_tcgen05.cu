@@ -30,20 +30,12 @@ namespace ub {
 constexpr int BM = 128;
 constexpr int BK = 64;
 constexpr int GEMM_THREADS = 320;  // warp 0 TMA, warp 1 MMA, warps 2..9 epilogue
-// Staging slabs (32 rows x 128 B) per epilogue warp: two.  -DUB_GEMM_EPI_NBUF=3 gives the epilogues that READ an operand through
-// TMA (fp32 / fp16 residual, GELU pre-activation) a third one, so that the operand of slab n+2 is requested while slab n is
-// processed (with two, the request goes out one slab, ~0.4 us, ahead of its use against a TMA round trip of ~1 us) — paid for with
-// one mainloop stage (4 instead of 5).  Measured on B200, A/B/A/B/A/B over whole steps: 17.998 ms (three slabs) vs 17.918 ms (two):
-// what the K = 768 residual GEMMs gain, the K = 3072 ones lose with the shallower ring.  So the default stays at two.
-#ifndef UB_GEMM_EPI_NBUF
-#define UB_GEMM_EPI_NBUF 2
-#endif
-template <int BN, int EPI, int NCTA>
-struct GemmCfg {
-  static constexpr int NBUF = (EPI != 0 && EPI != 4 && !(BN == 256 && NCTA == 1)) ? UB_GEMM_EPI_NBUF : 2;
-  static constexpr int EPI_BYTES = 8 * NBUF * 4096;      // 8 epilogue warps x NBUF staging slabs
-  static constexpr int stages(int requested) { return NBUF == 3 && requested > 4 ? 4 : requested; }
-};
+constexpr int EPI_BYTES = 8 * 2 * 4096;   // 8 epilogue warps x 2 staging slabs of 32 rows x 128 B
+// Dynamic shared memory of a GEMM CTA (the layout gemm_body carves out): the STAGES-deep A / B ring, the staging slabs, the bias
+// tile [2][BN], the mbarriers (full / empty per stage, tfull / tempty x 2, two residual barriers per epilogue warp) and the TMEM slot.
+constexpr int gemm_smem_bytes(int BN, int STAGES, int NCTA) {
+  return STAGES * (BM * BK * 2 + (BN / (NCTA >= 2 ? 2 : 1)) * BK * 2) + EPI_BYTES + 2 * BN * 4 + (2 * STAGES + 4 + 16) * 8 + 16;
+}
 
 struct GemmParams {
   int M, N, K;
@@ -72,59 +64,7 @@ struct GemmParams {
   int n_prob;
   int tile_off[5];
   int ntile_n[4];
-  // stream-K tail (ub_gemm_epilogue.sk_workspace): tiles [sk_first, sk_first + sk_tiles) — the partial last wave — are cut along K
-  // into sk_units contiguous ranges of k-blocks, one per CTA pair; 0 tiles = every tile is computed whole
-  int sk_first, sk_tiles, sk_units;
-  float* sk_ws;             // partial accumulators: [sk tile][2 slots][2 CTAs][8 warps][4096] fp32 after SK_FLAG_BYTES of counters
 };
-
-constexpr int SK_FLAG_BYTES = 8192;          // (sk tile, CTA, warp) arrival counters, zero between launches
-constexpr int SK_MAX_TILES = SK_FLAG_BYTES / (16 * 4);
-constexpr size_t SK_TILE_BYTES = 2 * 2 * 8 * 4096 * sizeof(float);     // two slots of one 256 x 256 fp32 pair tile
-
-// Stream-K tail, the part shared by the kernel, the host and the CPU tests (ub_gemm_sk_schedule).
-// Plan: T tiles on U CTA pairs, KB k-blocks per tile.  The R = T mod U tiles of the partial last wave are cut into `units`
-// contiguous k-block ranges [u W / units, (u + 1) W / units) of their W = R * KB k-blocks, one per pair, each at least half a tile
-// long — so a range touches at most two tiles and a tile is shared by at most three pairs (two workspace slots).  Cost in
-// k-blocks per pair: whole tiles ceil(T / U) * KB, split tail floor(T / U) * KB + ceil(W / units) + a fix-up charge.
-static int64_t g_sk_launches = 0;        // GEMM launches that split their tail (diagnostic: ub_gemm_sk_launches)
-struct SkPlan { int first, tiles, units; };
-__host__ __device__ inline SkPlan sk_plan(int T, int U, int KB, int overhead) {
-  SkPlan pl{0, 0, 0};
-  if (T <= 0 || U <= 0 || KB < 4) return pl;
-  const int R = T % U;
-  if (R == 0 || R > SK_MAX_TILES) return pl;
-  long us = ((long)R * KB) / ((KB + 1) / 2);
-  if (us > U) us = U;
-  const long dp_cost = (long)((T + U - 1) / U) * KB;
-  const long sk_cost = (long)(T / U) * KB + ((long)R * KB + us - 1) / us + overhead;
-  if (sk_cost >= dp_cost || us < R) return pl;
-  pl.first = T - R; pl.tiles = R; pl.units = (int)us;
-  return pl;
-}
-// Pair u's share: n_dp whole tiles (u, u + U, ... below pl.first), at most one partial piece (k-blocks [part_kb0, part_kb1) of
-// part_tile, parked in slot part_slot) and at most one finishing piece (k-blocks [fin_kb0, KB) of fin_tile, which adds fin_wait
-// parked pieces: slots 0 .. fin_wait - 1).  The piece holding a tile's LAST k-block finishes it.
-struct SkShare { int n_dp, part_tile, part_kb0, part_kb1, part_slot, fin_tile, fin_kb0, fin_wait; };
-__host__ __device__ inline SkShare sk_share(const SkPlan& pl, int u, int U, int KB) {
-  SkShare sh{0, -1, 0, 0, 0, -1, 0, 0};
-  sh.n_dp = u < pl.first ? (pl.first - u + U - 1) / U : 0;
-  if (u >= pl.units) return sh;
-  const long W = (long)pl.tiles * KB;
-  const int s = (int)(((long)u * W) / pl.units), e = (int)(((long)(u + 1) * W) / pl.units);
-  const int ta = s / KB, tb = (e - 1) / KB;
-  const int uf = (int)((((long)ta * KB + 1) * pl.units - 1) / W);          // the pair whose range holds k-block 0 of tile ta
-  const int a0 = s - ta * KB;
-  if (tb > ta) {                       // tail of ta (finishes it) + head of the next tile (partial, slot 0)
-    sh.fin_tile = pl.first + ta; sh.fin_kb0 = a0; sh.fin_wait = u - uf;
-    sh.part_tile = pl.first + tb; sh.part_kb0 = 0; sh.part_kb1 = e - tb * KB; sh.part_slot = 0;
-  } else if (e - ta * KB == KB) {      // reaches the end of ta: finishes it
-    sh.fin_tile = pl.first + ta; sh.fin_kb0 = a0; sh.fin_wait = u - uf;
-  } else {                             // strictly inside ta (or its head): partial, slot = position among the tile's pieces
-    sh.part_tile = pl.first + ta; sh.part_kb0 = a0; sh.part_kb1 = e - ta * KB; sh.part_slot = u - uf;
-  }
-  return sh;
-}
 
 constexpr int GEMM_MAX_PROB = 4;
 struct GemmMultiMaps {
@@ -153,8 +93,6 @@ UB_DEVINL void gemm_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const C
   const uint32_t IDESC = p.ab_f16 ? (IDESC_BF16 & ~FMT_BF16) : IDESC_BF16;
   constexpr int CW = OUT32 ? 32 : 64;        // columns per epilogue slab
   constexpr int SLABS = (BN / 2) / CW;       // slabs per warp per tile
-  constexpr int NBUF = GemmCfg<BN, EPI, NCTA>::NBUF;
-  constexpr int EPI_BYTES = GemmCfg<BN, EPI, NCTA>::EPI_BYTES;
   static_assert(EPI != 1 || OUT32, "residual epilogue writes fp32");
   static_assert(EPI != 2 || !OUT32, "DGELU epilogue writes bf16");
   static_assert(EPI != 3 || !OUT32, "the fp16-residual epilogue writes fp16");
@@ -165,14 +103,14 @@ UB_DEVINL void gemm_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const C
   const bool leader = pr == 0;
 
   extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* epi_s = smem + STAGES * STAGE_BYTES;                       // [8 warps][NBUF][4096], 1024-aligned
+  uint8_t* epi_s = smem + STAGES * STAGE_BYTES;                       // [8 warps][2][4096], 1024-aligned
   float* bias_s = reinterpret_cast<float*>(epi_s + EPI_BYTES);         // [2][BN]
   uint64_t* full = reinterpret_cast<uint64_t*>(bias_s + 2 * BN);
   uint64_t* empty = full + STAGES;
   uint64_t* tfull = empty + STAGES;
   uint64_t* tempty = tfull + 2;
-  uint64_t* rbar = tempty + 2;                                         // [8 warps][3] residual / aux slab arrived
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(rbar + 24);
+  uint64_t* rbar = tempty + 2;                                         // [8 warps][2] residual / aux slab arrived
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(rbar + 16);
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -190,7 +128,7 @@ UB_DEVINL void gemm_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const C
       mbar_init(&tfull[i], 1);
       mbar_init(&tempty[i], 8 * CG);     // the leader's copy collects the epilogue warps of both CTAs
     }
-    for (int i = 0; i < 24; ++i) mbar_init(&rbar[i], 1);
+    for (int i = 0; i < 16; ++i) mbar_init(&rbar[i], 1);
     fence_mbar_init();
   }
   if (warp == 1) {
@@ -206,7 +144,6 @@ UB_DEVINL void gemm_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const C
   if (NCTA >= 2) cluster_sync(); else __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_grid_sync();     // everything above overlapped the previous kernel's tail; global memory is touched only below
 
   const int m_tiles = (p.M + BM * NCTA - 1) / (BM * NCTA);
   const int n_tiles = (p.N + BN - 1) / BN;
@@ -229,48 +166,14 @@ UB_DEVINL void gemm_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const C
   };
   const int w_first = blockIdx.x / NCTA, w_step = gridDim.x / NCTA;   // both CTAs of a pair walk the same work items
 
-  // ---- this pair's list of work items.  Ordinarily item i is work index w_first + i * w_step = (tile, k-split).  With a
-  // stream-K tail (p.sk_tiles > 0; CTA pairs on 256 x 256 tiles only; sk_plan / sk_share above) the pair works in the order
-  // [partial piece] [its whole tiles] [finishing piece]: partial accumulators (fp32, parked in the workspace by the epilogue warps
-  // and announced through a per-(tile, CTA, warp) counter) are written at the start of the kernel and consumed at its end, so the
-  // wait is off the critical path and cannot form a cycle (a partial piece waits for nothing).
-  // The stream-K tail is a BUILD option (-DUB_GEMM_STREAMK, libunite_b200_sk.so): compiled in, its item bookkeeping costs the ordinary
-  // whole-tile schedule 0.9 % of the step (17.385 vs 17.536 ms, A/B/A/B/A/B, profiles/ab_streamk_scaffolding_r02.txt) — more than any
-  // shape gains from it on B200 (profiles/gemm_streamk_r02.md) — so the default library is built without it.
-#ifdef UB_GEMM_STREAMK
-  constexpr bool SK_OK = NCTA == 2 && BN == 256 && !MULTI;
-#else
-  constexpr bool SK_OK = false;
-#endif
-  const bool sk = SK_OK && p.sk_tiles > 0;
-  int n_items, n_dp = 0;
-  int part_tile = -1, part_kb0 = 0, part_kb1 = 0, part_slot = 0;      // this pair's partial piece (at most one)
-  int fin_tile = -1, fin_kb0 = 0, fin_wait = 0;                        // this pair's finishing piece (at most one)
-  if (sk) {
-    const SkShare sh = sk_share(SkPlan{p.sk_first, p.sk_tiles, p.sk_units}, w_first, w_step, total_kb);
-    n_dp = sh.n_dp;
-    part_tile = sh.part_tile; part_kb0 = sh.part_kb0; part_kb1 = sh.part_kb1; part_slot = sh.part_slot;
-    fin_tile = sh.fin_tile; fin_kb0 = sh.fin_kb0; fin_wait = sh.fin_wait;
-    n_items = (part_tile >= 0 ? 1 : 0) + n_dp + (fin_tile >= 0 ? 1 : 0);
-  } else {
-    n_items = w_first < total_work ? (total_work - w_first + w_step - 1) / w_step : 0;
-  }
-  const int n_part = (sk && part_tile >= 0) ? 1 : 0;              // the partial piece comes first in the list
-  // item i -> (tile, k-block range, kind: 0 whole tile / k-split item, 1 partial piece (aux = slot), 2 finishing piece (aux = pieces to add))
-  auto get_item = [&](int i, int& tile, int& kb0, int& kb1, int& kind, int& aux) {
-    if (!sk) {
-      const int w = w_first + i * w_step, ks = w % p.splits;
-      tile = w / p.splits;
-      kb0 = ks * p.kb_per_split;
-      kb1 = min(total_kb, kb0 + p.kb_per_split);
-      kind = 0; aux = 0;
-    } else if (i < n_part) {
-      tile = part_tile; kb0 = part_kb0; kb1 = part_kb1; kind = 1; aux = part_slot;
-    } else if (i < n_part + n_dp) {
-      tile = w_first + (i - n_part) * w_step; kb0 = 0; kb1 = total_kb; kind = 0; aux = 0;
-    } else {
-      tile = fin_tile; kb0 = fin_kb0; kb1 = total_kb; kind = fin_wait > 0 ? 2 : 0; aux = fin_wait;
-    }
+  // ---- this pair's list of work items: item i is work index w_first + i * w_step = (tile, k-split)
+  const int n_items = w_first < total_work ? (total_work - w_first + w_step - 1) / w_step : 0;
+  // item i -> (tile, k-block range)
+  auto get_item = [&](int i, int& tile, int& kb0, int& kb1) {
+    const int w = w_first + i * w_step, ks = w % p.splits;
+    tile = w / p.splits;
+    kb0 = ks * p.kb_per_split;
+    kb1 = min(total_kb, kb0 + p.kb_per_split);
   };
 
   if (warp == 0) {
@@ -278,8 +181,8 @@ UB_DEVINL void gemm_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const C
     int stage = 0;
     uint32_t phase = 0;
     for (int it = 0; it < n_items; ++it) {
-      int tile, kb0, kb1, kind, aux;
-      get_item(it, tile, kb0, kb1, kind, aux);
+      int tile, kb0, kb1;
+      get_item(it, tile, kb0, kb1);
       int pi, tm, tn;
       decode(tile, pi, tm, tn);
       const CUtensorMap* pA = MULTI ? &mm->a[pi] : &tmA;
@@ -344,8 +247,8 @@ UB_DEVINL void gemm_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const C
     int as = 0;
     uint32_t aphase = 0;
     for (int it = 0; it < n_items; ++it) {
-      int tile, kb0, kb1, kind, aux;
-      get_item(it, tile, kb0, kb1, kind, aux);
+      int tile, kb0, kb1;
+      get_item(it, tile, kb0, kb1);
       if (NCTA >= 2) mbar_wait_cluster(&tempty[as], aphase ^ 1); else mbar_wait(&tempty[as], aphase ^ 1);
       tc_fence_after();
       const uint32_t d_tmem = tmem_base + (uint32_t)(as * BN);
@@ -386,9 +289,9 @@ UB_DEVINL void gemm_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const C
     const int sp = warp & 3;            // TMEM sub-partition this warp may read
     const int half = we >> 2;           // which half of the BN columns
     const int etid = threadIdx.x - 64;  // 0..255
-    uint8_t* const slab0 = epi_s + we * (NBUF * 4096);   // NBUF 4 KB staging slabs: slab0 + (b << 12)
+    uint8_t* const slab0 = epi_s + we * (2 * 4096);      // two 4 KB staging slabs: slab0 + (b << 12)
     const uint32_t slab0_a = smem_u32(slab0);
-    uint64_t* rb = rbar + we * 3;
+    uint64_t* rb = rbar + we * 2;
     const uint32_t sw = (uint32_t)(lane & 7);      // 16-byte chunk XOR of this lane's row (128B swizzle)
     const uint32_t rowoff = (uint32_t)lane * 128u;
     int as = 0;
@@ -396,8 +299,8 @@ UB_DEVINL void gemm_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const C
     uint32_t cc = 0;                    // running slab counter of this warp: staging buffer = cc & 1
     // (row, col) of this warp's slab `c` of work item `i`
     auto item_tile = [&](int i) {
-      int tile, kb0, kb1, kind, aux;
-      get_item(i, tile, kb0, kb1, kind, aux);
+      int tile, kb0, kb1;
+      get_item(i, tile, kb0, kb1);
       return tile;
     };
     auto slab_row = [&](int i) {
@@ -410,58 +313,14 @@ UB_DEVINL void gemm_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const C
       decode(item_tile(i), pi, tm, tn);
       return tn * BN + half * (BN / 2) + c * CW;
     };
-    // the partial piece of a stream-K tail comes first and uses neither the staging slabs nor the operand prefetch chain
-    if (EPI != 0 && EPI != 4 && n_part < n_items && lane == 0) {
-      // residual / pre-activation slabs of the first NBUF - 1 (tile, slab) pairs of this warp
+    if (EPI != 0 && EPI != 4 && n_items > 0 && lane == 0) {
+      // residual / pre-activation slab of the first (tile, slab) pair of this warp
       mbar_expect_tx(&rb[0], 4096);
-      tma_load_2d(&tmR, &rb[0], slab0, slab_col(n_part, 0), slab_row(n_part));
-      if (NBUF == 3) {
-        int ni = n_part, nc = 1;
-        if (nc == SLABS) { nc = 0; ++ni; }
-        if (ni < n_items) {
-          mbar_expect_tx(&rb[1], 4096);
-          tma_load_2d(&tmR, &rb[1], slab0 + 4096, slab_col(ni, nc), slab_row(ni));
-        }
-      }
+      tma_load_2d(&tmR, &rb[0], slab0, slab_col(0, 0), slab_row(0));
     }
-    // this warp's corner of the stream-K workspace: a [32 rows x 128 columns] fp32 block per (sk tile, slot, CTA, warp), stored as
-    // four 32 x 32 sub-blocks in register order (float4 j of lane l at (j * 32 + l) * 16 bytes: 512 contiguous bytes per access)
-    uint32_t* const sk_flags = reinterpret_cast<uint32_t*>(p.sk_ws);
-    float* const sk_data = p.sk_ws + SK_FLAG_BYTES / 4;
-    if (SK_OK && n_part) {
-      // ---- partial piece: accumulators -> workspace, then announce them
-      const int ti = part_tile - p.sk_first;
-      float* dst = sk_data + (size_t)((((ti * 2 + part_slot) * 2 + (int)pr) * 8 + we)) * 4096 + lane * 4;
-      mbar_wait(&tfull[as], aphase);
-      tc_fence_after();
-      const uint32_t t_row = tmem_base + ((uint32_t)(sp * 32) << 16) + (uint32_t)(as * BN + half * (BN / 2));
-#pragma unroll 1
-      for (int blk = 0; blk < (BN / 2) / 32; ++blk) {
-        uint32_t r[32];
-        tmem_ld_32x32(t_row + (uint32_t)(blk * 32), r);
-        tmem_ld_wait();
-#pragma unroll
-        for (int j = 0; j < 8; ++j)
-          asm volatile("st.global.cg.v4.b32 [%0], {%1, %2, %3, %4};" ::"l"(dst + blk * 1024 + j * 128), "r"(r[4 * j]), "r"(r[4 * j + 1]),
-                       "r"(r[4 * j + 2]), "r"(r[4 * j + 3])
-                       : "memory");
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) {
-        __threadfence();
-        atomicAdd(sk_flags + (ti * 2 + (int)pr) * 8 + we, 1u);
-        if (NCTA >= 2) mbar_arrive_cluster(mapa_u32(smem_u32(&tempty[as]), leader_rank)); else mbar_arrive(&tempty[as]);
-      }
-      as ^= 1;
-      if (as == 0) aphase ^= 1;
-    }
-    for (int it = n_part; it < n_items; ++it) {
-      int w_tile, w_kb0, w_kb1, w_kind, w_aux;
-      get_item(it, w_tile, w_kb0, w_kb1, w_kind, w_aux);
+    for (int w = 0; w < n_items; ++w) {
       int w_pi, w_tm, w_tn;
-      decode(w_tile, w_pi, w_tm, w_tn);
-      const int w = it;       // slab_row / slab_col take the item index
+      decode(item_tile(w), w_pi, w_tm, w_tn);
       const CUtensorMap* pC = MULTI ? &mm->c[w_pi] : &tmC;
       const int n0 = w_tn * BN;
       const int row0 = slab_row(w);
@@ -487,48 +346,12 @@ UB_DEVINL void gemm_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const C
         }
       }
       float st1 = 0.0f, st2 = 0.0f;             // EPI 3: row statistics of the fp16 values this thread writes
-      // finishing piece of a stream-K tile: the other pieces' accumulators for the next 32 x 32 block travel one block ahead
-      float4 skp[SK_OK ? 8 : 1];
-      const float* sk_src = nullptr;
-      const int sk_add = (SK_OK && w_kind == 2) ? w_aux : 0;
-      auto sk_fetch = [&](int blk) {
-#pragma unroll
-        for (int j = 0; j < (SK_OK ? 8 : 1); ++j) {
-          const float* a = sk_src + blk * 1024 + j * 128;
-          asm volatile("ld.global.cg.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(skp[j].x), "=f"(skp[j].y), "=f"(skp[j].z), "=f"(skp[j].w) : "l"(a) : "memory");
-        }
-        if (sk_add > 1) {
-#pragma unroll
-          for (int j = 0; j < (SK_OK ? 8 : 1); ++j) {
-            float4 t;
-            const float* a = sk_src + 2 * 8 * 4096 + blk * 1024 + j * 128;     // slot 1
-            asm volatile("ld.global.cg.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(t.x), "=f"(t.y), "=f"(t.z), "=f"(t.w) : "l"(a) : "memory");
-            skp[j].x += t.x; skp[j].y += t.y; skp[j].z += t.z; skp[j].w += t.w;
-          }
-        }
-      };
-      if (SK_OK && sk_add > 0) {
-        const int ti = w_tile - p.sk_first;
-        uint32_t* flag = sk_flags + (ti * 2 + (int)pr) * 8 + we;
-        if (lane == 0) {
-          uint32_t seen;
-          const long long t0 = clock64();
-          do {
-            asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(seen) : "l"(flag) : "memory");
-            if ((int)seen < sk_add && clock64() - t0 > 20000000000ll) __trap();      // ~10 s: a partial piece never arrived
-          } while ((int)seen < sk_add);
-          *flag = 0u;          // zero again for the next launch (nobody else touches it any more in this one)
-        }
-        __syncwarp();
-        sk_src = sk_data + (size_t)(((ti * 2) * 2 + (int)pr) * 8 + we) * 4096 + lane * 4;
-        sk_fetch(0);
-      }
       mbar_wait(&tfull[as], aphase);
       tc_fence_after();
       const uint32_t t_row = tmem_base + ((uint32_t)(sp * 32) << 16) + (uint32_t)(as * BN + half * (BN / 2));
 #pragma unroll 1
       for (int c = 0; c < SLABS; ++c, ++cc) {
-        const int b = NBUF == 3 ? (int)(cc % 3u) : (int)(cc & 1u);
+        const int b = (int)(cc & 1u);
         const int col0 = slab_col(w, c);
         // ---- staging-buffer hand-over with the TMA engine
         if (EPI == 0 || EPI == 4) {
@@ -538,20 +361,19 @@ UB_DEVINL void gemm_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const C
           }
           __syncwarp();
         } else {
-          // the store of the previous slab read buffer (cc - 1) % NBUF: once done, the operand of the slab NBUF - 1 ahead is
-          // prefetched into it
+          // the store of the previous slab read buffer b ^ 1: once done, the operand of the next slab is prefetched into it
           if (lane == 0) {
             tma_store_wait_read<0>();
-            int nw = w, nc = c + (NBUF - 1);
+            int nw = w, nc = c + 1;
             while (nc >= SLABS) { nc -= SLABS; ++nw; }
             if (nw < n_items) {
-              const int nb = NBUF == 3 ? (int)((cc + 2u) % 3u) : (b ^ 1);
+              const int nb = b ^ 1;
               mbar_expect_tx(&rb[nb], 4096);
               tma_load_2d(&tmR, &rb[nb], slab0 + (nb << 12), slab_col(nw, nc), slab_row(nw));
             }
           }
           __syncwarp();
-          mbar_wait(&rb[b], NBUF == 3 ? ((cc / 3u) & 1u) : ((cc >> 1) & 1u));
+          mbar_wait(&rb[b], (cc >> 1) & 1u);
         }
         // ---- accumulators -> registers -> epilogue math -> staging slab (row per lane, 128 B per row)
         float dsum = 0.0f;        // UB_ACT_DOT_AUX: this lane's row of the slab (64 columns = one head) dotted with aux
@@ -572,14 +394,6 @@ UB_DEVINL void gemm_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const C
           float v[32];
 #pragma unroll
           for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-          if (SK_OK && sk_add > 0) {
-#pragma unroll
-            for (int j = 0; j < (SK_OK ? 8 : 1); ++j) {
-              v[4 * j] += skp[j].x; v[4 * j + 1] += skp[j].y; v[4 * j + 2] += skp[j].z; v[4 * j + 3] += skp[j].w;
-            }
-            const int blk = c * (CW / 32) + h + 1;
-            if (blk < (BN / 2) / 32) sk_fetch(blk);
-          }
           if (EPI == 4) {
             const float2 rs2 = make_float2(ln_rstd, ln_rstd), nrm2 = make_float2(-ln_rm, -ln_rm);
 #pragma unroll
@@ -855,11 +669,9 @@ struct GemmMaps {
   CUtensorMap a, b, c, r, x;
 };
 
-template <int BN, int STAGES_REQ, bool A_MN, bool B_MN, int EPI, bool OUT32, int NCTA>
+template <int BN, int STAGES, bool A_MN, bool B_MN, int EPI, bool OUT32, int NCTA>
 static int launch_gemm_epi(const GemmMaps& m, const GemmParams& p, int grid, cudaStream_t stream) {
-  constexpr int STAGES = GemmCfg<BN, EPI, NCTA>::stages(STAGES_REQ);
-  constexpr int SMEM = STAGES * (BM * BK * 2 + (BN / (NCTA >= 2 ? 2 : 1)) * BK * 2) + GemmCfg<BN, EPI, NCTA>::EPI_BYTES + 2 * BN * 4 +
-                       (2 * STAGES + 4 + 24) * 8 + 16;
+  constexpr int SMEM = gemm_smem_bytes(BN, STAGES, NCTA);
   static_assert(SMEM <= 232448, "exceeds the 227 KB per-CTA shared memory limit");
   static bool configured = false;
   auto kern = gemm_kernel<BN, STAGES, A_MN, B_MN, EPI, OUT32, NCTA>;
@@ -873,15 +685,13 @@ static int launch_gemm_epi(const GemmMaps& m, const GemmParams& p, int grid, cud
   cfg.blockDim = dim3(GEMM_THREADS);
   cfg.dynamicSmemBytes = SMEM;
   cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
+  cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
   attr[0].val.clusterDim.x = NCTA;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 2 : 1;
+  cfg.numAttrs = 1;
   cudaError_t e = cudaLaunchKernelEx(&cfg, kern, m.a, m.b, m.c, m.r, m.x, p);
   UB_REQUIRE(e == cudaSuccess, "gemm_kernel launch: %s", cudaGetErrorString(e));
   return check_launch("gemm_kernel");
@@ -892,7 +702,7 @@ static int max_clusters4() {
   static int cached = -1;
   if (cached >= 0) return cached;
   auto kern = gemm_kernel<256, 5, false, false, 0, false, 4>;
-  constexpr int SMEM = 5 * (BM * BK * 2 + 128 * BK * 2) + GemmCfg<256, 0, 4>::EPI_BYTES + 2 * 256 * 4 + (2 * 5 + 4 + 24) * 8 + 16;
+  constexpr int SMEM = gemm_smem_bytes(256, 5, 4);
   int n = 0;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM) == cudaSuccess) {
     cudaLaunchConfig_t q{};
@@ -936,28 +746,6 @@ static int launch_gemm(const GemmMaps& m, const GemmParams& p, int epi, bool out
 }  // namespace ub
 
 extern "C" int ub_gemm_cluster4_capacity(void) { return ub::max_clusters4(); }
-extern "C" int64_t ub_gemm_sk_launches(void) { return ub::g_sk_launches; }
-extern "C" int ub_gemm_sk_compiled(void) {
-#ifdef UB_GEMM_STREAMK
-  return 1;
-#else
-  return 0;
-#endif
-}
-// test hook: the stream-K plan for T tiles on U pairs with KB k-blocks per tile and pair u's share of it, as the kernel computes them
-// out = {first, tiles, units, n_dp, part_tile, part_kb0, part_kb1, part_slot, fin_tile, fin_kb0, fin_wait}; returns 1 if the tail is split
-extern "C" int ub_gemm_sk_schedule(int T, int U, int KB, int overhead, int u, int32_t* out) {
-  const ub::SkPlan pl = ub::sk_plan(T, U, KB, overhead);
-  const ub::SkShare sh = ub::sk_share(pl, u, U, KB);
-  const int32_t v[11] = {pl.first, pl.tiles, pl.units, sh.n_dp, sh.part_tile, sh.part_kb0, sh.part_kb1, sh.part_slot, sh.fin_tile, sh.fin_kb0, sh.fin_wait};
-  if (out) memcpy(out, v, sizeof(v));
-  return pl.tiles > 0 ? 1 : 0;
-}
-extern "C" int64_t ub_gemm_sk_workspace_bytes(void) {
-  // the tail of a persistent schedule on sms / 2 CTA pairs holds at most sms / 2 - 1 tiles
-  const int64_t tiles = ub::sm_count() / 2 < ub::SK_MAX_TILES ? ub::sm_count() / 2 : ub::SK_MAX_TILES;
-  return ub::SK_FLAG_BYTES + tiles * (int64_t)ub::SK_TILE_BYTES;
-}
 
 extern "C" int ub_gemm_wgrad_multi(const ub_gemm_problem* pr, int n, int K, int split_k, void* stream) {
   using namespace ub;
@@ -993,7 +781,7 @@ extern "C" int ub_gemm_wgrad_multi(const ub_gemm_problem* pr, int n, int K, int 
   const int units = sm_count() / 2;
   const int grid = (int)(total_work < units ? total_work : units) * 2;
   constexpr int STAGES = 5;
-  constexpr int SMEM = STAGES * (BM * BK * 2 + 128 * BK * 2) + GemmCfg<256, 0, 2>::EPI_BYTES + 2 * 256 * 4 + (2 * STAGES + 4 + 24) * 8 + 16;
+  constexpr int SMEM = gemm_smem_bytes(256, STAGES, 2);
   static_assert(SMEM <= 232448, "exceeds the 227 KB per-CTA shared memory limit");
   static bool configured = false;
   auto kern = gemm_multi_kernel<STAGES>;
@@ -1007,13 +795,11 @@ extern "C" int ub_gemm_wgrad_multi(const ub_gemm_problem* pr, int n, int K, int 
   cfg.blockDim = dim3(GEMM_THREADS);
   cfg.dynamicSmemBytes = SMEM;
   cfg.stream = reinterpret_cast<cudaStream_t>(stream);
-  cudaLaunchAttribute attr[2];
+  cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
   attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 2 : 1;
+  cfg.numAttrs = 1;
   cudaError_t e = cudaLaunchKernelEx(&cfg, kern, mm, p);
   UB_REQUIRE(e == cudaSuccess, "gemm_multi_kernel launch: %s", cudaGetErrorString(e));
   return check_launch("gemm_multi_kernel");
@@ -1153,34 +939,7 @@ extern "C" int ub_gemm_bf16(const void* A, int64_t lda, int a_mn_major, const vo
   const long total_work = (long)((M + BM * ncta - 1) / (BM * ncta)) * ((N + bn - 1) / bn) * split_k;
   int units = ncta == 4 ? units4 : sms / ncta;
   if (ep.max_ctas > 0 && ep.max_ctas / ncta >= 1 && ep.max_ctas / ncta < units) units = ep.max_ctas / ncta;
-  // stream-K tail: when the last wave of 256 x 256 pair tiles is partial, cut its R tiles along K over all the pairs.  Time in
-  // k-blocks per pair: whole tiles ceil(T / U) * KB; with the tail split floor(T / U) * KB + ceil(R * KB / U') + a fix-up charge
-  // (the partial accumulators' round trip through L2 and the finishing epilogue that waits for them; UB_GEMM_SK_OVERHEAD, in
-  // k-blocks).  U' <= U keeps every range at least half a tile long (at most three pieces per tile, two workspace slots).
-  p.sk_first = p.sk_tiles = p.sk_units = 0;
-  p.sk_ws = nullptr;
-  static int sk_overhead = -1;
-  if (sk_overhead < 0) {
-    const char* o = getenv("UB_GEMM_SK_OVERHEAD");
-    sk_overhead = o ? atoi(o) : 4;
-    if (sk_overhead < 0) sk_overhead = 0;
-  }
-#ifdef UB_GEMM_STREAMK
-  if (ep.sk_workspace != nullptr && ncta == 2 && bn == 256 && split_k == 1 && ep.group_rows == 0 && ep.max_ctas >= 0 &&
-      total_work > 0 && total_work < (1l << 30)) {
-    const SkPlan pl = sk_plan((int)total_work, units, total_kb, sk_overhead);
-    const int64_t need = SK_FLAG_BYTES + (int64_t)pl.tiles * (int64_t)SK_TILE_BYTES;
-    if (pl.tiles > 0 && ep.sk_workspace_bytes >= need && (reinterpret_cast<uintptr_t>(ep.sk_workspace) & 15) == 0) {
-      p.sk_first = pl.first; p.sk_tiles = pl.tiles; p.sk_units = pl.units;
-      p.sk_ws = reinterpret_cast<float*>(ep.sk_workspace);
-      ++g_sk_launches;
-    }
-  }
-#else
-  (void)sk_overhead;
-#endif
-  int grid = (int)(total_work < units ? total_work : units) * ncta;
-  if (p.sk_tiles > 0) grid = (p.sk_first > 0 ? units : p.sk_units) * ncta;      // every pair of the split takes part
+  const int grid = (int)(total_work < units ? total_work : units) * ncta;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
 
 #define UB_GEMM_CASE(AMN, BMN)                                                                       \

@@ -17,7 +17,6 @@ namespace ub {
 
 // out[b, d] = mean_n x[b, n, d];  grid (D/128, B), 128 threads, each thread one column, rows strided by 8 sub-rows
 __global__ void __launch_bounds__(256) meanpool_fwd_kernel(const float* __restrict__ x, float* __restrict__ out, int N, int D) {
-  pdl_grid_sync();
   __shared__ float s_part[8][32];
   const int b = blockIdx.y, d = blockIdx.x * 32 + (threadIdx.x & 31), rg = threadIdx.x >> 5;
   float acc = 0.f;
@@ -38,7 +37,6 @@ __global__ void __launch_bounds__(256) meanpool_fwd_kernel(const float* __restri
 // dx[b, n, :] = g[b, :] / N   (fp32, 128-bit stores)
 __global__ void __launch_bounds__(256) meanpool_bwd_kernel(const float4* __restrict__ g, float4* __restrict__ dx, int N, int D4,
                                                            long total4, float invN) {
-  pdl_grid_sync();
   for (long id = (long)blockIdx.x * blockDim.x + threadIdx.x; id < total4; id += (long)gridDim.x * blockDim.x) {
     const int d4 = (int)(id % D4);
     const long b = id / ((long)N * D4);
@@ -52,7 +50,6 @@ __global__ void __launch_bounds__(256) meanpool_bwd_kernel(const float4* __restr
 __global__ void __launch_bounds__(256) linear_small_fwd_kernel(const float* __restrict__ x, const float* __restrict__ W,
                                                                const float* __restrict__ bias, float* __restrict__ out, int B,
                                                                int C, int D) {
-  pdl_grid_sync();
   const int w = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (w >= B * C) return;
   const int b = w / C, c = w % C;
@@ -66,7 +63,6 @@ __global__ void __launch_bounds__(256) linear_small_fwd_kernel(const float* __re
 __global__ void __launch_bounds__(256) linear_small_bwd_kernel(const float* __restrict__ x, const float* __restrict__ W,
                                                                const float* __restrict__ dout, float* __restrict__ dx,
                                                                float* __restrict__ dW, float* __restrict__ db, int B, int C, int D) {
-  pdl_grid_sync();
   const int d = blockIdx.x * blockDim.x + threadIdx.x;
   if (d < D) {
     if (dx != nullptr) {
@@ -96,7 +92,6 @@ __global__ void __launch_bounds__(256) linear_small_bwd_kernel(const float* __re
 __global__ void __launch_bounds__(256) softmax_ce_kernel(const float* __restrict__ logits, const int* __restrict__ labels,
                                                          const float* __restrict__ weights, float scale, float* __restrict__ loss_acc,
                                                          float* __restrict__ dlogits, int B, int C) {
-  pdl_grid_sync();
   const int b = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (b >= B) return;
   const float* l = logits + (int64_t)b * C;
@@ -122,7 +117,6 @@ __global__ void __launch_bounds__(256) softmax_ce_kernel(const float* __restrict
 __global__ void __launch_bounds__(256) soft_target_ce_kernel(const float* __restrict__ logits, const int* __restrict__ labels,
                                                              const float* __restrict__ mix, float scale, float* __restrict__ loss_acc,
                                                              float* __restrict__ dlogits, int B, int C) {
-  pdl_grid_sync();
   const int b = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (b >= B) return;
   const float lam = mix[0], on = mix[1], off = mix[2], lam1 = 1.0f - lam;
@@ -152,7 +146,6 @@ __global__ void __launch_bounds__(256) soft_target_ce_kernel(const float* __rest
 // probs[b, c] = mean_t softmax_c(100 * <img[b*T+t]/|.|, txt[c]/|.|>)   one block per clip, one warp per frame, C <= 32*? (loop)
 __global__ void __launch_bounds__(256) clip_zero_shot_kernel(const float* __restrict__ img, const float* __restrict__ txt,
                                                              float* __restrict__ probs, int T, int C, int D) {
-  pdl_grid_sync();
   extern __shared__ float s_acc[];   // [C] accumulated probabilities, then [warps][C] similarities
   const int b = blockIdx.x, warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
   float* sim = s_acc + C + warp * C;
@@ -192,7 +185,6 @@ __global__ void __launch_bounds__(256) pseudo_label_fusion_kernel(const float* _
                                                                   float thr, int conf_weighted, float* __restrict__ msp_out,
                                                                   int* __restrict__ pseudo, uint8_t* __restrict__ sel,
                                                                   float* __restrict__ weight, int B, int C) {
-  pdl_grid_sync();
   const int b = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (b >= B) return;
   const float* l = logits + (int64_t)b * C;

@@ -131,7 +131,6 @@ struct LnFwdArgs {
 
 template <int NV>
 __global__ void __launch_bounds__(256) ln_fwd_kernel(const LnFwdArgs a) {
-  pdl_grid_sync();
   const int lane = threadIdx.x & 31;
   constexpr int nv = NV;
   const int wpb = blockDim.x >> 5;
@@ -171,7 +170,6 @@ __global__ void __launch_bounds__(256) teacher_embed_ln_kernel(const float* __re
                                                                const float* __restrict__ beta, void* __restrict__ out,
                                                                int frames, int P, int D, float eps, int out_f16,
                                                                float* __restrict__ stats) {
-  pdl_grid_sync();
   const int lane = threadIdx.x & 31;
   constexpr int nv = NV;
   const int wpb = blockDim.x >> 5;
@@ -257,7 +255,6 @@ UB_DEVINL void block_col_reduce_atomic(const RowT<NV>& part, float* s_buf, float
 // warps.
 template <int NV>
 __global__ void __launch_bounds__(128, 4) ln_bwd_kernel(const LnBwdArgs a) {
-  pdl_grid_sync();
   extern __shared__ float s_red[];  // [warps][3][D]
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   constexpr int nv = NV;
@@ -339,7 +336,6 @@ __global__ void __launch_bounds__(128, 4) ln_bwd_kernel(const LnBwdArgs a) {
 constexpr int LNB_ROWS = 8;          // rows per block = consumer warps
 template <int NV>
 __global__ void __launch_bounds__(256, 1) ln_bwd_staged_kernel(const LnBwdArgs a, int n_stages) {
-  pdl_grid_sync();
   extern __shared__ __align__(128) uint8_t lnb_smem[];
   constexpr int D = NV * 128;
   constexpr int X_BYTES = LNB_ROWS * D * 4, DY_BYTES = LNB_ROWS * D * 2;
@@ -461,7 +457,6 @@ __global__ void __launch_bounds__(256) dec_tail_fwd_kernel(const float* __restri
                                                            const float* __restrict__ tgt, float* __restrict__ loss_acc,
                                                            float loss_scale, int rows, int D, float eps, int loss_lo,
                                                            int loss_hi) {
-  pdl_grid_sync();
   __shared__ float s_loss[8];
   const int lane = threadIdx.x & 31;
   constexpr int nv = NV;
@@ -509,7 +504,6 @@ __global__ void __launch_bounds__(256) dec_tail_bwd_kernel(const float* __restri
                                                            float go_scale, bf16* __restrict__ dy_out, float* __restrict__ dgamma,
                                                            float* __restrict__ dbeta, int rows, int D, float eps, int go_lo,
                                                            int go_hi) {
-  pdl_grid_sync();
   extern __shared__ float s_red[];
   const int lane = threadIdx.x & 31;
   constexpr int nv = NV;
@@ -562,7 +556,6 @@ __global__ void __launch_bounds__(256) dec_tail_bwd_kernel(const float* __restri
 // x[row] /= ||x[row]||   (teacher targets, clip.py:173)
 template <int NV>
 __global__ void __launch_bounds__(256) l2norm_rows_kernel(float* __restrict__ x, int rows, int D) {
-  pdl_grid_sync();
   const int lane = threadIdx.x & 31;
   constexpr int nv = NV;
   const int wpb = blockDim.x >> 5;

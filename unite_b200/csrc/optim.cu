@@ -12,7 +12,6 @@ namespace ub {
 
 // sum of squares of a flat fp32 buffer, accumulated into out[0] with one red.add per block
 __global__ void __launch_bounds__(256) sumsq_kernel(const float4* __restrict__ g, long n4, float* __restrict__ out) {
-  pdl_grid_sync();
   __shared__ float s_part[8];
   float acc = 0.f;
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long)gridDim.x * blockDim.x) {
@@ -35,7 +34,6 @@ __global__ void __launch_bounds__(256) adamw_kernel(float4* __restrict__ p, cons
                                                     float4* __restrict__ v, uint2* __restrict__ w_bf16, long n4, long n4_decay,
                                                     float lr, float wd, float beta1, float beta2, float eps, float bc1,
                                                     float bc2_sqrt, float grad_scale) {
-  pdl_grid_sync();
   const float step_size = lr / bc1;
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long)gridDim.x * blockDim.x) {
     float4 pp = p[i], gg = g[i], mm = m[i], vv = v[i];
@@ -66,7 +64,6 @@ __global__ void __launch_bounds__(256) adamw_kernel(float4* __restrict__ p, cons
 __global__ void __launch_bounds__(256) adamw_dev_kernel(float4* __restrict__ p, const float4* __restrict__ g, float4* __restrict__ m,
                                                         float4* __restrict__ v, uint2* __restrict__ w_bf16, long n4, long n4_decay,
                                                         const float* __restrict__ hyper, float* __restrict__ gnorm_sq) {
-  pdl_grid_sync();
   __shared__ float s_part[8];
   float gacc = 0.f;                    // sum of squares of the raw gradients this thread reads (utils.py:631-643 for free)
   const float lr = hyper[0], wd = hyper[1], beta1 = hyper[2], beta2 = hyper[3], eps = hyper[4], bc1 = hyper[5], bc2_sqrt = hyper[6],
@@ -118,7 +115,6 @@ __global__ void __launch_bounds__(256) adamw_seg_kernel(float4* __restrict__ p, 
                                                         float4* __restrict__ v, uint2* __restrict__ w_bf16, long n4,
                                                         const int* __restrict__ seg_end4, int n_seg, const float* __restrict__ hyper,
                                                         float* __restrict__ gnorm_sq) {
-  pdl_grid_sync();
   __shared__ float s_part[8];
   __shared__ float s_lr[kMaxSeg], s_wd[kMaxSeg];
   __shared__ int s_end[kMaxSeg];
@@ -172,7 +168,6 @@ __global__ void __launch_bounds__(256) adamw_seg_kernel(float4* __restrict__ p, 
 // sum of squares over the non-frozen groups only (clip_grad needs the norm before the update)
 __global__ void __launch_bounds__(256) sumsq_seg_kernel(const float4* __restrict__ g, long n4, const int* __restrict__ seg_end4, int n_seg,
                                                         const float* __restrict__ hyper, float* __restrict__ out) {
-  pdl_grid_sync();
   __shared__ float s_part[8];
   __shared__ float s_wd[kMaxSeg];
   __shared__ int s_end[kMaxSeg];
@@ -200,7 +195,6 @@ __global__ void __launch_bounds__(256) sumsq_seg_kernel(const float4* __restrict
 }
 
 __global__ void __launch_bounds__(256) cast_bf16_kernel(const float4* __restrict__ x, uint2* __restrict__ out, long n4) {
-  pdl_grid_sync();
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long)gridDim.x * blockDim.x) {
     const float4 v = x[i];
     uint2 o;
@@ -215,7 +209,6 @@ __global__ void __launch_bounds__(256) cast_bf16_kernel(const float4* __restrict
 // written in the same pass, so the EMA model can be evaluated at any time without a cast pass.
 __global__ void __launch_bounds__(256) ema_update_kernel(float4* __restrict__ ema, uint2* __restrict__ ema_w16, const float4* __restrict__ p,
                                                          long n4, float decay, float one_minus_decay) {
-  pdl_grid_sync();
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long)gridDim.x * blockDim.x) {
     float4 e = ema[i];
     const float4 q = p[i];

@@ -32,7 +32,6 @@ UB_DEVINL void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
 // out[(l*2 + branch)*B + b] = floor(keep_l + u) / keep_l; one block, every thread reads the step before thread 0 bumps it
 __global__ void __launch_bounds__(256) drop_path_draw_kernel(const float* __restrict__ rates, float* __restrict__ out, int depth, int B,
                                                              uint32_t seed_lo, uint32_t seed_hi, unsigned long long* __restrict__ step) {
-  pdl_grid_sync();
   const unsigned long long s = *step;
   __syncthreads();
   const int n = depth * 2 * B;

@@ -3,7 +3,6 @@
 #include "../../include/unite_b200.h"
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 
 namespace ub {
 
@@ -35,15 +34,6 @@ int sm_count() {
       n = 148;
   }
   return (g_sm_limit > 0 && g_sm_limit < n) ? g_sm_limit : n;
-}
-
-bool pdl_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("UB_PDL");
-    on = e ? (atoi(e) != 0) : 0;   // measured on B200 inside the CUDA-graph step: 20.1 ms with, 19.1 ms without -> off by default
-  }
-  return on != 0;
 }
 
 }  // namespace ub

@@ -23,7 +23,6 @@ namespace ub {
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) patchify_kernel(const float* __restrict__ x, bf16* __restrict__ out, int B, int T,
                                                        int H, int W, int tub, long total_runs) {
-  pdl_grid_sync();
   const int gh = H / 16, gw = W / 16, Tp = T / tub;
   const int runs_per_tok = 3 * tub * 16;
   for (long id = (long)blockIdx.x * blockDim.x + threadIdx.x; id < total_runs; id += (long)gridDim.x * blockDim.x) {
@@ -57,7 +56,6 @@ __global__ void __launch_bounds__(256) patchify_kernel(const float* __restrict__
 __global__ void __launch_bounds__(256) patchify_mix_kernel(const float* __restrict__ x, bf16* __restrict__ out,
                                                            const float* __restrict__ mix, int B, int T, int H, int W, int tub,
                                                            long total_runs) {
-  pdl_grid_sync();
   const bool apply = mix[0] != 0.f, cut = mix[3] != 0.f;
   const float lam = mix[1], lam1 = mix[2];
   const int t0 = (int)mix[4], t1 = (int)mix[5], h0 = (int)mix[6], h1 = (int)mix[7], w0 = (int)mix[8], w1 = (int)mix[9];
@@ -162,7 +160,6 @@ UB_DEVINL float u8_norm(uint8_t u, float mean, float sd) { return __fdiv_rn(__fs
 __global__ void __launch_bounds__(256) patchify_u8_kernel(const uint8_t* __restrict__ x, bf16* __restrict__ out, float m0, float m1,
                                                           float m2, float s0, float s1, float s2, int B, int T, int H, int W, int tub,
                                                           long total_runs) {
-  pdl_grid_sync();
   const float mean[3] = {m0, m1, m2}, sd[3] = {s0, s1, s2};
   for (long id = (long)blockIdx.x * blockDim.x + threadIdx.x; id < total_runs; id += (long)gridDim.x * blockDim.x) {
     const U8Run r = u8_run(id, T, H, W, tub);
@@ -198,7 +195,6 @@ __global__ void __launch_bounds__(256) patchify_mix_u8_kernel(const uint8_t* __r
     lut[c][i % 256] = u8_norm((uint8_t)(i % 256), c == 0 ? m0 : (c == 1 ? m1 : m2), c == 0 ? s0 : (c == 1 ? s1 : s2));
   }
   __syncthreads();
-  pdl_grid_sync();
   const bool apply = mix[0] != 0.f, cut = mix[3] != 0.f;
   const float lam = mix[1], lam1 = mix[2];
   const int t0 = (int)mix[4], t1 = (int)mix[5], h0 = (int)mix[6], h1 = (int)mix[7], w0 = (int)mix[8], w1 = (int)mix[9];
@@ -286,7 +282,6 @@ template <bool U8>
 __global__ void __launch_bounds__(256) resize_patchify_kernel(const void* __restrict__ xin, bf16* __restrict__ out, long ld, float m0,
                                                               float m1, float m2, float s0, float s1, float s2, int T, int H, int W,
                                                               int R, int p, int tub, int rows_max, float sy, float sx, int identity) {
-  pdl_grid_sync();
   extern __shared__ float rp_smem[];
   const int gr = R / p, Tp = T / tub;
   int blk = blockIdx.x;
@@ -403,7 +398,6 @@ __global__ void __launch_bounds__(128) mask_select_kernel(const float* __restric
                                                           uint8_t* __restrict__ mask, int* __restrict__ vis_idx,
                                                           int* __restrict__ tea_rows, int frames, int P, int T, int k,
                                                           int n_vis) {
-  pdl_grid_sync();
   extern __shared__ float s_scores[];  // [warps][P] scores, then ranks as int
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int f = blockIdx.x * (blockDim.x >> 5) + warp;
@@ -456,7 +450,6 @@ __global__ void __launch_bounds__(128) mask_select_kernel(const float* __restric
 __global__ void __launch_bounds__(256) gather_rows_kernel(const uint4* __restrict__ in, const int* __restrict__ idx,
                                                           uint4* __restrict__ out, long n_rows, int chunks_per_row,
                                                           int rows_per_group, long group_stride) {
-  pdl_grid_sync();
   const long total = n_rows * chunks_per_row;
   for (long id = (long)blockIdx.x * blockDim.x + threadIdx.x; id < total; id += (long)gridDim.x * blockDim.x) {
     const long r = id / chunks_per_row;
@@ -475,7 +468,6 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const uint4* __restric
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) colsum_bf16_kernel(const bf16* __restrict__ x, int64_t ld, float* __restrict__ out,
                                                           int M, int N, int CS_ROWS, int skip_lo, int skip_hi) {
-  pdl_grid_sync();
   __shared__ float s_part[8][256];
   const int lane = threadIdx.x & 31, rg = threadIdx.x >> 5;
   const int col = blockIdx.x * 256 + lane * 8;
@@ -516,7 +508,6 @@ __global__ void __launch_bounds__(256) colsum_bf16_kernel(const bf16* __restrict
 __global__ void __launch_bounds__(256) cast_scale_bf16_kernel(const float4* __restrict__ x, uint2* __restrict__ out,
                                                               const float* __restrict__ row_scale, int rows_per_scale,
                                                               long n4, int d4) {
-  pdl_grid_sync();
   for (long id = (long)blockIdx.x * blockDim.x + threadIdx.x; id < n4; id += (long)gridDim.x * blockDim.x) {
     float4 v = x[id];
     if (row_scale) {

@@ -5,7 +5,6 @@ and calls straight into libunite_b200.so.  torch is used for memory and streams 
 implementation of any op behind these functions, and no fallback.
 """
 import ctypes as C
-import os
 from typing import Optional
 
 import torch
@@ -71,28 +70,10 @@ def _p2d(t: torch.Tensor, dtype, what):
     return t.data_ptr(), t.stride(0)
 
 
-# Stream-K scratch of the GEMM (ub_gemm_epilogue.sk_workspace): one zero-filled buffer per (device, stream) — the library
-# requires that a workspace serves one stream at a time.  Allocated on first use; a buffer first requested while a CUDA graph is
-# being captured lives in that graph's pool and stays alive here.
-_SK_WS = {}
-_SK_DEFAULT = os.environ.get("UB_GEMM_SK", "0") not in ("", "0")
-_SK_COMPILED = bool(lib.ub_gemm_sk_compiled())      # only libunite_b200_sk.so (UB_LIB_VARIANT=sk) contains the schedule
-
-
-def _sk_workspace(ep):
-    st = _stream()
-    key = (torch.cuda.current_device(), st)
-    ws = _SK_WS.get(key)
-    if ws is None:
-        ws = torch.zeros(int(lib.ub_gemm_sk_workspace_bytes()), dtype=U8, device="cuda")
-        _SK_WS[key] = ws
-    ep.sk_workspace, ep.sk_workspace_bytes = ws.data_ptr(), ws.numel()
-
-
 @_instrument("gemm", 1)
 def gemm(a: torch.Tensor, b: torch.Tensor, out: torch.Tensor, *, a_t=False, b_t=False, bias=None, residual=None,
          row_scale=None, rows_per_scale=0, act=UB_ACT_NONE, aux_in=None, aux_out=None, accumulate=False, split_k=1, tile_ctas=0,
-         max_ctas=0, ln_stats=None, ln_c=None, ln_eps=0.0, stats_out=None, colsum_out=None, group=None, stream_k=None, dot_out=None, dot_seq_len=0):
+         max_ctas=0, ln_stats=None, ln_c=None, ln_eps=0.0, stats_out=None, colsum_out=None, group=None, dot_out=None, dot_seq_len=0):
     """out[M,N] = epilogue(A[M,K] @ B[N,K]^T).  a_t / b_t: the operand is stored transposed ([K,M] / [K,N]).
     A and B are both bf16 or both fp16.  ln_stats / ln_c: LayerNorm of A's rows folded into the epilogue (see the header);
     stats_out: row (sum, sumsq) of an fp16-residual output, accumulated.  colsum_out (DGELU epilogue): fp32 [N], += column sums
@@ -101,9 +82,7 @@ def gemm(a: torch.Tensor, b: torch.Tensor, out: torch.Tensor, *, a_t=False, b_t=
     groups' outputs along M, K is the per-group contraction length and the operands are addressed with the group offsets.
     act=UB_ACT_DOT_AUX with aux_in, dot_out (fp32 [M // dot_seq_len, N // 64, dot_seq_len]) and dot_seq_len: besides C, the per-(row,
     64-column head) dot product of the bf16 output with aux_in (D = rowsum(dO o O) for the attention backward, from the GEMM that
-    produces dO).
-    stream_k: hand the library this stream's stream-K scratch, so that a partial last wave of tiles may be cut along K
-    (None = the UB_GEMM_SK environment default, off: measured slower on B200, see profiles/gemm_streamk_r02.md)."""
+    produces dO)."""
     ab = F16 if a.dtype == F16 else BF16
     pa, lda = _p2d(a, ab, "gemm A")
     pb, ldb = _p2d(b, ab, "gemm B")
@@ -172,10 +151,6 @@ def gemm(a: torch.Tensor, b: torch.Tensor, out: torch.Tensor, *, a_t=False, b_t=
         if act != UB_ACT_DOT_AUX or aux_in is None or dot_seq_len <= 0 or M % dot_seq_len or N % 64 or dot_out.numel() != M * (N // 64):
             raise _cabi.UBError("gemm: dot_out needs act=UB_ACT_DOT_AUX, aux_in, dot_seq_len dividing M and fp32 [M / S, N / 64, S]")
         ep.dot_out, ep.dot_seq_len = _p(dot_out, F32, "dot_out"), int(dot_seq_len)
-    if stream_k is None:
-        stream_k = _SK_DEFAULT
-    if stream_k and _SK_COMPILED and split_k == 1 and group is None and M > 256 and N > 128:
-        _sk_workspace(ep)
     check(lib.ub_gemm_bf16(pa, lda, int(a_t), pb, ldb, int(b_t), pc, ldc, M, N, K, C.byref(ep), split_k, _stream()), "ub_gemm_bf16")
     return out
 
