@@ -193,6 +193,19 @@ UB_API int ub_patchify_u8(const uint8_t* x, void* out, const float* mean3, const
  * B even, H and W multiples of 16, x 16-byte aligned; mean3 / std3 are HOST pointers to 3 floats. */
 UB_API int ub_patchify_mix_u8(const uint8_t* x, void* out, const float* mix, const float* mean3, const float* std3, int B, int T, int H,
                               int W, int tubelet, void* stream);
+/* the stage-2 training loader's spatial augmentation of decoded uint8 frames [B,T,H,W,3] (any H, W >= 1), fused into the normalising
+ * im2col of the augmented S x S clip (S a multiple of 16): rows [B*(T/tubelet)*(S/16)^2, 3*tubelet*256] as ub_patchify lays them out.
+ * draw: DEVICE int32 [B][10] = {i, j, h, w, flip, erase, top, left, eh, ew} per clip (unite_b200/augment.py; in range of H, W, S).
+ * Per clip: normalise as ub_patchify_u8, crop rows [i, i+h) and columns [j, j+w), resize to S x S as F.interpolate(mode="bilinear",
+ * align_corners=False), mirror the columns when flip != 0, then when erase != 0 fill [top, top+eh) x [left, left+ew) of every frame:
+ * erase_mode 0 with zeros; 1 ('rand') with one standard normal per (clip, frame, channel); 2 ('pixel') with one per element.  The
+ * normals are noise[n] when noise != NULL (fp32 [B,T,3] or [B,T,3,S,S]), else Philox4x32-10 normals keyed by seed at the DEVICE
+ * counter rng[0] (uint64 [2], {counter, 0}): the launch advances it, so a captured launch draws fresh noise on every replay.
+ * mix: NULL, or ub_patchify_mix's DEVICE draw, applied to the augmented clips as there (B even).  x is not written; mean3 / std3 are
+ * HOST pointers to 3 floats. */
+UB_API int ub_patchify_aug_u8(const uint8_t* x, void* out, const int32_t* draw, const float* mix, int erase_mode, const float* noise,
+                              uint64_t seed, uint64_t* rng, const float* mean3, const float* std3, int B, int T, int H, int W, int S,
+                              int tubelet, void* stream);
 /* resize + patchify for the teacher: fp32 clip [B,3,T,H,W] (x_is_u8 = 0) or decoded uint8 frames [B,T,H,W,3] (x_is_u8 = 1,
  * normalised with the HOST mean3 / std3 as ub_patchify_u8 does, before the resize) -> bicubic resize of every (c, t) plane to
  * R x R (torch interpolate mode="bicubic", align_corners=False, antialias=False; no resize when R == H == W) -> bf16 im2col rows

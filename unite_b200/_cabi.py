@@ -87,7 +87,9 @@ SIGNATURES = {
     "ub_patchify_mix": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "ub_patchify_u8": (C.c_int, [_P, _P, C.POINTER(C.c_float), C.POINTER(C.c_float), _I, _I, _I, _I, _I, _P]),
     "ub_patchify_mix_u8": (C.c_int, [_P, _P, _P, C.POINTER(C.c_float), C.POINTER(C.c_float), _I, _I, _I, _I, _I, _P]),
-    "ub_resize_patchify": (C.c_int, [_P, _I, C.POINTER(C.c_float), C.POINTER(C.c_float), _P, _L, _I, _I, _I, _I, _I, _I, _I, _P]),
+    "ub_patchify_aug_u8": (C.c_int, [_P, _P, _P, _P, _I, _P, C.c_uint64, _P, C.POINTER(C.c_float), C.POINTER(C.c_float), _I, _I, _I, _I,
+                                     _I, _I, _P]),
+    "ub_resize_patchify":(C.c_int, [_P, _I, C.POINTER(C.c_float), C.POINTER(C.c_float), _P, _L, _I, _I, _I, _I, _I, _I, _I, _P]),
     "ub_mask_select": (C.c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "ub_gather_rows": (C.c_int, [_P, _P, _P, _L, _L, _I, _L, _P]),
     "ub_colsum_bf16": (C.c_int, [_P, _L, _P, _I, _I, _I, _I, _P]),

@@ -53,6 +53,22 @@ UB_DEVINL float2 unpack_bf16x2(uint32_t u) {
   __nv_bfloat162 v = *reinterpret_cast<__nv_bfloat162*>(&u);
   return __bfloat1622float2(v);
 }
+// Philox4x32-10 (Salmon et al. SC'11), the counter-based generator of the device-side draws (rng.cu's DropPath factors, tokens.cu's
+// random-erasing noise); oracle/philox.py restates it on the host.
+UB_DEVINL void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1, uint32_t out[4]) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
+    const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
+    c0 = hi1 ^ c1 ^ k0;
+    c1 = lo1;
+    c2 = hi0 ^ c3 ^ k1;
+    c3 = lo0;
+    k0 += 0x9E3779B9u;
+    k1 += 0xBB67AE85u;
+  }
+  out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
+}
 UB_DEVINL float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

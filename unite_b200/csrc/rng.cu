@@ -14,21 +14,6 @@
 
 namespace ub {
 
-UB_DEVINL void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1, uint32_t out[4]) {
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
-    const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
-    c0 = hi1 ^ c1 ^ k0;
-    c1 = lo1;
-    c2 = hi0 ^ c3 ^ k1;
-    c3 = lo0;
-    k0 += 0x9E3779B9u;
-    k1 += 0xBB67AE85u;
-  }
-  out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
-}
-
 // out[(l*2 + branch)*B + b] = floor(keep_l + u) / keep_l; one block, every thread reads the step before thread 0 bumps it
 __global__ void __launch_bounds__(256) drop_path_draw_kernel(const float* __restrict__ rates, float* __restrict__ out, int depth, int B,
                                                              uint32_t seed_lo, uint32_t seed_hi, unsigned long long* __restrict__ step) {

@@ -4,6 +4,7 @@
 //                    clip.py:123-128,146 (teacher conv1), modeling_finetune.py:165-174 (student PatchEmbed.proj)
 //   ub_patchify_mix  the same rows of the batch-mode mixup / cutmix of the clip (stage-2 mixup_fn), x left untouched
 //   ub_patchify_u8 / ub_patchify_mix_u8   the same two from decoded uint8 frames, normalised on the way
+//   ub_patchify_aug_u8  the rows of the stage-2 training crop, flip and random erasing of decoded uint8 frames (mixed optionally)
 //   ub_mask_select   attention-guided visible-token selection, bit-exact
 //                    run_stage1.py:379-387 (multinomial == top-N_vis of attn/q, q ~ Exp(1) supplied by the caller)
 //                    utils.py:89-120 get_greedy_masks (k committee members take ranks i, i+k, ...; q == NULL)
@@ -245,6 +246,209 @@ __global__ void __launch_bounds__(256) patchify_mix_u8_kernel(const uint8_t* __r
       stg_v4(da + co + 8, make_uint4(oa[4], oa[5], oa[6], oa[7]));
       stg_v4(db + co, make_uint4(om[0], om[1], om[2], om[3]));
       stg_v4(db + co + 8, make_uint4(om[4], om[5], om[6], om[7]));
+    }
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
+// patchify_aug_u8: the stage-2 training loader's spatial augmentation of decoded uint8 frames [B,T,H,W,3], fused into the
+// normalising im2col of the augmented S x S clip (kinetics_sparse.py _aug_frame after RandAugment: ToTensor + tensor_normalize,
+// spatial_sampling's random_resized_crop + horizontal flip, RandomErasing(cube=True) on every frame), then optionally the batch
+// mixup / cutmix of ub_patchify_mix_u8 (the reference's mixup_fn runs after its loader).
+//   draw (device int32 [B][10]) = {i, j, h, w, flip, erase, top, left, eh, ew} per clip, drawn by unite_b200/augment.py.
+//   crop + resize: F.interpolate(x[..., i:i+h, j:j+w], (S, S), mode="bilinear", align_corners=False) as ATen's CUDA kernel computes
+//     it: src = (h / S) * (o + 0.5) - 0.5 clamped at 0, i0 = (int)src, i1 = i0 + (i0 < h - 1), l1 = src - i0, l0 = 1 - l1,
+//     v = l0y * (l0x * p00 + l1x * p01) + l1y * (l0x * p10 + l1x * p11).  Each tap is normalised through the per-CTA byte table
+//     of ub_patchify_mix_u8 first; the weights sum to one, so this is the reference's normalise-then-resize up to fp32 rounding.
+//   flip: output column o is resized column S-1-o.  erase: inside [top, top+eh) x [left, left+ew) of every frame the value is 0
+//     (mode 0, 'const'), one normal per (clip, frame, channel) (mode 1, 'rand') or per element (mode 2, 'pixel'): noise[n] when
+//     the caller supplies them, else Philox normals keyed by the seed at the device counter rng[0], which the launch advances.
+// One thread = one (token, kt, kh) run of 16 output pixels in all three channels, of clips b and B-1-b under a mix, in two halves of
+// 8 (one 16-byte store per channel).  Reads are byte gathers through L1 (four taps x RGB a pixel); every output byte is written
+// once.  128-thread CTAs: 119 / 197 registers (unmixed / mixed, no spills) leave 4 / 2 CTAs per SM.
+// ------------------------------------------------------------------------------------------------
+struct AugClip {
+  int i, j, h, w, flip, erase, top, left, eh, ew;
+  float sy, sx;
+};
+
+UB_DEVINL AugClip aug_clip(const int* __restrict__ draw, int b, int S) {
+  const int* d = draw + 10 * b;
+  AugClip a;
+  a.i = __ldg(d); a.j = __ldg(d + 1); a.h = __ldg(d + 2); a.w = __ldg(d + 3); a.flip = __ldg(d + 4);
+  a.erase = __ldg(d + 5); a.top = __ldg(d + 6); a.left = __ldg(d + 7); a.eh = __ldg(d + 8); a.ew = __ldg(d + 9);
+  a.sy = __fdiv_rn((float)a.h, (float)S);                   // ATen area_pixel_compute_scale (align_corners=False)
+  a.sx = __fdiv_rn((float)a.w, (float)S);
+  return a;
+}
+
+// bilinear taps of output coordinate o over n source pixels: first tap, offset of the second (0 at the last pixel), weights.
+// The source index is one FMA, as nvcc contracts ATen's `scale * (dst + 0.5) - 0.5`.
+UB_DEVINL void bilinear_taps(int o, float scale, int n, int& i0, int& step, float& l0, float& l1) {
+  float src = fmaf(scale, (float)o + 0.5f, -0.5f);
+  src = src < 0.f ? 0.f : src;
+  i0 = (int)src;
+  step = i0 < n - 1 ? 1 : 0;
+  l1 = __fsub_rn(src, (float)i0);
+  l0 = __fsub_rn(1.f, l1);
+}
+
+// standard normal number n of a Philox stream: Box-Muller on the first two words of block (n / 2, stream, s); even n take the
+// cosine, odd n the sine.  The stream word keeps the erasing noise apart from the DropPath draws (rng.cu, word 0).
+UB_DEVINL float philox_normal(unsigned long long n, uint32_t stream, unsigned long long s, uint32_t k0, uint32_t k1) {
+  uint32_t r[4];
+  philox4x32_10((uint32_t)(n >> 1), (uint32_t)(n >> 33) ^ stream, (uint32_t)s, (uint32_t)(s >> 32), k0, k1, r);
+  const float u1 = ((float)(r[0] >> 8) + 1.0f) * 5.9604644775390625e-8f;      // (0, 1]
+  const float u2 = (float)(r[1] >> 8) * 5.9604644775390625e-8f;                // [0, 1)
+  const float rad = sqrtf(-2.0f * logf(u1));
+  float sn, cs;
+  sincospif(2.0f * u2, &sn, &cs);
+  return (n & 1ull) ? rad * sn : rad * cs;
+}
+
+struct AugNoise {
+  int mode;                      // 0 const, 1 rand, 2 pixel
+  const float* noise;            // caller-supplied: [B,T,3] (rand) or [B,T,3,S,S] (pixel); NULL: Philox
+  unsigned long long s;
+  uint32_t k0, k1;
+};
+
+// the erased value of channel c at (oy, ox) of frame bt = b * T + t
+UB_DEVINL float erase_value(const AugNoise& z, long bt, int c, int oy, int ox, int S) {
+  if (z.mode == 0) return 0.f;
+  const long n = z.mode == 1 ? bt * 3 + c : ((bt * 3 + c) * S + oy) * (long)S + ox;
+  if (z.noise) return __ldg(z.noise + n);
+  return philox_normal((unsigned long long)n, z.mode == 1 ? 0x80000000u : 0x40000000u, z.s, z.k0, z.k1);
+}
+
+// the two source rows (as THWC byte pointers at the crop's first column) and weights of output row oy of clip b, frame t
+struct AugRow {
+  const uint8_t* r0;
+  const uint8_t* r1;
+  float l0, l1;
+  bool erase_row;
+};
+
+UB_DEVINL AugRow aug_row(const uint8_t* __restrict__ x, const AugClip& a, int b, int t, int oy, int T, int H, int W) {
+  AugRow r;
+  int y0, dy;
+  bilinear_taps(oy, a.sy, a.h, y0, dy, r.l0, r.l1);
+  r.r0 = x + ((((long)b * T + t) * H + a.i + y0) * W + a.j) * 3;
+  r.r1 = r.r0 + (long)dy * W * 3;
+  r.erase_row = a.erase && oy >= a.top && oy < a.top + a.eh;
+  return r;
+}
+
+// the three channels of output pixel (oy, ox) of the augmented clip, erasing included
+UB_DEVINL void aug_pixel(const float (*lut)[256], const AugClip& a, const AugRow& r, const AugNoise& z, long bt, int oy, int ox, int S,
+                         float v[3]) {
+  if (r.erase_row && ox >= a.left && ox < a.left + a.ew) {
+#pragma unroll
+    for (int c = 0; c < 3; ++c) v[c] = erase_value(z, bt, c, oy, ox, S);
+    return;
+  }
+  int x0, dx;
+  float l0, l1;
+  bilinear_taps(a.flip ? S - 1 - ox : ox, a.sx, a.w, x0, dx, l0, l1);
+  const uint8_t* p00 = r.r0 + 3 * x0;
+  const uint8_t* p10 = r.r1 + 3 * x0;
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    const float top = l0 * lut[c][__ldg(p00 + c)] + l1 * lut[c][__ldg(p00 + 3 * dx + c)];
+    const float bot = l0 * lut[c][__ldg(p10 + c)] + l1 * lut[c][__ldg(p10 + 3 * dx + c)];
+    v[c] = r.l0 * top + r.l1 * bot;
+  }
+}
+
+// 8 consecutive output pixels from column ox0 of output row oy, clip b, frame t: v[c][k]
+UB_DEVINL void aug_pixels8(const uint8_t* __restrict__ x, const float (*lut)[256], const int* __restrict__ draw, const AugNoise& z, int b,
+                           int t, int oy, int ox0, int T, int H, int W, int S, float v[3][8]) {
+  const AugClip a = aug_clip(draw, b, S);
+  const AugRow r = aug_row(x, a, b, t, oy, T, H, W);
+#pragma unroll
+  for (int k = 0; k < 8; ++k) {
+    float p[3];
+    aug_pixel(lut, a, r, z, (long)b * T + t, oy, ox0 + k, S, p);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) v[c][k] = p[c];
+  }
+}
+
+template <bool MIX>
+__global__ void __launch_bounds__(128) patchify_aug_u8_kernel(const uint8_t* __restrict__ x, bf16* __restrict__ out,
+                                                              const int* __restrict__ draw, const float* __restrict__ mix, int mode,
+                                                              const float* __restrict__ noise, uint32_t seed_lo, uint32_t seed_hi,
+                                                              unsigned long long* __restrict__ rng, float m0, float m1, float m2,
+                                                              float s0, float s1, float s2, int B, int T, int H, int W, int S, int tub,
+                                                              long total_runs) {
+  __shared__ float lut[3][256];
+  for (int i = threadIdx.x; i < 3 * 256; i += blockDim.x) {
+    const int c = i / 256;
+    lut[c][i % 256] = u8_norm((uint8_t)(i % 256), c == 0 ? m0 : (c == 1 ? m1 : m2), c == 0 ? s0 : (c == 1 ? s1 : s2));
+  }
+  AugNoise z;
+  z.mode = mode;
+  z.noise = noise;
+  z.s = rng ? rng[0] : 0ull;                                  // every CTA reads the counter before it counts itself done below
+  z.k0 = seed_lo;
+  z.k1 = seed_hi;
+  __syncthreads();
+  bool apply = false, cut = false;
+  float lam = 1.f, lam1 = 0.f;
+  int t0 = 0, t1 = 0, h0 = 0, h1 = 0, w0 = 0, w1 = 0;
+  if (MIX) {
+    apply = mix[0] != 0.f; cut = mix[3] != 0.f; lam = mix[1]; lam1 = mix[2];
+    t0 = (int)mix[4]; t1 = (int)mix[5]; h0 = (int)mix[6]; h1 = (int)mix[7]; w0 = (int)mix[8]; w1 = (int)mix[9];
+  }
+  const long clip_rows = (long)(T / tub) * (S / 16) * (S / 16) * (3 * tub * 256);
+  for (long id = (long)blockIdx.x * blockDim.x + threadIdx.x; id < total_runs; id += (long)gridDim.x * blockDim.x) {
+    const U8Run r = u8_run(id, T, S, S, tub);                 // output run (under a mix: of the first half of the batch)
+    const int bm = B - 1 - r.b;
+    const bool in_box = MIX && apply && cut && r.t >= t0 && r.t < t1 && r.h >= h0 && r.h < h1;
+    bf16* da = out + u8_dst(r, tub);
+    bf16* db = da + (long)(bm - r.b) * clip_rows;
+#pragma unroll
+    for (int half = 0; half < 2; ++half) {                   // 8 pixels = one 16-byte store per channel and clip
+      const int ox0 = r.w + 8 * half;
+      float a[3][8], m[3][8];
+      aug_pixels8(x, lut, draw, z, r.b, r.t, r.h, ox0, T, H, W, S, a);
+      if (MIX) {
+        aug_pixels8(x, lut, draw, z, bm, r.t, r.h, ox0, T, H, W, S, m);
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {
+#pragma unroll
+          for (int c = 0; c < 3; ++c) {
+            const float va = a[c][k], vm = m[c][k];
+            if (in_box) {
+              if (ox0 + k >= w0 && ox0 + k < w1) { a[c][k] = vm; m[c][k] = va; }
+            } else if (apply && !cut) {
+              a[c][k] = __fadd_rn(__fmul_rn(va, lam), __fmul_rn(vm, lam1));
+              m[c][k] = __fadd_rn(__fmul_rn(vm, lam), __fmul_rn(va, lam1));
+            }
+          }
+        }
+      }
+#pragma unroll
+      for (int c = 0; c < 3; ++c) {
+        const long co = (long)c * (tub * 256) + 8 * half;
+        stg_v4(da + co, make_uint4(pack_bf16x2(a[c][0], a[c][1]), pack_bf16x2(a[c][2], a[c][3]), pack_bf16x2(a[c][4], a[c][5]),
+                                   pack_bf16x2(a[c][6], a[c][7])));
+        if (MIX)
+          stg_v4(db + co, make_uint4(pack_bf16x2(m[c][0], m[c][1]), pack_bf16x2(m[c][2], m[c][3]), pack_bf16x2(m[c][4], m[c][5]),
+                                     pack_bf16x2(m[c][6], m[c][7])));
+      }
+    }
+  }
+  // advance the noise counter once every CTA has read it: the last CTA to finish bumps it and re-arms the arrival count, so the
+  // next launch (or graph replay) draws fresh noise
+  if (rng) {
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      __threadfence();
+      if (atomicAdd(rng + 1, 1ull) == (unsigned long long)gridDim.x - 1ull) {
+        rng[1] = 0ull;
+        rng[0] = z.s + 1ull;
+      }
     }
   }
 }
@@ -576,6 +780,25 @@ extern "C" int ub_patchify_mix_u8(const uint8_t* x, void* out, const float* mix,
   UB_LAUNCH(patchify_mix_u8_kernel, flat_grid(runs, 256), 256, 0, (cudaStream_t)stream, x, (bf16*)out, mix, mean3[0], mean3[1], mean3[2],
             std3[0], std3[1], std3[2], B, T, H, W, tubelet, runs);
   return check_launch("patchify_mix_u8_kernel");
+}
+
+extern "C" int ub_patchify_aug_u8(const uint8_t* x, void* out, const int32_t* draw, const float* mix, int erase_mode, const float* noise,
+                                  uint64_t seed, uint64_t* rng, const float* mean3, const float* std3, int B, int T, int H, int W, int S,
+                                  int tubelet, void* stream) {
+  UB_REQUIRE(x && out && draw && mean3 && std3, "patchify_aug_u8: null pointer");
+  UB_REQUIRE(B > 0 && T > 0 && tubelet > 0 && T % tubelet == 0 && H > 0 && W > 0, "patchify_aug_u8: bad shape B=%d T=%d H=%d W=%d tub=%d", B,
+             T, H, W, tubelet);
+  UB_REQUIRE(S > 0 && S % 16 == 0, "patchify_aug_u8: the crop size %d must be a multiple of the 16-pixel patch", S);
+  UB_REQUIRE(!mix || B % 2 == 0, "patchify_aug_u8: the batch must be even to pair clip b with clip B-1-b (B=%d)", B);
+  UB_REQUIRE(erase_mode >= 0 && erase_mode <= 2, "patchify_aug_u8: erase mode %d is not 0 (const), 1 (rand) or 2 (pixel)", erase_mode);
+  UB_REQUIRE(erase_mode == 0 || noise || rng, "patchify_aug_u8: 'rand' / 'pixel' erasing needs the noise or the generator's counter");
+  UB_REQUIRE(std3[0] != 0.f && std3[1] != 0.f && std3[2] != 0.f, "patchify_aug_u8: zero std");
+  const long runs = (long)(mix ? B / 2 : B) * (T / tubelet) * (S / 16) * (S / 16) * tubelet * 16;
+  unsigned long long* counter = (erase_mode != 0 && !noise) ? (unsigned long long*)rng : nullptr;
+  auto kern = mix ? patchify_aug_u8_kernel<true> : patchify_aug_u8_kernel<false>;
+  UB_LAUNCH(kern, flat_grid(runs, 128), 128, 0, (cudaStream_t)stream, x, (bf16*)out, draw, mix, erase_mode, noise, (uint32_t)seed,
+            (uint32_t)(seed >> 32), counter, mean3[0], mean3[1], mean3[2], std3[0], std3[1], std3[2], B, T, H, W, S, tubelet, runs);
+  return check_launch("patchify_aug_u8_kernel");
 }
 
 extern "C" int ub_resize_patchify(const void* x, int x_is_u8, const float* mean3, const float* std3, void* out, int64_t ld_out, int B,

@@ -10,6 +10,9 @@ on the device inside the im2col (ub_patchify_mix), so the caller's clip is never
 one in finetune_core.py; gradients accumulate in the parameter arena across micro-steps like `.grad` does in torch.
 A batch may carry decoded uint8 frames [B,T,H,W,3] instead of the fp32 clip: they are normalised on the device inside the im2col
 (ub_patchify_u8, or ub_patchify_mix_u8 when mixed), a quarter of the host-to-device copy.
+With `spatial_aug` (augment.SpatialAugment) the uint8 frames are the loader's output after RandAugment: each clip's training crop,
+flip and random erasing are drawn on the host as the reference's loader draws them and applied on the device inside the im2col
+(ub_patchify_aug_u8), before the mixup of the augmented clips.
     model_ema.update(model)                                   engine_for_finetuning.py:126-127 (after every optimizer update)
 With `model_ema` (ema.ModelEma or timm's ModelEma) the EMA arena is updated by one fused kernel (ub_ema_update) right after the
 optimizer, inside the CUDA graph of the step.
@@ -21,6 +24,7 @@ import torch
 
 from . import ops
 from .ema import resolve_model_ema
+from .augment import AugBuffer
 from .engine import (FusedAdamW, GraphReplay, StepEngine, apply_schedule, exit_if_not_finite, require_fused_optimizer,
                      schedule_stats)
 from .mixup import NO_MIX, MixBuffer, draw, resolve_loss
@@ -44,17 +48,18 @@ def _default_optimizer(net):
     return opt
 
 
-def finetune_step(model, samples, targets, loss_acc, scale=1.0, grad_sync=None, mix=None):
+def finetune_step(model, samples, targets, loss_acc, scale=1.0, grad_sync=None, mix=None, aug=None):
     """One micro-step: forward, CE, backward.  Adds scale * mean CE to loss_acc (fp32 [1]).  Returns logits.
     grad_sync: pass the model's GradSync on the micro-step that is followed by the optimizer step — its range all-reduces then
     overlap this backward.
     mix: None (plain CE), or a mixup.MixBuffer holding this step's draw on the device: the clip is mixed on its way into the
-    im2col (mix.clip, None for label smoothing alone) and the loss is the soft-target CE of the mixed, smoothed target."""
-    ops.clip_shape(samples, paired=mix is not None and mix.clip is not None)
+    im2col (mix.clip, None for label smoothing alone) and the loss is the soft-target CE of the mixed, smoothed target.
+    aug: None, or an augment.AugBuffer holding this batch's crop / flip / erasing draws for the uint8 frames `samples`."""
+    ops.clip_shape(samples, paired=mix is not None and mix.clip is not None, crop_size=None if aug is None else aug.aug.crop_size)
     net = model.module if hasattr(model, "module") else model
     core = net.core()
     dp = core.drop_path.draw(samples.shape[0]) if net.training else None       # modeling_finetune.py:42-50 (device-side draws)
-    logits, state = core.run_forward(samples, dp, save=True, mix=None if mix is None else mix.clip)
+    logits, state = core.run_forward(samples, dp, save=True, mix=None if mix is None else mix.clip, aug=aug)
     B = logits.shape[0]
     dlogits = torch.empty_like(logits)
     if mix is None:
@@ -93,11 +98,14 @@ class Stage2Engine(StepEngine):
         self.logits = None
         self._mix_bufs = {}                                 # loss kind -> MixBuffer (fixed addresses the graphs read)
         self._mix = None                                    # the buffer of the current step, None for plain CE
+        self._aug_bufs = {}                                 # (batch, SpatialAugment) -> AugBuffer (fixed addresses the graphs read)
+        self._aug = None
 
     def _body(self, samples, targets):
         self.optimizer.zero_grad()
         self.loss.zero_()
-        logits = finetune_step(self.model, samples, targets, self.loss, scale=1.0, grad_sync=self._backward_hook(), mix=self._mix)
+        logits = finetune_step(self.model, samples, targets, self.loss, scale=1.0, grad_sync=self._backward_hook(), mix=self._mix,
+                               aug=self._aug)
         self._update()
         if self.ema is not None:
             self.ema.update(self.model)
@@ -105,16 +113,25 @@ class Stage2Engine(StepEngine):
                                  self.optimizer.grad_norm(self.grad_scale)])
         self.logits = logits
 
-    def step(self, samples, targets, private_inputs=False, mix=None, smoothing=None):
+    def step(self, samples, targets, private_inputs=False, mix=None, smoothing=None, aug=None):
         """samples fp32 [B,3,T,H,W] or decoded uint8 frames [B,T,H,W,3] (normalised on the device), targets integer [B], both on
         the device.  Returns the device loss tensor [1].
         private_inputs: the batch lives in fresh tensors every step (a loader), so the graph keeps its own static inputs.
         smoothing None: plain CE.  smoothing s: soft-target CE with label smoothing s, and with mix (a mixup.MixDraw, NO_MIX for a
         batch the draw left unmixed) the clip is mixed as drawn.  The draw is uploaded to device memory before the step, so every
-        replay of the one graph per loss kind reads its own draw."""
+        replay of the one graph per loss kind reads its own draw.
+        aug: None, or an augment.AugDraw of these uint8 frames (SpatialAugment.draw): the clips are cropped, flipped and erased as
+        drawn on the device; the draws are uploaded like the mixup draw."""
         if mix is not None and smoothing is None:
             raise ValueError("Stage2Engine.step: a mixup draw needs the soft-target loss (pass smoothing=)")
-        ops.clip_shape(samples, paired=mix is not None)
+        ops.clip_shape(samples, paired=mix is not None, crop_size=None if aug is None else aug.aug.crop_size)
+        self._aug = None
+        if aug is not None:
+            akey = (samples.shape[0], aug.aug)
+            if akey not in self._aug_bufs:
+                self._aug_bufs[akey] = AugBuffer(aug.aug, samples.shape[0], self.core.arena.device)
+            self._aug = self._aug_bufs[akey]
+            self._aug.upload(aug)
         self.optimizer.prepare_step(grad_scale=self.grad_scale)
         kind = "ce" if smoothing is None else ("mix" if mix is not None else "smooth")
         self._mix = None
@@ -129,6 +146,8 @@ class Stage2Engine(StepEngine):
         key = (tuple(samples.shape), samples.dtype, targets.dtype, float(self.max_norm or 0.0), bool(self.net.training), kind)
         if self.ema is not None:
             key += (("ema", self.ema.decay),)               # the decay is a launch argument recorded in the graph
+        if aug is not None:
+            key += (("aug", aug.aug),)                      # its mode, crop size, mean, std and seed are launch arguments too
         self.logits = self.graphs.run(key, (samples, targets), self._body, state_fn=lambda: self.logits, private=private_inputs)
         return self.loss
 
@@ -145,11 +164,14 @@ def _stage2_engine(model, net, optimizer, gs, model_ema=None):
 def train_one_epoch(model: torch.nn.Module, criterion=None, data_loader: Iterable = (), optimizer=None, device=None, epoch: int = 0,
                     loss_scaler=None, max_norm: float = 0, model_ema=None, mixup_fn=None, log_writer=None, start_steps=None,
                     lr_schedule_values=None, wd_schedule_values=None, num_training_steps_per_epoch=None, update_freq=None,
-                    num_epochs=None, train_head_only=False, wandb_run=None, args=None):
+                    num_epochs=None, train_head_only=False, wandb_run=None, args=None, spatial_aug=None):
     """mixup_fn: a mixup.Mixup (or the reference's timm Mixup) in batch mode, drawn once per loader batch; criterion: see
     mixup.resolve_loss.  With mixup_fn the returned dict has no class_acc (the reference logs None there).
     model_ema: an ema.ModelEma (or the reference's timm ModelEma) of this model, updated once per optimizer update (see
-    ema.resolve_model_ema for what is refused)."""
+    ema.resolve_model_ema for what is refused).
+    spatial_aug: an augment.SpatialAugment: the loader's batches are decoded uint8 frames [B,T,H,W,3] of any size, after
+    RandAugment; every clip is cropped to crop_size, flipped and erased on the device as drawn here per batch (before the mixup
+    draw, whose cutmix box is drawn on the augmented clip's shape).  fp32 batches are refused."""
     ema = resolve_model_ema(model_ema, model)
     if train_head_only:
         raise NotImplementedError("head-only training is not implemented in the fused stage-2 loop")
@@ -166,8 +188,10 @@ def train_one_epoch(model: torch.nn.Module, criterion=None, data_loader: Iterabl
     gs = getattr(model, "grad_sync", None)
     if update_freq == 1:
         return _train_one_epoch_graphed(model, net, data_loader, optimizer, gs, max_norm, start_steps, lr_schedule_values,
-                                        wd_schedule_values, num_training_steps_per_epoch, mixup_fn, smoothing, model_ema)
+                                        wd_schedule_values, num_training_steps_per_epoch, mixup_fn, smoothing, model_ema, spatial_aug)
     mix = None if smoothing is None else MixBuffer(dev, mix_clips=mixup_fn is not None)
+    crop = None if spatial_aug is None else spatial_aug.crop_size
+    aug_bufs = {}                                                                  # batch size -> AugBuffer
     loss_sum = torch.zeros(1, device=dev)
     loss_acc = torch.zeros(1, device=dev)
     correct = torch.zeros(1, device=dev)
@@ -183,14 +207,21 @@ def train_one_epoch(model: torch.nn.Module, criterion=None, data_loader: Iterabl
             continue                                                               # engine_for_finetuning.py:71-72
         if data_iter_step % update_freq == 0:                                      # engine_for_finetuning.py:76-81
             apply_schedule(optimizer, start_steps + step, lr_schedule_values, wd_schedule_values)
+        shape = ops.clip_shape(samples, crop_size=crop)
+        aug = None
+        if spatial_aug is not None:
+            if samples.shape[0] not in aug_bufs:
+                aug_bufs[samples.shape[0]] = AugBuffer(spatial_aug, samples.shape[0], dev)
+            aug = aug_bufs[samples.shape[0]]
+            aug.upload(spatial_aug.draw(samples.shape))
         if mix is not None:
-            mix.upload((draw(mixup_fn, ops.clip_shape(samples)) if mixup_fn is not None else NO_MIX).packed(smoothing, core.C))
+            mix.upload((draw(mixup_fn, shape) if mixup_fn is not None else NO_MIX).packed(smoothing, core.C))
         samples = samples.to(dev, non_blocking=True)
         targets = targets.to(dev, non_blocking=True)
         loss_acc.zero_()
         last_micro = (data_iter_step + 1) % update_freq == 0
         logits = finetune_step(model, samples, targets, loss_acc, scale=1.0 / update_freq, grad_sync=gs if last_micro else None,
-                               mix=mix)
+                               mix=mix, aug=aug)
         loss_sum += loss_acc * update_freq
         correct += (logits.argmax(-1) == targets).sum()
         seen += samples.shape[0]
@@ -213,7 +244,7 @@ def train_one_epoch(model: torch.nn.Module, criterion=None, data_loader: Iterabl
 
 
 def _train_one_epoch_graphed(model, net, data_loader, optimizer, gs, max_norm, start_steps, lr_schedule_values, wd_schedule_values,
-                             num_training_steps_per_epoch, mixup_fn=None, smoothing=None, model_ema=None):
+                             num_training_steps_per_epoch, mixup_fn=None, smoothing=None, model_ema=None, spatial_aug=None):
     """update_freq == 1 (the shipped stage-2 recipe): every loader batch is one whole update, run through Stage2Engine (CUDA-graph
     replay).  Same schedule handling and return dict as the general loop above."""
     eng = _stage2_engine(model, net, optimizer, gs, model_ema)
@@ -225,9 +256,11 @@ def _train_one_epoch_graphed(model, net, data_loader, optimizer, gs, max_norm, s
         if num_training_steps_per_epoch is not None and data_iter_step >= num_training_steps_per_epoch:
             continue                                                               # engine_for_finetuning.py:71-72
         apply_schedule(optimizer, start_steps + data_iter_step, lr_schedule_values, wd_schedule_values)   # :76-81
-        mix = draw(mixup_fn, ops.clip_shape(batch[0])) if mixup_fn is not None else None
+        shape = ops.clip_shape(batch[0], crop_size=None if spatial_aug is None else spatial_aug.crop_size)
+        aug = spatial_aug.draw(batch[0].shape) if spatial_aug is not None else None
+        mix = draw(mixup_fn, shape) if mixup_fn is not None else None
         eng.step(batch[0].to(dev, non_blocking=True), batch[1].to(dev, non_blocking=True), private_inputs=True, mix=mix,
-                 smoothing=smoothing)
+                 smoothing=smoothing, aug=aug)
         seen += batch[0].shape[0]
         n += 1
     loss_sum, correct, gn_sum = eng.stats.tolist()

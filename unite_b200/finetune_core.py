@@ -53,15 +53,31 @@ class FinetuneCore:
             self._pos_full[B] = self.pos.repeat(B, 1).contiguous()
         return self._pos_full[B]
 
-    def run_forward(self, x, dp, save, mix=None):
+    def run_forward(self, x, dp, save, mix=None, aug=None):
         """x: the fp32 clip [B,3,T,H,W], or decoded uint8 frames [B,T,H,W,3], normalised on the device (ops.patchify_u8).
         mix: None, or the device draw of batch-mode mixup / cutmix (mixup.MixBuffer.clip): the trunk then sees the mixed clip,
-        mixed on the way into the im2col (x itself is not written)."""
+        mixed on the way into the im2col (x itself is not written).
+        aug: None, or an augment.AugBuffer holding this batch's crop / flip / erasing draws: uint8 frames of any size are augmented
+        to the crop_size x crop_size clip on the way into the im2col (ops.patchify_aug_u8), then mixed by `mix`."""
         u8 = x.dtype == U8
+        if aug is not None:
+            S = aug.aug.crop_size
+            if not u8 or x.dim() != 5:
+                raise ValueError("run_forward: the spatial augmentation takes decoded uint8 frames [B,T,H,W,3]")
+            n = (x.shape[1] // self.tubelet) * (S // 16) ** 2
+            if n != self.N:
+                raise ValueError(f"run_forward: a {S}x{S} crop of {x.shape[1]} frames gives {n} tokens, the model has {self.N} "
+                                 "(num_patches follows the crop size)")
+            if aug.batch != x.shape[0]:
+                raise ValueError(f"run_forward: draws for {aug.batch} clips, batch of {x.shape[0]}")
         self.sync_shadow()
         B, dev, a = x.shape[0], x.device, self.arena
         patches = torch.empty(B * self.N, 3 * self.tubelet * 256, device=dev, dtype=BF16)
-        if u8 and mix is None:
+        if aug is not None:
+            g = aug.aug
+            ops.patchify_aug_u8(x, patches, aug.draw, g.crop_size, self.tubelet, g.erase_mode, mix=mix, rng=aug.rng, seed=g.seed,
+                                mean=g.mean, std=g.std)
+        elif u8 and mix is None:
             ops.patchify_u8(x, patches, self.tubelet)
         elif u8:
             ops.patchify_mix_u8(x, patches, mix, self.tubelet)

@@ -18,7 +18,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 __all__ = ["Mixup", "SoftTargetCrossEntropy", "LabelSmoothingCrossEntropy", "MixDraw", "draw", "clip_box", "cutmix_bbox_and_lam",
-           "rand_bbox", "rand_bbox_minmax", "resolve_loss", "MixBuffer"]
+           "rand_bbox", "rand_bbox_minmax", "resolve_loss", "MixBuffer", "PinnedUpload"]
 
 
 # ---- timm 0.4.12 timm/data/mixup.py: box draws ------------------------------------------------------------------------------------
@@ -213,18 +213,16 @@ def resolve_loss(criterion, mixup_fn) -> Optional[float]:
                               f"(LabelSmoothingCrossEntropy(s), CrossEntropyLoss(label_smoothing=s)), got {name}")
 
 
-class MixBuffer:
-    """Device copy of one step's packed draw (MixDraw.packed): `clip` feeds ub_patchify_mix, `target` ub_soft_target_ce.  Each
-    upload is one async copy from a ring of pinned slots, as FusedAdamW.prepare_step uploads its scalars: a slot is rewritten
-    only after the copy that last read it has executed, since a host that queues graph replays can be many steps ahead of the
-    device.  Both views keep their addresses, so a captured step reads each fresh draw on replay.  mix_clips=False (label
-    smoothing without mixup_fn): `clip` is None and the clip is patchified as it comes."""
+class PinnedUpload:
+    """A fixed-address device tensor rewritten from the host once per step.  Each upload is one async copy from a ring of pinned
+    slots, as FusedAdamW.prepare_step uploads its scalars: a slot is rewritten only after the copy that last read it has executed,
+    since a host that queues graph replays can be many steps ahead of the device.  `dev` keeps its address, so a captured step
+    reads each fresh upload on replay."""
     _RING = 8
 
-    def __init__(self, device, mix_clips: bool = True):
-        self.dev = torch.zeros(16, device=device, dtype=torch.float32)
-        self.clip, self.target = (self.dev[:10] if mix_clips else None), self.dev[10:13]
-        self._pin = [torch.zeros(16, dtype=torch.float32).pin_memory() for _ in range(self._RING)]
+    def __init__(self, shape, dtype, device):
+        self.dev = torch.zeros(shape, device=device, dtype=dtype)
+        self._pin = [torch.zeros(shape, dtype=dtype).pin_memory() for _ in range(self._RING)]
         self._ev = [None] * self._RING
         self._k = 0
 
@@ -233,7 +231,16 @@ class MixBuffer:
         k = self._k
         if self._ev[k] is not None:
             self._ev[k].synchronize()
-        self._pin[k].copy_(torch.tensor(values, dtype=torch.float32))
+        self._pin[k].copy_(torch.as_tensor(values, dtype=self.dev.dtype))
         self.dev.copy_(self._pin[k], non_blocking=True)
         self._ev[k] = torch.cuda.Event()
         self._ev[k].record()
+
+
+class MixBuffer(PinnedUpload):
+    """Device copy of one step's packed draw (MixDraw.packed): `clip` feeds ub_patchify_mix, `target` ub_soft_target_ce, both views
+    of the PinnedUpload.  mix_clips=False (label smoothing without mixup_fn): `clip` is None and the clip is patchified as it comes."""
+
+    def __init__(self, device, mix_clips: bool = True):
+        super().__init__(16, torch.float32, device)
+        self.clip, self.target = (self.dev[:10] if mix_clips else None), self.dev[10:13]

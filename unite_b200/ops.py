@@ -302,10 +302,44 @@ def patchify_mix_u8(x, out, mix, tubelet, mean=IMAGENET_MEAN, std=IMAGENET_STD):
     return out
 
 
-def clip_shape(x, paired=False):
+@_instrument("patchify_aug", 1)
+def patchify_aug_u8(x, out, draw, crop_size, tubelet, erase_mode=0, mix=None, noise=None, rng=None, seed=0, mean=IMAGENET_MEAN,
+                    std=IMAGENET_STD):
+    """Rows of the stage-2 training crop, flip and random erasing of decoded uint8 frames x [B,T,H,W,3] (any H, W), normalised on the
+    way: out bf16 [B*(T/tubelet)*(crop_size/16)^2, 3*tubelet*256].  draw: device int32 [B,10] per-clip draws (augment.AugBuffer.draw);
+    erase_mode 0 const, 1 rand, 2 pixel; noise: fp32 [B,T,3] (rand) or [B,T,3,S,S] (pixel) normals in place of the generator, whose
+    counter rng (device int64 [2]) the launch advances; mix: ub_patchify_mix's device draw (fp32 [10]) or None.  x is not written."""
+    if x.dim() != 5 or x.shape[-1] != 3 or not x.is_contiguous():
+        raise _cabi.UBError(f"patchify_aug_u8: contiguous uint8 [B,T,H,W,3] expected, got {tuple(x.shape)}")
+    B, T, H, W, _ = x.shape
+    S = int(crop_size)
+    if tuple(draw.shape) != (B, 10):
+        raise _cabi.UBError(f"patchify_aug_u8: draw must be int32 [{B}, 10], got {tuple(draw.shape)}")
+    if mix is not None and mix.numel() < 10:
+        raise _cabi.UBError("patchify_aug_u8: mix must hold 10 floats")
+    if noise is not None and tuple(noise.shape) != ((B, T, 3) if erase_mode == 1 else (B, T, 3, S, S)):
+        raise _cabi.UBError(f"patchify_aug_u8: noise of shape {tuple(noise.shape)} does not fit erase mode {erase_mode}")
+    if rng is not None and (rng.dtype != torch.int64 or rng.numel() != 2):
+        raise _cabi.UBError("patchify_aug_u8: rng must be a device int64 [2] counter")
+    n_tok = B * (T // tubelet) * (S // 16) ** 2
+    if tuple(out.shape) != (n_tok, 3 * tubelet * 256):
+        raise _cabi.UBError(f"patchify_aug_u8: out must be [{n_tok}, {3 * tubelet * 256}], got {tuple(out.shape)}")
+    m3, s3 = (C.c_float * 3)(*mean), (C.c_float * 3)(*std)
+    check(lib.ub_patchify_aug_u8(_p(x, U8, "frames"), _p(out, BF16, "patches"), _p(draw, I32, "draw"), _p(mix, F32, "mix"), int(erase_mode),
+                                 _p(noise, F32, "noise"), int(seed) & 0xFFFFFFFFFFFFFFFF, _p(rng, torch.int64, "rng"), m3, s3, B, T, H, W, S,
+                                 tubelet, _stream()), "ub_patchify_aug_u8")
+    return out
+
+
+def clip_shape(x, paired=False, crop_size=None):
     """The [B,3,T,H,W] shape of the clip a batch stands for: an fp32 clip's own shape, or that of the clip decoded uint8 frames
     [B,T,H,W,3] normalise to.  A uint8 batch that patchify_u8 / patchify_mix_u8 cannot read raises ValueError here, before any
-    launch: not contiguous [B,T,H,W,3], H or W not a multiple of 16, or (paired: clip b is mixed with clip B-1-b) an odd batch."""
+    launch: not contiguous [B,T,H,W,3], H or W not a multiple of 16, or (paired: clip b is mixed with clip B-1-b) an odd batch.
+    crop_size S (a spatial augmentation, patchify_aug_u8): the batch must be uint8 frames, of any H, W, and stands for the augmented
+    clip [B,3,T,S,S]."""
+    if crop_size is not None and x.dtype != U8:
+        raise ValueError(f"the spatial augmentation runs on decoded uint8 frames [B,T,H,W,3]; got a {x.dtype} batch (a loader that "
+                         "augments on the host feeds the augmented fp32 clip without spatial_aug)")
     if x.dtype != U8:
         return tuple(x.shape)
     if x.dim() != 5 or x.shape[-1] != 3:
@@ -313,11 +347,11 @@ def clip_shape(x, paired=False):
     if not x.is_contiguous():
         raise ValueError(f"uint8 frames must be contiguous; got shape {tuple(x.shape)} with strides {x.stride()}")
     B, T, H, W, _ = x.shape
-    if H % 16 or W % 16:
+    if crop_size is None and (H % 16 or W % 16):
         raise ValueError(f"uint8 frames of {H}x{W} pixels: H and W must be multiples of the 16-pixel patch")
     if paired and B % 2:
         raise ValueError(f"mixup: the batch size must be even (clip b is mixed with clip B-1-b), got {B}")
-    return (B, 3, T, H, W)
+    return (B, 3, T, H, W) if crop_size is None else (B, 3, T, crop_size, crop_size)
 
 
 def padded_k(features: int) -> int:
