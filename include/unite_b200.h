@@ -41,6 +41,12 @@ UB_API int ub_set_sm_limit(int n);
  * ---------------------------------------------------------------------------------------------- */
 enum { UB_ACT_NONE = 0, UB_ACT_QUICKGELU = 1, UB_ACT_GELU = 2, UB_ACT_DGELU = 3, UB_ACT_DOT_AUX = 4 };
 
+/* The epilogue applies its options in this order, in fp32, to the accumulator acc = A B^T of each element:
+ *   LayerNorm fold (rstd * (acc - mu * ln_c[n])) -> + bias[n] -> activation (QuickGELU / GELU, whose input is what aux_out stores;
+ *   or DGELU: * gelu'(aux_in); or DOT_AUX: dot_out from the rounded C) -> * row_scale -> + residual, or C += (accumulate)
+ * and rounds once, to C's type.  colsum_out sums the fp32 values before that rounding; stats_out sums the rounded fp16 values.
+ * split_k > 1 (after its clamp to the number of 64-deep k-blocks) needs accumulate and allows no bias and no activation; DGELU
+ * allows no bias. */
 typedef struct ub_gemm_epilogue {
   const float* bias;      /* [N] added to the accumulator, or NULL                                         */
   const float* residual;  /* fp32 [M, ldr] added last, or NULL (may alias C when C is fp32)                 */
@@ -54,8 +60,8 @@ typedef struct ub_gemm_epilogue {
   int32_t out_fp32; /* 0: C is bf16, 1: C is fp32                                                         */
   int32_t accumulate; /* 1: C (fp32) += result with red.add (required when split_k > 1)                   */
   int32_t tile_ctas;  /* scheduling hint: 0 = cost model, 1 / 2 / 4 = CTAs per work item (4 = two pairs + B multicast) */
-  int32_t max_ctas;   /* scheduling hint: 0 = whole device, > 0 = cap on the persistent grid (a GEMM run beside another),
-                       * < 0 = non-persistent: one CTA (pair) per work item, for off-critical-path GEMMs on a low-priority stream */
+  int32_t max_ctas;   /* scheduling hint: 0 = whole device, > 0 = cap on the persistent grid (a GEMM run beside another);
+                       * negative values are refused                                                                   */
   int32_t residual_f16; /* 1: `residual` is fp16 [M, ldr] and C is fp16 too (out_fp32 must be 0): the teacher's residual stream */
   int32_t ab_f16;       /* 1: A and B hold fp16 (not bf16) values                                                          */
   /* LayerNorm folded into the GEMM (frozen teacher): with A = the raw residual stream x (fp16), B = gamma o W, ln_c[n] =
@@ -72,7 +78,8 @@ typedef struct ub_gemm_epilogue {
   /* Grouped GEMM: several independent products of the same shape in ONE launch (the K alignment decoders of
    * modeling_adaptation.py:203-213, 322-325: y_k = z_k W_k^T + b_k, their dgrad and wgrad) — one wave-quantisation loss and one
    * launch instead of K.  C is the groups' outputs stacked along M (M = total rows, group_rows rows each, a multiple of 256);
-   * the tile whose first row is m0 belongs to group g = m0 / group_rows and reads its operands at
+   * every row m belongs to group g = m / group_rows (cluster-of-4 tiles, 512 rows each, are only used when group_rows is a
+   * multiple of 512) and reads its operands at
    *   A: k + g * group_a_k, m - g * group_a_m        B: k + g * group_b_k, n + g * group_b_n        bias[n + g * group_bias]
    * (offsets in elements of the respective dimension; K is the per-group contraction length).  All 0 = ordinary GEMM.          */
   int32_t group_rows, group_a_k, group_a_m, group_b_k, group_b_n, group_bias;

@@ -824,6 +824,9 @@ extern "C" int ub_gemm_bf16(const void* A, int64_t lda, int a_mn_major, const vo
                                           ep.colsum_out == nullptr && ep.group_rows == 0),
              "gemm: UB_ACT_DOT_AUX needs aux_in, dot_out, dot_seq_len dividing M, a bf16 output with N %% 64 == 0 and no other epilogue option");
   UB_REQUIRE(!(ep.act == UB_ACT_DGELU && ep.residual != nullptr), "gemm: DGELU with a residual is not supported");
+  // the epilogue would add the bias to the zero-filled rows past M as well, and colsum_out would sum gelu'(0) * bias over them
+  UB_REQUIRE(!(ep.act == UB_ACT_DGELU && ep.bias != nullptr), "gemm: DGELU with a bias is not supported");
+  UB_REQUIRE(ep.max_ctas >= 0, "gemm: max_ctas=%d must be >= 0", ep.max_ctas);
   UB_REQUIRE(ep.residual == nullptr || ep.out_fp32 || ep.residual_f16, "gemm: the residual epilogue writes fp32 (or fp16 with residual_f16)");
   UB_REQUIRE(!ep.residual_f16 || (ep.residual != nullptr && !ep.out_fp32), "gemm: residual_f16 needs a residual and a 2-byte (fp16) output");
   UB_REQUIRE((ep.ln_stats == nullptr) == (ep.ln_c == nullptr), "gemm: ln_stats and ln_c go together");
@@ -851,6 +854,9 @@ extern "C" int ub_gemm_bf16(const void* A, int64_t lda, int a_mn_major, const vo
   if (split_k > total_kb) split_k = total_kb;
   int kb_per_split = (total_kb + split_k - 1) / split_k;
   split_k = (total_kb + kb_per_split - 1) / kb_per_split;  // no empty splits
+  // every split runs the whole epilogue on its partial sum: a bias would be added once per split, an activation applied to parts
+  UB_REQUIRE(split_k == 1 || (ep.bias == nullptr && ep.act == UB_ACT_NONE),
+             "gemm: split_k=%d (after the clamp to %d k-blocks) cannot be combined with a bias or an activation", split_k, total_kb);
 
   // tile choice: 256-wide tiles unless that costs a whole extra wave; CTA pairs (256 x 256 per pair) for the wide tiles
   const int sms = sm_count();
@@ -897,6 +903,8 @@ extern "C" int ub_gemm_bf16(const void* A, int64_t lda, int a_mn_major, const vo
   if (ep.tile_ctas == 1) ncta = 1;
   if (ep.tile_ctas == 2 && bn == 256 && M > BM) ncta = 2;
   if (ep.tile_ctas == 4 && bn == 256 && M >= 4 * BM && units4 > 0) ncta = 4;
+  // a work item takes its group from its first row: a 512-row item must not straddle two groups
+  if (ncta == 4 && ep.group_rows % (4 * BM) != 0) ncta = 2;
 
   const int epi = ep.residual != nullptr ? (ep.residual_f16 ? 3 : 1)
                                          : ((ep.act == UB_ACT_DGELU || ep.act == UB_ACT_DOT_AUX) ? 2 : (ep.ln_stats != nullptr ? 4 : 0));
